@@ -33,6 +33,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: importing the package must not write __pycache__ into it
 
 import numpy as np  # noqa: E402
 
@@ -73,6 +74,9 @@ def parse():
     ap.add_argument("--pipeline-diagnostics", action="store_true", help="also time the rest of the step (two more event records per call): rest_of_step_ms, pipeline_gaps")
     ap.add_argument("--no-pin", action="store_true", help="diagnostic: leave the CPU affinity alone")
     ap.add_argument("--ref-passes", type=int, default=8, help="reference arm: ring passes per host thread per step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the weak leg, write what its caller holds (rank 0's channels) as DIR/<name>.npy, float32/float64, "
+                         "under 64 MB; the inputs are seeded, so two builds can be compared array for array")
     a = ap.parse_args()
     if a.channels is None:
         world = int(os.environ.get("WORLD_SIZE", "1"))   # ranks actually launched (torchrun); --gpus is informational
@@ -336,13 +340,15 @@ def decode_leg(D: Dist, args, n_local, ch0, n_total, steps, warmup, timing=True,
         if not any(dec.poll_chars(c) for c in (0, n_local // 2, n_local - 1)):
             break
         dec.gather_results(sink)
+    # the sink hands each stream out once: take this rank's channels here for the parity check and --dump-outputs
+    got = [(sink.poll_chars(g), sink.poll_sentences(g)) for g in range(ch0, ch0 + n_local)]
     per_rank_diag = {"k1_avg_ms": D.all_values(k1_ms / max(k1_cnt, 1)), "host_replay_ms_total": D.all_values(replay_ms),
                      "issue_max_ms": D.all_values(issue_max * 1e3), "drain_max_ms": D.all_values(drain_max * 1e3), "final_ms": D.all_values(final_ms), "final_gather_ms": D.all_values(final_gather_ms),
                      "sm_mhz": D.all_values(float(clocks["sm_mhz"] or 0)), "throttle_reasons": D.all_values(float(len(clocks["reasons"])))}
     per_rank_ms = D.all_values(ms)
     per_rank_issue = D.all_values(t_issue * 1e3 / max(steps, 1))
     per_rank_drain = D.all_values((t_drain * 1e3 + final_ms) / max(steps, 1))
-    return {"dec": dec, "sink": sink, "ring": ring, "ms": ms, "ms_max": max(per_rank_ms), "per_rank_ms": per_rank_ms,
+    return {"dec": dec, "sink": sink, "got": got, "ring": ring, "ms": ms, "ms_max": max(per_rank_ms), "per_rank_ms": per_rank_ms,
             "per_rank_issue_ms": per_rank_issue, "per_rank_drain_ms": per_rank_drain, "per_rank_diag": per_rank_diag, "k1_ms": k1_ms, "k1_cnt": k1_cnt,
             "rest_ms": rest_ms, "rest_cnt": rest_cnt, "gaps": gaps, "launches": launches, "clocks": clocks, "final_ms": final_ms,
             "chunks_decoded": n_done, "preroll": preroll, "gathers": gathers, "L": L}
@@ -357,7 +363,7 @@ def parity_check(D: Dist, args, leg, n_local, ch0):
         threads = len(os.sched_getaffinity(0))
     except Exception:
         threads = os.cpu_count() or 1
-    sink, ring, L = leg["sink"], leg["ring"], leg["L"]
+    ring, L = leg["ring"], leg["L"]
     torch = D.torch
     t0 = time.time()
     bad, n_chars, n_sent, sent_min = [], 0, 0, None
@@ -388,7 +394,7 @@ def parity_check(D: Dist, args, leg, n_local, ch0):
         ref_chars, ref_sents = po.run_ring(kind, cfg, iq, threads, FS, args.chunk, 0, leg["chunks_decoded"])
         for k in range(c1 - c0):
             g = ch0 + c0 + k
-            got_c, got_s = sink.poll_chars(g), sink.poll_sentences(g)
+            got_c, got_s = leg["got"][c0 + k]
             n_chars += len(ref_chars[k]); n_sent += len(ref_sents[k])
             sent_min = len(got_s) if sent_min is None else min(sent_min, len(got_s))
             if got_c != ref_chars[k] or got_s != ref_sents[k]:
@@ -400,6 +406,44 @@ def parity_check(D: Dist, args, leg, n_local, ch0):
     return {"channels_checked": checked, "mismatches": mism, "first_bad": bad[:4], "oracle": "reference" if kind == "ref" else "port",
             "chunks_per_channel": leg["chunks_decoded"], "chars_compared": D.sum_int(n_chars), "sentences_compared": D.sum_int(n_sent),
             "sentences_min": smin, "seconds": round(time.time() - t0, 1), "host_threads_per_rank": threads}
+
+
+DUMP_TAIL = 512                 # newest bytes kept of each channel's character and sentence streams (a step adds about one)
+DUMP_POWER_CHANNELS = 256       # power spectra are fft_n floats per channel: a fixed sample of channels
+
+
+def dump_outputs(out_dir, leg, n_local, ch0):
+    """What the caller of the weak leg holds after its last timed step, for comparing two builds output for output:
+    the newest characters and sentences gathered per channel, the newest record's scalars (frequency correction, shift,
+    noise floor, noise variance, left and right peak), the last step's demodulated block and the current power spectrum.
+    Rows are padded with NaN; characters are byte values.  Channels (local numbers in channels.npy) are a fixed, seeded
+    sample where all of them would exceed 64 MB."""
+    dec, sink = leg["dec"], leg["sink"]
+
+    def rows(items):
+        a = np.full((len(items), max([len(x) for x in items] + [1])), np.nan, dtype=np.float32)
+        for i, x in enumerate(items):
+            a[i, :len(x)] = x
+        return a
+
+    rng = np.random.default_rng(20240601)
+    demod_w = max(len(dec.getDemodulated(0)), 1)
+    per_channel = 4 * (2 * DUMP_TAIL + demod_w) + 8 * 7
+    n = min(n_local, (48 << 20) // per_channel)          # + at most 16 MB of power spectra
+    chans = np.arange(n_local) if n == n_local else np.sort(rng.choice(n_local, n, replace=False))
+    tail = lambda b: np.frombuffer(b[-DUMP_TAIL:], dtype=np.uint8)
+    stats = [sink.stats(ch0 + int(c)) for c in chans]
+    pchans = chans if n <= DUMP_POWER_CHANNELS else np.sort(rng.choice(chans, DUMP_POWER_CHANNELS, replace=False))
+    out = {"channels": chans.astype(np.float64),
+           "chars": rows([tail(leg["got"][c][0]) for c in chans]),
+           "sentences": rows([tail(b"".join(s + b"\n" for s in leg["got"][c][1])) for c in chans]),
+           "stats": np.stack([s if s is not None else np.full(6, np.nan) for s in stats]).astype(np.float64),
+           "demodulated": rows([dec.getDemodulated(int(c)) for c in chans]),
+           "power_spectrum": rows([dec.getPowerSpectrum(int(c)) for c in pchans]),
+           "power_spectrum_channels": pchans.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_e2e(D: Dist, args, ring, C):
@@ -460,7 +504,9 @@ def run_wideband(D: Dist, args):
     from habdec_b200 import api
     fs, n_ch, chunk, steps = 20e6, 1024, 65536, 40
     n_slices = 64
-    cap = torch.randn((n_slices * chunk, 2), dtype=torch.float32, device=D.dev) * 0.7
+    gen = torch.Generator(device=D.dev)
+    gen.manual_seed(2024)
+    cap = torch.randn((n_slices * chunk, 2), dtype=torch.float32, device=D.dev, generator=gen) * 0.7
     dec = api.BatchDecoder(n_ch, device=D.local_rank, baud=300.0, rtty_bits=8, rtty_stops=2.0, dec_factor=FACTOR)
     stream = torch.cuda.current_stream()
     dec.set_stream(stream.cuda_stream)
@@ -515,6 +561,8 @@ def run_ours(args):
 
     # ---- weak leg: the headline ------------------------------------------------------------------------
     leg = decode_leg(D, args, C, ch0, args.channels, args.steps, args.warmup, timing=not args.no_kernel_timing)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, leg, C, ch0)
     ms_max = leg["ms_max"]
     total_samples = float(args.channels) * args.chunk * args.steps
     value = total_samples / (ms_max * 1e-3) / 1e6
