@@ -17,6 +17,42 @@ LIB_PATH = os.environ.get("HBD_LIB") or os.path.join(_HERE, "libhabdec_b200.so")
 HBD_OK, HBD_ERR_ARG, HBD_ERR_CUDA, HBD_ERR_STATE, HBD_ERR_NOMEM = 0, -1, -2, -3, -4
 STAGE_DECIMATED, STAGE_FILTERED, STAGE_DEMOD, STAGE_LPTAPS, STAGE_PENDING, STAGE_BITS = 0, 1, 2, 5, 6, 7
 
+# input sample formats (hbd_iq_format): interleaved I, Q, little endian
+IQ_CF32, IQ_CS16, IQ_CS8, IQ_CU8 = 0, 1, 2, 3
+IQ_BYTES = {IQ_CF32: 8, IQ_CS16: 4, IQ_CS8: 2, IQ_CU8: 2}          # per complex sample
+_IQ_DTYPE = {IQ_CF32: np.float32, IQ_CS16: np.int16, IQ_CS8: np.int8, IQ_CU8: np.uint8}
+
+
+def dequantise(q, fmt: int) -> np.ndarray:
+    """The value the decoder sees for integer IQ `q` ([..., 2] or [..., 2n] interleaved I, Q of the format's dtype):
+    CS16 v / 32768, CS8 v / 128, CU8 (v - 128) / 128; complex64 [...]/[..., n].  Every value is exact in float32."""
+    q = np.asarray(q)
+    if fmt == IQ_CF32:
+        return np.ascontiguousarray(q, dtype=np.float32).view(np.complex64).reshape(q.shape[:-1] + (-1,))
+    if q.dtype != _IQ_DTYPE[fmt]:
+        raise ValueError("format %d needs %s samples, got %s" % (fmt, np.dtype(_IQ_DTYPE[fmt]).name, q.dtype))
+    v = q.astype(np.float64)
+    v = v / 32768.0 if fmt == IQ_CS16 else (v / 128.0 if fmt == IQ_CS8 else (v - 128.0) / 128.0)
+    return np.ascontiguousarray(v.astype(np.float32)).view(np.complex64).reshape(q.shape[:-1] + (-1,))
+
+
+def quantise(iq, fmt: int, scale: float = 1.0):
+    """Integer IQ of the format from complex samples: round(iq * scale * 2^k) (+ 128 for CU8), clipped to the format's range;
+    interleaved [..., 2n].  numpy in -> numpy out, torch in -> torch out (on the tensor's device)."""
+    if fmt == IQ_CF32:
+        raise ValueError("quantise makes integer formats")
+    full = {IQ_CS16: 32768.0, IQ_CS8: 128.0, IQ_CU8: 128.0}[fmt]
+    lo, hi = (-32768, 32767) if fmt == IQ_CS16 else ((-128, 127) if fmt == IQ_CS8 else (0, 255))
+    off = 128.0 if fmt == IQ_CU8 else 0.0
+    if not isinstance(iq, np.ndarray) and type(iq).__module__.startswith("torch"):
+        import torch
+        ri = torch.view_as_real(iq.to(torch.complex64)).reshape(*iq.shape[:-1], -1)
+        dt = {IQ_CS16: torch.int16, IQ_CS8: torch.int8, IQ_CU8: torch.uint8}[fmt]
+        return torch.clamp(torch.round(ri * float(scale * full)) + off, lo, hi).to(dt)
+    iq = np.asarray(iq, dtype=np.complex64)
+    ri = iq.view(np.float32).reshape(iq.shape[:-1] + (-1,)).astype(np.float64)
+    return np.clip(np.round(ri * (scale * full)) + off, lo, hi).astype(_IQ_DTYPE[fmt])
+
 
 class SpectrumInfo(C.Structure):
     _fields_ = [("min_", C.c_float), ("max_", C.c_float), ("noise_floor_", C.c_double), ("noise_variance_", C.c_double),
@@ -89,6 +125,11 @@ SIGNATURES = {
     "hbd_afc_retune": (C.c_int, [_H, C.c_double, C.c_void_p]),
     "hbd_push_wideband": (C.c_int, [_H, C.c_void_p, C.c_size_t, C.c_double]),
     "hbd_push_wideband_device": (C.c_int, [_H, C.c_void_p, C.c_size_t, C.c_double]),
+    "hbd_push_iq": (C.c_int, [_H, C.c_int, C.c_void_p, C.c_int, C.c_size_t, C.c_double]),
+    "hbd_push_iq_batch": (C.c_int, [_H, C.c_void_p, C.c_int, C.c_size_t, C.c_size_t, C.c_double]),
+    "hbd_push_iq_device": (C.c_int, [_H, C.c_void_p, C.c_int, C.c_size_t, C.c_size_t, C.c_double]),
+    "hbd_push_iq_wideband": (C.c_int, [_H, C.c_void_p, C.c_int, C.c_size_t, C.c_double]),
+    "hbd_push_iq_wideband_device": (C.c_int, [_H, C.c_void_p, C.c_int, C.c_size_t, C.c_double]),
     "hbd_process": (C.c_int, [_H]),
     "hbd_process_async": (C.c_int, [_H]),
     "hbd_collect": (C.c_int, [_H]),
@@ -524,6 +565,36 @@ class BatchDecoder:
 
     def pushWidebandDevice(self, ptr: int, n: int, fs: float):
         self._chk(self._lib.hbd_push_wideband_device(self._h, ptr, n, float(fs)))
+
+    # ---- integer IQ input (hbd_push_iq*): arrays are interleaved I, Q of the format's dtype, [..., 2n]
+    @staticmethod
+    def _iq_arr(arr, fmt, ndim):
+        arr = np.ascontiguousarray(arr, dtype=_IQ_DTYPE[fmt])
+        assert arr.ndim == ndim and arr.shape[-1] % 2 == 0, "interleaved I, Q expected"
+        return arr
+
+    def pushIQ(self, ch: int, arr: np.ndarray, fmt: int, fs: float):
+        arr = self._iq_arr(arr, fmt, 1)
+        self._chk(self._lib.hbd_push_iq(self._h, ch, arr.ctypes.data, int(fmt), arr.shape[-1] // 2, float(fs)))
+
+    def pushIQBatch(self, arr: np.ndarray, fmt: int, fs: float):
+        """arr: [n_channels, n, 2] or [n_channels, 2n] (rows may be a strided view of a wider matrix)"""
+        arr = np.asarray(arr)
+        if arr.ndim == 3:
+            arr = arr.reshape(arr.shape[0], -1)
+        assert arr.ndim == 2 and arr.shape[0] == self.n_channels and arr.dtype == _IQ_DTYPE[fmt]
+        assert arr.strides[1] == arr.itemsize and arr.strides[0] % IQ_BYTES[fmt] == 0
+        self._chk(self._lib.hbd_push_iq_batch(self._h, arr.ctypes.data, int(fmt), arr.shape[1] // 2, arr.strides[0] // IQ_BYTES[fmt], float(fs)))
+
+    def pushIQDevice(self, ptr: int, fmt: int, n: int, pitch: int, fs: float):
+        self._chk(self._lib.hbd_push_iq_device(self._h, ptr, int(fmt), n, pitch, float(fs)))
+
+    def pushIQWideband(self, arr: np.ndarray, fmt: int, fs: float):
+        arr = self._iq_arr(arr, fmt, 1)
+        self._chk(self._lib.hbd_push_iq_wideband(self._h, arr.ctypes.data, int(fmt), arr.shape[-1] // 2, float(fs)))
+
+    def pushIQWidebandDevice(self, ptr: int, fmt: int, n: int, fs: float):
+        self._chk(self._lib.hbd_push_iq_wideband_device(self._h, ptr, int(fmt), n, float(fs)))
 
     # ---- run
     def process(self): self._chk(self._lib.hbd_process(self._h))

@@ -18,6 +18,7 @@
 #include <vector>
 
 #include "decim1.cuh"
+#include "iq_format.cuh"
 #include "mid.cuh"
 #include "decim_taps.inc"
 #include "fft_afc.cuh"
@@ -27,6 +28,7 @@
 #include "telemetry_abi.h"
 #include "api_internal.h"
 #include "nco.cuh"
+#include "iq_format.cuh"
 #include "ssdv.cuh"
 #include "tail.cuh"
 #include "wire.cuh"
@@ -250,6 +252,13 @@ struct hbd_decoder {
     // input
     float2* d_stage = nullptr; size_t stage_pitch = 0;   // host pushes land here
     const float2* ext = nullptr; size_t ext_pitch = 0; size_t ext_n = 0; // zero-copy device push
+    int ext_format = HBD_IQ_CF32;    // ... of integer samples that K1 reads itself (decim1_supports_native_iq); ext then points at them
+    // integer input that K1 does not read natively: host data is uploaded as integers to d_iq_up, device data is widened
+    // to cf32 into d_widen and pushed from there like a cf32 device matrix
+    unsigned char* d_iq_up = nullptr; size_t iq_up_bytes = 0;
+    float2* d_widen = nullptr; size_t widen_bytes = 0;
+    int ensure_iq_up(size_t bytes);
+    int widen_device(const void* src, int format, size_t n, size_t pitch, size_t* out_pitch);
     // fused-NCO parameter ring: pinned host slots + device slots, so a push never waits for the GPU
     static constexpr unsigned kNcoSlots = 16;
     NcoChan* h_nco_pin = nullptr; NcoChan* d_nco_ring = nullptr; cudaEvent_t ev_nco[kNcoSlots] = {}; unsigned nco_seq = 0;
@@ -271,7 +280,7 @@ struct hbd_decoder {
     float2* d_wide = nullptr; size_t wide_cap = 0;       // wideband capture row shared by all channels
     bool nco_any = false;    // some channel has (had) a non-zero NCO frequency or phase (set by hbd_set_nco, never cleared)
     bool nco_active() const { return nco_any; }
-    int mix_into_stage(const float2* src, size_t src_pitch, int c0, int nc, size_t dst_off, size_t n);
+    int mix_into_stage(const void* src, size_t src_pitch, int c0, int nc, size_t dst_off, size_t n, int format = HBD_IQ_CF32);
     int pending_marks = 0;   // async calls since the last collect
     int sv_override = -1;
     bool mask_cache = true;      // HBD_MASK_CACHE=0 (test hook): the slicer's position masks are rebuilt from scratch in every call
@@ -535,7 +544,7 @@ void hbd_decoder::free_all()
     if (ev_in) cudaEventDestroy(ev_in);
     void* ptrs[] = {d_state, d_plan, d_carry2[0], d_carry2[1], d_s1x[0], d_s1x[1], d_decq, d_fftbuf, d_spectrum, d_power, d_lptaps, d_slicer, d_demod, d_uart_runs, d_maskc, d_log, d_log_ctl,
                     d_taps1, d_taps2, d_twiddle, d_cfg_baud, d_cfg_stops, d_cfg_bits, d_cfg_dc, d_cfg_ntaps,
-                    d_cfg_dirty, d_rec_dec, d_rec_filt, d_rec_bits, d_rec_bits_n, d_stage, d_nco, d_wide, d_dacc, d_dacc_n, d_frames, d_frame_sizes,
+                    d_cfg_dirty, d_rec_dec, d_rec_filt, d_rec_bits, d_rec_bits_n, d_stage, d_nco, d_wide, d_iq_up, d_widen, d_dacc, d_dacc_n, d_frames, d_frame_sizes,
                     d_ssdv_ring, d_ssdv_total, d_ssdv_scanned, d_ssdv_log};
     for (void* p : ptrs) if (p) cudaFree(p);
     if (h_pinned) cudaFreeHost(h_pinned);
@@ -841,6 +850,12 @@ int hbd_decoder::process_async_locked()
     int sv_want = int(std::min<double>(6144.0, 16.0 * max_spb_c + double(max_nf) + 64.0));
     if (sv_override >= 0) sv_want = sv_override;   // test hook (HBD_SV_WANT): 0 forces the slicer's HBM path
 
+    if (ext && ext_format != HBD_IQ_CF32 && !decim1_supports_native_iq(M1, T1)) {   // the plan changed after an integer device push
+        size_t wp = 0;
+        const int rc = widen_device(ext, ext_format, ext_n, ext_pitch, &wp);
+        if (rc) return rc;
+        ext = d_widen; ext_pitch = wp; ext_format = HBD_IQ_CF32;
+    }
     const float2* chunk = ext ? ext : d_stage;
     const size_t chunk_pitch = ext ? ext_pitch : stage_pitch;
     int nl = 0;
@@ -857,7 +872,7 @@ int hbd_decoder::process_async_locked()
         da.plan = d_plan; da.uplan = uplan; da.uniform = plan_uniform ? 1 : 0; da.taps = d_taps1; da.ch0 = 0; da.n_channels = n_ch;
         da.nco = ext_nco ? ext_nco_ptr : nullptr;
         if (timing) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_k1, ev_used_k1), hi));
-        HBD_CUDA_CHECK(launch_decim1(da, M1, T1, max_n1, n_sms, hi, &nl));
+        HBD_CUDA_CHECK(launch_decim1(da, M1, T1, max_n1, n_sms, hi, &nl, ext ? ext_format : HBD_IQ_CF32));
         if (timing) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_k1, ev_used_k1), hi));
     }
     HBD_CUDA_CHECK(cudaEventRecord(ev_consumed, hi)); // input no longer needed; stage-1 output ready
@@ -930,7 +945,7 @@ int hbd_decoder::process_async_locked()
     HBD_CUDA_CHECK(cudaEventRecord(ev_call[slot], lo)); // everything of this call is done
     ++call_seq;
     ++pending_marks;
-    ext = nullptr; ext_n = 0; ext_nco = false;
+    ext = nullptr; ext_n = 0; ext_nco = false; ext_format = HBD_IQ_CF32;
     return HBD_OK;
 }
 
@@ -1490,8 +1505,9 @@ static int ensure_stage(hbd_decoder* h, size_t need)
 }
 
 // Mix `n` samples per channel of channels [c0, c0+nc) from src into the staging rows at dst_off and advance the
-// channels' NCO phases.  src_pitch 0: one shared (wideband) row.  Runs on the handle's stream.
-int hbd_decoder::mix_into_stage(const float2* src, size_t src_pitch, int c0, int nc, size_t dst_off, size_t n)
+// channels' NCO phases.  src_pitch 0: one shared (wideband) row.  Integer src (format) is widened on the way; a channel
+// without an offset is then a plain widening copy.  Runs on the handle's stream.
+int hbd_decoder::mix_into_stage(const void* src, size_t src_pitch, int c0, int nc, size_t dst_off, size_t n, int format)
 {
     if (!n) return HBD_OK;
     for (int c = c0; c < c0 + nc; ++c) {
@@ -1506,7 +1522,7 @@ int hbd_decoder::mix_into_stage(const float2* src, size_t src_pitch, int c0, int
     }
     HBD_CUDA_CHECK(cudaMemcpyAsync(d_nco + c0, h_nco.data() + c0, sizeof(NcoChan) * size_t(nc), cudaMemcpyHostToDevice, stream));
     int nl = 0;
-    HBD_CUDA_CHECK(launch_nco_mix(src, src_pitch, d_stage, stage_pitch, dst_off, n, d_nco, c0, nc, stream, &nl));
+    HBD_CUDA_CHECK(launch_nco_mix(src, src_pitch, d_stage, stage_pitch, dst_off, n, d_nco, c0, nc, stream, &nl, format));
     launches += unsigned(nl);
     HBD_CUDA_CHECK(cudaStreamSynchronize(stream)); // h_nco is rewritten by the next push
     return HBD_OK;
@@ -1596,10 +1612,11 @@ int hbd_push_samples_batch(hbd_decoder* h, const float* iq, size_t n, size_t pit
 
 // One capture shared by every channel (frequency-offset channels of a wideband capture): each channel receives
 // iq * exp(-2 pi i f_nco t).  `device` != 0: iq is a device pointer.
-static int push_wideband(hbd_decoder* h, const float* iq, size_t n, double fs, bool device)
+static int push_wideband(hbd_decoder* h, const void* iq, size_t n, double fs, bool device, int format = HBD_IQ_CF32)
 {
     HBD_CHECK_H(h);
-    if (!iq && n) return HBD_ERR_ARG;
+    const size_t bytes = size_t(iq_bytes(format));
+    if (!bytes || (!iq && n)) return HBD_ERR_ARG;
     std::lock_guard<std::mutex> l(h->mtx);
     if (h->ext) { h->set_error("device push pending"); return HBD_ERR_STATE; }
     if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
@@ -1607,14 +1624,29 @@ static int push_wideband(hbd_decoder* h, const float* iq, size_t n, double fs, b
     if (!h->queue_depth_equal(base)) { h->set_error("wideband push needs equal queue depth in all channels"); return HBD_ERR_STATE; }
     latch_rate(h, fs);
     const float2* src = reinterpret_cast<const float2*>(iq);
-    if (!device) {
+    if (!device || format != HBD_IQ_CF32) {
         if (n > h->wide_cap) {
             if (h->d_wide) { cudaStreamSynchronize(h->stream); cudaFree(h->d_wide); h->d_wide = nullptr; }
             if (cudaMalloc((void**)&h->d_wide, n * sizeof(float2)) != cudaSuccess) { h->set_error("wideband buffer alloc"); return HBD_ERR_NOMEM; }
             h->wide_cap = n;
         }
-        cudaError_t e = cudaMemcpyAsync(h->d_wide, iq, n * sizeof(float2), cudaMemcpyHostToDevice, h->stream);
-        if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
+        if (format == HBD_IQ_CF32) {
+            cudaError_t e = cudaMemcpyAsync(h->d_wide, iq, n * sizeof(float2), cudaMemcpyHostToDevice, h->stream);
+            if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
+        } else if (n) {   // integer capture: widened once into the row every channel reads, the rest is the cf32 path
+            const void* row = iq;
+            if (!device) {
+                const int rc = h->ensure_iq_up(n * bytes);
+                if (rc) return rc;
+                cudaError_t e = cudaMemcpyAsync(h->d_iq_up, iq, n * bytes, cudaMemcpyHostToDevice, h->stream);
+                if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
+                row = h->d_iq_up;
+            }
+            int nl = 0;
+            cudaError_t e = launch_nco_mix(row, 0, h->d_wide, 0, 0, n, nullptr, 0, 1, h->stream, &nl, format);
+            h->launches += unsigned(nl);
+            if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
+        }
         src = h->d_wide;
     }
     if (h->nco_fused && base == 0 && n && decim1_supports_fused_nco(h->M1, h->T1) && !(reinterpret_cast<uintptr_t>(src) & 15)) {
@@ -1631,6 +1663,8 @@ static int push_wideband(hbd_decoder* h, const float* iq, size_t n, double fs, b
 }
 int hbd_push_wideband(hbd_decoder* h, const float* iq, size_t n, double fs) { return push_wideband(h, iq, n, fs, false); }
 int hbd_push_wideband_device(hbd_decoder* h, const float* d_iq, size_t n, double fs) { return push_wideband(h, d_iq, n, fs, true); }
+int hbd_push_iq_wideband(hbd_decoder* h, const void* iq, int format, size_t n, double fs) { return push_wideband(h, iq, n, fs, false, format); }
+int hbd_push_iq_wideband_device(hbd_decoder* h, const void* d_iq, int format, size_t n, double fs) { return push_wideband(h, d_iq, n, fs, true, format); }
 
 int hbd_set_nco(hbd_decoder* h, int ch, double freq_hz)
 {
@@ -1670,6 +1704,112 @@ int hbd_push_samples_device(hbd_decoder* h, const float* d_iq, size_t n, size_t 
     { unsigned base = 0; if (!h->queue_depth_equal(base) || base) { h->set_error("host push pending"); return HBD_ERR_STATE; } }
     h->ext = reinterpret_cast<const float2*>(d_iq); h->ext_pitch = pitch; h->ext_n = n;
     return HBD_OK;
+}
+
+// ---- integer IQ input (include/habdec_b200.h: hbd_push_iq*) -------------------------------------------------------------
+int hbd_decoder::ensure_iq_up(size_t bytes)
+{
+    if (bytes <= iq_up_bytes) return HBD_OK;
+    HBD_CUDA_CHECK(cudaStreamSynchronize(stream));   // a widen of the previous push may still read the old buffer
+    cudaFree(d_iq_up); d_iq_up = nullptr; iq_up_bytes = 0;
+    HBD_CUDA_CHECK(cudaMalloc((void**)&d_iq_up, bytes));
+    iq_up_bytes = bytes;
+    return HBD_OK;
+}
+
+// device matrix [n_ch][pitch] of `format` -> cf32 d_widen [n_ch][*out_pitch] (even pitch: 16-byte rows), on the stream.  Work
+// put on the stream after a call waits for that call's K1 (process_async_locked), so d_widen is free again by then.
+int hbd_decoder::widen_device(const void* src, int format, size_t n, size_t pitch, size_t* out_pitch)
+{
+    const size_t wp = (n + 1) & ~size_t(1);
+    const size_t bytes = std::max<size_t>(size_t(n_ch) * wp * sizeof(float2), 256);
+    if (bytes > widen_bytes) {
+        HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
+        cudaFree(d_widen); d_widen = nullptr; widen_bytes = 0;
+        HBD_CUDA_CHECK(cudaMalloc((void**)&d_widen, bytes));
+        widen_bytes = bytes;
+    }
+    int nl = 0;
+    HBD_CUDA_CHECK(launch_nco_mix(src, pitch, d_widen, wp, 0, n, nullptr, 0, n_ch, stream, &nl, format));
+    launches += unsigned(nl);
+    *out_pitch = wp;
+    return HBD_OK;
+}
+
+int hbd_push_iq(hbd_decoder* h, int ch, const void* iq, int format, size_t n, double fs)
+{
+    if (format == HBD_IQ_CF32) return hbd_push_samples(h, ch, static_cast<const float*>(iq), n, fs);
+    HBD_CHECK_CH(h, ch);
+    const size_t bytes = size_t(iq_bytes(format));
+    if (!bytes || (!iq && n)) return HBD_ERR_ARG;
+    std::lock_guard<std::mutex> l(h->mtx);
+    if (h->ext) { h->set_error("device push pending"); return HBD_ERR_STATE; }
+    if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
+    if (h->n_ch > 1) h->leave_uniform();
+    HostChan& x = h->hc[size_t(ch)];
+    int rc = ensure_stage(h, size_t(x.pushed) + n);
+    if (!rc && n) rc = h->ensure_iq_up(n * bytes);
+    if (rc) return rc;
+    if (n) {
+        cudaError_t e = cudaMemcpyAsync(h->d_iq_up, iq, n * bytes, cudaMemcpyHostToDevice, h->stream);
+        if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
+    }
+    latch_rate(h, fs);
+    // widened (and mixed, where the channel has an NCO offset) into the staging row; returns after the stream has caught up,
+    // so the caller owns `iq` again
+    rc = h->mix_into_stage(h->d_iq_up, 0, ch, 1, x.pushed, n, format);
+    if (rc) return rc;
+    x.pushed += unsigned(n);
+    return HBD_OK;
+}
+
+int hbd_push_iq_batch(hbd_decoder* h, const void* iq, int format, size_t n, size_t pitch, double fs)
+{
+    if (format == HBD_IQ_CF32) return hbd_push_samples_batch(h, static_cast<const float*>(iq), n, pitch, fs);
+    HBD_CHECK_H(h);
+    const size_t bytes = size_t(iq_bytes(format));
+    if (!bytes || (!iq && n) || pitch < n) return HBD_ERR_ARG;
+    std::lock_guard<std::mutex> l(h->mtx);
+    if (h->ext) { h->set_error("device push pending"); return HBD_ERR_STATE; }
+    if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
+    unsigned base = 0;
+    if (!h->queue_depth_equal(base)) { h->set_error("batch push needs equal queue depth in all channels"); return HBD_ERR_STATE; }
+    int rc = ensure_stage(h, size_t(base) + n);
+    if (!rc && n) rc = h->ensure_iq_up(size_t(h->n_ch) * n * bytes);
+    if (rc) return rc;
+    if (n) {   // the integers cross PCIe, packed [n_ch][n]
+        cudaError_t e = cudaMemcpy2DAsync(h->d_iq_up, n * bytes, iq, pitch * bytes, n * bytes, size_t(h->n_ch), cudaMemcpyHostToDevice, h->stream);
+        if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
+    }
+    latch_rate(h, fs);
+    rc = h->mix_into_stage(h->d_iq_up, n, 0, h->n_ch, base, n, format);   // synchronises: the caller owns `iq` again
+    if (rc) return rc;
+    h->add_pushed(unsigned(n));
+    return HBD_OK;
+}
+
+int hbd_push_iq_device(hbd_decoder* h, const void* d_iq, int format, size_t n, size_t pitch, double fs)
+{
+    if (format == HBD_IQ_CF32) return hbd_push_samples_device(h, static_cast<const float*>(d_iq), n, pitch, fs);
+    HBD_CHECK_H(h);
+    const size_t bytes = size_t(iq_bytes(format));
+    if (!bytes || !d_iq || pitch < n || (pitch * bytes) % 16 || (reinterpret_cast<uintptr_t>(d_iq) & 15)) return HBD_ERR_ARG;
+    size_t wp = 0;
+    {
+        std::lock_guard<std::mutex> l(h->mtx);
+        if (h->ext) { h->set_error("device push pending"); return HBD_ERR_STATE; }
+        if (!h->nco_active() && decim1_supports_native_iq(h->M1, h->T1)) {   // zero copy: K1 streams the integers itself
+            latch_rate(h, fs);
+            { unsigned base = 0; if (!h->queue_depth_equal(base) || base) { h->set_error("host push pending"); return HBD_ERR_STATE; } }
+            h->ext = reinterpret_cast<const float2*>(d_iq); h->ext_pitch = pitch; h->ext_n = n; h->ext_format = format;
+            return HBD_OK;
+        }
+        if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
+        const int rc = h->widen_device(d_iq, format, n, pitch, &wp);
+        if (rc) return rc;
+    }
+    // every other case: the widened matrix takes the cf32 device push's path (fused NCO, K0 pre-mix or zero copy)
+    return hbd_push_samples_device(h, reinterpret_cast<const float*>(h->d_widen), n, wp, fs);
 }
 
 int hbd_process_async(hbd_decoder* h) { HBD_CHECK_H(h); return locked_then_fire(h, [h] { return h->process_async_locked(); }); }

@@ -27,6 +27,7 @@
 // so results match to ~1e-7 relative, inside the 1e-5 relative-L2 budget of the north star.
 #include "hbd_common.cuh"
 #include "decim1.cuh"
+#include "iq_format.cuh"
 #include <algorithm>
 
 namespace hbd {
@@ -131,11 +132,19 @@ constexpr int kRedPitch = 36;            // float2 per row: 16-byte aligned rows
 // (288 B) is written after superblock b (512 B) of the slot has been read, so it only ever covers consumed samples, and
 // the tile is summed before the slot is handed back to the TMA.  That takes 27 KB per CTA off K1's footprint, which is
 // what lets a third tail CTA (or a second FFT CTA) co-reside with K1 on an SM.
-template <int M, int T, int PSBMIN = HBD_K1_PSB_MIN, int STAGES = kStages>
+//
+// Integer input (GRAN = 16 B / sample size > 2): a slot still holds a whole piece as cf32 (boundary pieces are widened in
+// place), and the TMA puts the integers RIGHT-aligned into it, at kIntOff.  Widening forward in batches of 32 samples is then
+// safe in place (cf32 of samples < s ends at 8 s <= kIntOff + s * bytes, where the integers of sample s start), and the
+// reduction rows (288 B per consumed 64 samples) stay below the integers not yet read.
+template <int M, int T, int PSBMIN = HBD_K1_PSB_MIN, int STAGES = kStages, int GRAN = 2>
 struct WarpSmem {
     using G = Geo<M, T, PSBMIN>;
     static constexpr bool kRedInRing = HBD_K1_RED_IN_RING && G::NOUT == 1 && G::PSB * kRedPitch * 8 <= G::PSB * 64 * 8;
-    alignas(16) unsigned char ring[STAGES][G::PIECE_BYTES];
+    static constexpr int kSlotSamples = G::PIECE_SAMPLES + GRAN;               // + alignment slack on both sides
+    static constexpr int kIntOff = (8 - 16 / GRAN) * kSlotSamples;             // byte offset of the integers (GRAN > 2)
+    static_assert(GRAN != 2 || kSlotSamples * 8 == G::PIECE_BYTES, "cf32 slot layout");
+    alignas(16) unsigned char ring[STAGES][kSlotSamples * 8];
     alignas(16) float2 red[kRedInRing ? 1 : G::RED_ROWS][kRedPitch];
     alignas(8) uint64_t full[STAGES];
 };
@@ -250,13 +259,20 @@ __device__ __forceinline__ void nco_fill_e(NcoWarpSmem& ns, const NcoChan& nc, i
     __syncwarp();
 }
 
-template <int M, int T, bool NCO>
+// F: input format (iq_format.cuh).  An integer format streams the integers (2 or 4 B per sample instead of 8) into the ring;
+// interior pieces are widened in registers on their way into the FIR, boundary pieces (carry, ragged channel ends) in
+// place first -- the same values either way, so the result is bit for bit that of the cf32 kernel on the widened input.
+template <int M, int T, bool NCO, int F = HBD_IQ_CF32>
 __global__ void __launch_bounds__(K1Cfg<NCO>::kWarps * 32, 1)
 decim1_kernel(DecimArgs a)
 {
+    using In = typename IqFmt<F>::T;
+    constexpr bool kInt = F != HBD_IQ_CF32;
+    constexpr int kG = 16 / int(sizeof(In));   // samples per 16-byte TMA granule
+    static_assert(!(NCO && kInt), "the fused NCO reads cf32");
     constexpr int kWarps = K1Cfg<NCO>::kWarps;
     using G = Geo<M, T, K1Cfg<NCO>::kPsbMin>;
-    using WS = WarpSmem<M, T, K1Cfg<NCO>::kPsbMin, K1Cfg<NCO>::kSt>;
+    using WS = WarpSmem<M, T, K1Cfg<NCO>::kPsbMin, K1Cfg<NCO>::kSt, kG>;
     constexpr int kSt = K1Cfg<NCO>::kSt;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -295,8 +311,9 @@ decim1_kernel(DecimArgs a)
         g += b_span_hi - b_lo;
         const int ch = a.ch0 + chl;
         const ChanPlan pl = a.uniform ? a.uplan : a.plan[ch];
-        const float2* chunk = a.chunk + (size_t)ch * a.chunk_pitch;
+        const In* chunk = reinterpret_cast<const In*>(a.chunk) + (size_t)ch * a.chunk_pitch;
         const float2* carry = a.carry + (size_t)ch * a.carry_cap + a.carry_cap; // carry[j] valid for -carry_cap <= j < 0
+        auto sample = [&](int j) { return (j < 0) ? carry[j] : IqFmt<F>::dq(chunk[j]); };
         // superblock b covers step-local sample positions x in (64(b-1), 64b]; the outputs k with
         // (b-1)*NOUT < k <= b*NOUT end inside it.  This span owns superblocks [b_lo, b_hi) of the channel.
         const int n1 = int(pl.n1);
@@ -327,39 +344,42 @@ decim1_kernel(DecimArgs a)
         // sample addressing: j = x - r indexes the pushed chunk (j >= 0) or the carry (j < 0);
         // everything below is relative to the first sample of the walk, jw = j - j0 >= 0
         const int j0 = 64 * (b_first - 1) + 1 - int(pl.r);
-        const int odd = j0 & 1;                // ring sample s holds j = (j0 - odd) + p*PIECE_SAMPLES + s
+        const int odd = j0 & (kG - 1);         // ring sample s holds j = (j0 - odd) + p*PIECE_SAMPLES + s
         const int j_cap_lo = -a.carry_cap, j_end = int(pl.n);
 
         // ---- producer: copy piece p into its ring slot ----------------------------------------------------
         auto issue_piece = [&](int p) {
             const int slot = p % kSt;
             unsigned char* dst = sm.ring[slot];
-            const int A = j0 - odd + p * G::PIECE_SAMPLES;          // j of ring sample 0 (even)
+            const int A = j0 - odd + p * G::PIECE_SAMPLES;          // j of ring sample 0 (granule aligned)
             const int want_lo = A + odd, want_hi = want_lo + G::PIECE_SAMPLES;
-            const int lo = max(A, j_cap_lo);                          // even
-            const int hi = min(A + G::PIECE_SAMPLES + 2 * odd, j_end);
-            const int hi2 = max(hi & ~1, lo);                         // 16-byte granular end of the TMA part
+            const int lo = max(A, j_cap_lo);                          // granule aligned
+            const int hi = min(A + G::PIECE_SAMPLES + (kInt ? (odd ? kG : 0) : 2 * odd), j_end);
+            const int hi2 = max(hi & ~(kG - 1), lo);                  // 16-byte granular end of the TMA part
             if (lane == 0) {
                 if (hi2 > lo) {
                     const int c_hi = min(hi2, 0), d_lo = max(lo, 0);
-                    if (WS::kRedInRing) fence_proxy_async();   // the slot last held generic-proxy stores (reduction rows)
-                    mbar_expect_tx(&sm.full[slot], uint32_t(hi2 - lo) * 8u);
+                    // the slot last held generic-proxy stores (reduction rows, widened boundary samples)
+                    if (WS::kRedInRing || kInt) fence_proxy_async();
+                    if (kInt) mbar_expect_tx(&sm.full[slot], uint32_t(max(c_hi - lo, 0)) * 8u + uint32_t(max(hi2 - d_lo, 0)) * uint32_t(sizeof(In)));
+                    else mbar_expect_tx(&sm.full[slot], uint32_t(hi2 - lo) * 8u);
                     if (c_hi > lo) tma_load_1d(dst + (lo - A) * 8, carry + lo, uint32_t(c_hi - lo) * 8u, &sm.full[slot]);
                     if (hi2 > d_lo) {
-                        if (kHint) tma_load_1d_hint(dst + (d_lo - A) * 8, chunk + d_lo, uint32_t(hi2 - d_lo) * 8u, &sm.full[slot], l2_first);
-                        else tma_load_1d(dst + (d_lo - A) * 8, chunk + d_lo, uint32_t(hi2 - d_lo) * 8u, &sm.full[slot]);
+                        unsigned char* dd = kInt ? dst + WS::kIntOff + (d_lo - A) * int(sizeof(In)) : dst + (d_lo - A) * 8;
+                        if (kHint) tma_load_1d_hint(dd, chunk + d_lo, uint32_t(hi2 - d_lo) * uint32_t(sizeof(In)), &sm.full[slot], l2_first);
+                        else tma_load_1d(dd, chunk + d_lo, uint32_t(hi2 - d_lo) * uint32_t(sizeof(In)), &sm.full[slot]);
                     }
                 } else {
                     mbar_arrive(&sm.full[slot]);
                 }
             }
-            if (lo > want_lo || hi2 < want_hi) { // rare: TMA part does not cover the wanted range (ends of a channel)
+            if (!kInt && (lo > want_lo || hi2 < want_hi)) { // rare: TMA part does not cover the wanted range (ends of a channel)
                 float2* d2 = reinterpret_cast<float2*>(dst);
                 for (int j = want_lo + lane; j < want_hi; j += 32) {
                     if (j >= lo && j < hi2) continue;                 // delivered by the bulk copy
                     // odd trailing sample of an odd-length chunk: plain copy; everything not backed by data: zero
                     // (stale shared memory could hold NaN patterns and 0 * NaN would poison a valid output)
-                    d2[j - A] = (j >= lo && j < hi) ? ((j < 0) ? carry[j] : chunk[j]) : make_float2(0.f, 0.f);
+                    d2[j - A] = (j >= lo && j < hi) ? sample(j) : make_float2(0.f, 0.f);
                 }
             }
         };
@@ -423,43 +443,81 @@ decim1_kernel(DecimArgs a)
                     }
                 }
             }
-            const float2* src = reinterpret_cast<const float2*>(sm.ring[slot]) + odd + lane;
-            float2 (*red)[kRedPitch] = WS::kRedInRing ? reinterpret_cast<float2 (*)[kRedPitch]>(sm.ring[slot]) : sm.red;
-
+            // ---- integer input: a piece that the integers cover completely (all but the first and last of a channel) is widened
+            // in registers on its way into the FIR; a boundary piece (carry samples, ragged ends) is widened in place first
+            bool int_in_loop = false;
+            if (kInt) {
+                const int A = j0 - odd + p * G::PIECE_SAMPLES;    // as in issue_piece
+                const int want_lo = A + odd, want_hi = want_lo + G::PIECE_SAMPLES;
+                const int lo = max(A, j_cap_lo);
+                const int hi = min(A + G::PIECE_SAMPLES + (odd ? kG : 0), j_end);
+                const int hi2 = max(hi & ~(kG - 1), lo);
+                int_in_loop = A >= 0 && hi2 >= want_hi;
+                if (!int_in_loop) {
+                    float2* d2 = reinterpret_cast<float2*>(sm.ring[slot]);
+                    const In* q = reinterpret_cast<const In*>(sm.ring[slot] + WS::kIntOff);
+                    const int s_hi = hi2 - A;
 #pragma unroll 1
-            for (int g = 0; g < G::GROUPS_PER_PIECE; ++g) {
-#pragma unroll
-                for (int u = 0; u < G::U; ++u) {
-                    float2 x0 = src[(g * G::U + u) * 64];
-                    float2 x1 = src[(g * G::U + u) * 64 + 32];
-                    if (NCO && mix_in_loop) {
-                        x0 = nco_apply(x0, nco_phasor(ns.pq[g * G::U + u + w0], s2a, s2ar));
-                        x1 = nco_apply(x1, nco_phasor(ns.pq[g * G::U + u + w1], s2b, s2br));
+                    for (int s0 = max(lo, 0) - A; s0 < s_hi; s0 += 32) {   // ring positions delivered as integers, in place
+                        const int s = s0 + lane;
+                        float2 v = make_float2(0.f, 0.f);
+                        if (s < s_hi) v = IqFmt<F>::dq(q[s]);
+                        __syncwarp();
+                        if (s < s_hi) d2[s] = v;
                     }
-#pragma unroll
-                    for (int j = 0; j < G::NLIVE; ++j) {
-                        const int r = (j + u * G::NOUT) % G::NLIVE; // register holding live output j
-                        // tap index of position P for live output j (0-based): t = T - M*(j+1) + P; skip the
-                        // half-superblocks where no lane has a tap (compile-time)
-                        const int t0 = T - M * (j + 1);
-                        if (t0 + 31 >= 0 && t0 < T) acc[r] = cfma(x0, h0[j], acc[r]);
-                        if (t0 + 63 >= 0 && t0 + 32 < T) acc[r] = cfma(x1, h1[j], acc[r]);
-                    }
-#pragma unroll
-                    for (int j = 0; j < G::NOUT; ++j) {
-                        const int r = (j + u * G::NOUT) % G::NLIVE;
-                        if (G::NOUT == 1) {
-                            if (WS::kRedInRing) __syncwarp();     // every lane has read superblock (g*U+u) of the slot
-                            red[g * G::U + u][lane] = acc[r];               // row = superblock within the piece
-                        } else {
-                            sm.red[staged][lane] = acc[r];
-                            if (++staged == 16) { reduce_rows(sm.red, 16, k_next + j - 15, k_lo, k_hi, out, lane); staged = 0; }
+                    __syncwarp();
+                    if (lo > want_lo || hi2 < want_hi) {   // what the bulk copies did not deliver, as in the cf32 kernel
+                        for (int j = want_lo + lane; j < want_hi; j += 32) {
+                            if (j >= lo && j < hi2) continue;
+                            d2[j - A] = (j >= lo && j < hi) ? sample(j) : make_float2(0.f, 0.f);
                         }
-                        acc[r] = make_float2(0.f, 0.f);
                     }
-                    if (G::NOUT > 1) k_next += G::NOUT;
+                    __syncwarp();
                 }
             }
+            const float2* src = reinterpret_cast<const float2*>(sm.ring[slot]) + odd + lane;
+            const In* qsrc = reinterpret_cast<const In*>(sm.ring[slot] + WS::kIntOff) + odd + lane;
+            float2 (*red)[kRedPitch] = WS::kRedInRing ? reinterpret_cast<float2 (*)[kRedPitch]>(sm.ring[slot]) : sm.red;
+
+            // the FIR over the piece; `load(i)` yields sample i of it (the branch on the input path is taken once per piece)
+            auto fir_piece = [&](auto load) {
+#pragma unroll 1
+                for (int g = 0; g < G::GROUPS_PER_PIECE; ++g) {
+#pragma unroll
+                    for (int u = 0; u < G::U; ++u) {
+                        float2 x0 = load((g * G::U + u) * 64);
+                        float2 x1 = load((g * G::U + u) * 64 + 32);
+                        if (NCO && mix_in_loop) {
+                            x0 = nco_apply(x0, nco_phasor(ns.pq[g * G::U + u + w0], s2a, s2ar));
+                            x1 = nco_apply(x1, nco_phasor(ns.pq[g * G::U + u + w1], s2b, s2br));
+                        }
+#pragma unroll
+                        for (int j = 0; j < G::NLIVE; ++j) {
+                            const int r = (j + u * G::NOUT) % G::NLIVE; // register holding live output j
+                            // tap index of position P for live output j (0-based): t = T - M*(j+1) + P; skip the
+                            // half-superblocks where no lane has a tap (compile-time)
+                            const int t0 = T - M * (j + 1);
+                            if (t0 + 31 >= 0 && t0 < T) acc[r] = cfma(x0, h0[j], acc[r]);
+                            if (t0 + 63 >= 0 && t0 + 32 < T) acc[r] = cfma(x1, h1[j], acc[r]);
+                        }
+#pragma unroll
+                        for (int j = 0; j < G::NOUT; ++j) {
+                            const int r = (j + u * G::NOUT) % G::NLIVE;
+                            if (G::NOUT == 1) {
+                                if (WS::kRedInRing) __syncwarp();     // every lane has read superblock (g*U+u) of the slot
+                                red[g * G::U + u][lane] = acc[r];               // row = superblock within the piece
+                            } else {
+                                sm.red[staged][lane] = acc[r];
+                                if (++staged == 16) { reduce_rows(sm.red, 16, k_next + j - 15, k_lo, k_hi, out, lane); staged = 0; }
+                            }
+                            acc[r] = make_float2(0.f, 0.f);
+                        }
+                        if (G::NOUT > 1) k_next += G::NOUT;
+                    }
+                }
+            };
+            if (kInt && int_in_loop) fir_piece([&](int i) { return IqFmt<F>::dq(qsrc[i]); });
+            else fir_piece([&](int i) { return src[i]; });
             if (G::NOUT == 1) {
                 reduce_rows(red, G::PSB, k_next, k_lo, k_hi, out, lane);
                 k_next += G::PSB;
@@ -482,7 +540,7 @@ decim1_kernel(DecimArgs a)
             }
             for (int i = lane; i < keep; i += 32) {
                 const int j = jn - keep + i;
-                float2 v = (j < 0) ? carry[j] : chunk[j];
+                float2 v = (j < 0) ? carry[j] : IqFmt<F>::dq(chunk[j]);
                 if (NCO && mixing && j >= 0) { // the carry holds MIXED samples: same phasor as above
                     const float2 s2 = ns.s2[j & 63];
                     v = nco_apply(v, nco_phasor(nco_f4(nco_cmul(ns.e[(j >> 12) - ebase], ns.s1[(j >> 6) & 63])), s2, make_float2(-s2.y, s2.x)));
@@ -555,19 +613,20 @@ cudaError_t launch_carry(const ChanPlan* plan, ChanPlan uplan, int uniform, cons
 
 constexpr int kMinSpan = 48; // superblocks: keeps the ramp-in below ~12 % when there are few channels
 
-template <int M, int T, bool NCO = false>
+template <int M, int T, bool NCO = false, int F = HBD_IQ_CF32>
 static cudaError_t launch_fast(DecimArgs a, unsigned max_n1, int n_sms, cudaStream_t stream, int* launches)
 {
     constexpr int kWarps = K1Cfg<NCO>::kWarps;
     using G = Geo<M, T, K1Cfg<NCO>::kPsbMin>;
-    const size_t smem = sizeof(WarpSmem<M, T, K1Cfg<NCO>::kPsbMin, K1Cfg<NCO>::kSt>) * kWarps + (NCO ? sizeof(NcoWarpSmem) * kWarps : 0);
+    const size_t smem = sizeof(WarpSmem<M, T, K1Cfg<NCO>::kPsbMin, K1Cfg<NCO>::kSt, 16 / int(sizeof(typename IqFmt<F>::T))>) * kWarps +
+                        (NCO ? sizeof(NcoWarpSmem) * kWarps : 0);
     static bool configured = false; // one device per process (one process per GPU)
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(decim1_kernel<M, T, NCO>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(decim1_kernel<M, T, NCO, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
         // all kernels of the path ask for the same (maximum) shared-memory carve-out so that the low-priority tail kernels
         // can co-reside with K1 on an SM instead of forcing a carve-out reconfiguration
-        cudaFuncSetAttribute(decim1_kernel<M, T, NCO>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        cudaFuncSetAttribute(decim1_kernel<M, T, NCO, F>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
         configured = true;
     }
     a.sb_per_channel = max_n1 ? int((max_n1 - 1 + G::NOUT - 1) / G::NOUT + 1) : 1;
@@ -579,13 +638,22 @@ static cudaError_t launch_fast(DecimArgs a, unsigned max_n1, int n_sms, cudaStre
     const long long n_spans = (total_sb + span - 1) / span;
     int grid = (int)std::min<long long>(n_sms, (n_spans + kWarps - 1) / kWarps);
     if (grid < 1) grid = 1;
-    decim1_kernel<M, T, NCO><<<grid, kWarps * 32, smem, stream>>>(a);
+    decim1_kernel<M, T, NCO, F><<<grid, kWarps * 32, smem, stream>>>(a);
     if (launches) ++*launches;
     return cudaGetLastError();
 }
 
-cudaError_t launch_decim1(DecimArgs a, int M, int T, unsigned max_n1, int n_sms, cudaStream_t stream, int* launches)
+cudaError_t launch_decim1(DecimArgs a, int M, int T, unsigned max_n1, int n_sms, cudaStream_t stream, int* launches, int format)
 {
+    if (format != HBD_IQ_CF32) {   // integer input read natively: the /64 first stage only (decim1_supports_native_iq)
+        if (a.nco || !decim1_supports_native_iq(M, T)) return cudaErrorInvalidValue;
+        switch (format) {
+        case HBD_IQ_CS16: return launch_fast<64, 348, false, HBD_IQ_CS16>(a, max_n1, n_sms, stream, launches);
+        case HBD_IQ_CS8: return launch_fast<64, 348, false, HBD_IQ_CS8>(a, max_n1, n_sms, stream, launches);
+        case HBD_IQ_CU8: return launch_fast<64, 348, false, HBD_IQ_CU8>(a, max_n1, n_sms, stream, launches);
+        default: return cudaErrorInvalidValue;
+        }
+    }
     if (a.nco) {   // fused NCO: only the /64 first stage has it (decim1_supports_fused_nco)
         if (M == 64 && T == 348) return launch_fast<64, 348, true>(a, max_n1, n_sms, stream, launches);
         return cudaErrorInvalidValue;
@@ -608,5 +676,6 @@ cudaError_t launch_decim1(DecimArgs a, int M, int T, unsigned max_n1, int n_sms,
 }
 
 bool decim1_supports_fused_nco(int M, int T) { return M == 64 && T == 348; }
+bool decim1_supports_native_iq(int M, int T) { return M == 64 && T == 348; }
 
 } // namespace hbd

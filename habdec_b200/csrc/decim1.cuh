@@ -11,8 +11,8 @@ namespace hbd {
 constexpr int kDecimWarps = HBD_K1_WARPS; // warps per CTA; each warp runs its own TMA ring
 
 struct DecimArgs {
-    const float2* chunk;       // pushed samples, [channel][chunk_pitch] cf32, chunk[j] for j in [0, n)
-    size_t chunk_pitch;        // in samples, even (16-byte rows)
+    const float2* chunk;       // pushed samples, [channel][chunk_pitch] cf32 (or the integer format given to launch_decim1), chunk[j] for j in [0, n)
+    size_t chunk_pitch;        // in samples, 16-byte rows
     const float2* carry;       // [channel][carry_cap], right aligned: sample j (< 0) at carry[carry_cap + j]
     int carry_cap;             // row length of the carry buffers (>= T1 - 1 + total factor: history + unconsumed remainder)
     float2* s1;                // stage-1 output stream, [channel][s1_pitch]; outputs start at s1_hist
@@ -32,10 +32,13 @@ struct DecimArgs {
 };
 
 // M == 1 means "no decimator" (copy).  `launches` is incremented per kernel launched.  Writes the carry of the
-// next call into a.carry_next (inside K1 on the fast path, by carry_kernel otherwise).
-cudaError_t launch_decim1(DecimArgs a, int M, int T, unsigned max_n1, int n_sms, cudaStream_t stream, int* launches);
+// next call into a.carry_next (inside K1 on the fast path, by carry_kernel otherwise).  `format` (HBD_IQ_*) is that of
+// a.chunk; an integer format needs decim1_supports_native_iq and no NCO.  The carry is cf32 whatever the format.
+cudaError_t launch_decim1(DecimArgs a, int M, int T, unsigned max_n1, int n_sms, cudaStream_t stream, int* launches, int format = 0);
 // can launch_decim1 mix the channels through their NCOs itself (DecimArgs::nco) for this first stage?
 bool decim1_supports_fused_nco(int M, int T);
+// can launch_decim1 read integer input (CS16 / CS8 / CU8) itself for this first stage?
+bool decim1_supports_native_iq(int M, int T);
 // stage-1 carry (history + unconsumed remainder) for the next call: carry -> carry_next
 cudaError_t launch_carry(const ChanPlan* plan, ChanPlan uplan, int uniform, const float2* chunk, size_t chunk_pitch, const float2* carry, float2* carry_next, int T1, int ch0,
                          int n_channels, int carry_cap, cudaStream_t stream, int* launches);

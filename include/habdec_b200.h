@@ -91,6 +91,26 @@ int hbd_push_samples_batch(hbd_decoder* h, const float* iq, size_t n_complex, si
  * unchanged until the next hbd_process()/hbd_process_async() has completed (hbd_synchronize) */
 int hbd_push_samples_device(hbd_decoder* h, const float* d_iq, size_t n_complex, size_t pitch_complex, double sampling_rate);
 
+/* ---- integer IQ input (what receivers deliver; the reference gets cf32 from SoapySDR's CPU conversion) ---------------
+ * I, Q interleaved, little endian.  The decoder sees the dequantised value, exactly representable in float32:
+ *   HBD_IQ_CF32  8 B / sample   as is
+ *   HBD_IQ_CS16  4 B / sample   v / 32768          (Airspy, SDRplay, SoapySDR "CS16")
+ *   HBD_IQ_CS8   2 B / sample   v / 128            (HackRF)
+ *   HBD_IQ_CU8   2 B / sample   (v - 128) / 128    (RTL-SDR, rtl_sdr .cu8 files)
+ * so an integer push is bit for bit the cf32 push of its dequantised values.  CU8 is mapped exactly (CS8 of v ^ 0x80), not
+ * re-centred: a receiver's DC offset is left to dc_remove and the NCO.  The format may change from one push to the next.
+ * The five entries below mirror the cf32 ones (same rules for pending host / device pushes, queue depths and device
+ * pointer lifetime); n and pitch count complex samples; HBD_IQ_CF32 makes them exactly the cf32 entry points.  Integer
+ * data crosses PCIe and HBM as integers: with the /64 first stage (factor 256) and no NCO set, the decimator reads a
+ * device push in place; every other path widens on the GPU into the cf32 buffers the cf32 push would have used.
+ * Device matrices: 16-byte aligned, pitch * bytes a multiple of 16.  Unknown format / misalignment: HBD_ERR_ARG. */
+enum hbd_iq_format { HBD_IQ_CF32 = 0, HBD_IQ_CS16 = 1, HBD_IQ_CS8 = 2, HBD_IQ_CU8 = 3 };
+int hbd_push_iq(hbd_decoder* h, int ch, const void* iq, int format, size_t n_complex, double sampling_rate);
+int hbd_push_iq_batch(hbd_decoder* h, const void* iq, int format, size_t n_complex, size_t pitch_complex, double sampling_rate);
+int hbd_push_iq_device(hbd_decoder* h, const void* d_iq, int format, size_t n_complex, size_t pitch_complex, double sampling_rate);
+int hbd_push_iq_wideband(hbd_decoder* h, const void* iq, int format, size_t n_complex, double sampling_rate);
+int hbd_push_iq_wideband_device(hbd_decoder* h, const void* d_iq, int format, size_t n_complex, double sampling_rate);
+
 /* ---- NCO pre-mixer (new; the reference retunes the SDR instead: websocketServer/main.cpp:247-265) -----------
  * Channel `ch` (-1: all) is mixed down by freq_hz before the decimator: x[i] * exp(-2 pi i f t), phase kept in
  * float64 and continuous across pushes and frequency changes.  With it, one wideband capture can feed many

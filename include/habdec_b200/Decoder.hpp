@@ -81,10 +81,16 @@ public:
     bool pushSamples(int ch, const IQVector& v) { return hbd_push_samples(h_, ch, reinterpret_cast<const float*>(v.data()), v.size(), v.samplingRate()) == HBD_OK; }
     bool pushSamples(const std::complex<float>* host_matrix, size_t n, size_t pitch, double fs) { return hbd_push_samples_batch(h_, reinterpret_cast<const float*>(host_matrix), n, pitch, fs) == HBD_OK; }
     bool pushSamplesDevice(const void* device_matrix, size_t n, size_t pitch, double fs) { return hbd_push_samples_device(h_, static_cast<const float*>(device_matrix), n, pitch, fs) == HBD_OK; }
+    // the same from integer IQ (CS16 / CS8 / CU8 as receivers deliver it; n, pitch in complex samples)
+    bool pushSamples(int ch, const void* iq, hbd_iq_format format, size_t n, double fs) { return hbd_push_iq(h_, ch, iq, format, n, fs) == HBD_OK; }
+    bool pushSamples(const void* host_matrix, hbd_iq_format format, size_t n, size_t pitch, double fs) { return hbd_push_iq_batch(h_, host_matrix, format, n, pitch, fs) == HBD_OK; }
+    bool pushSamplesDevice(const void* device_matrix, hbd_iq_format format, size_t n, size_t pitch, double fs) { return hbd_push_iq_device(h_, device_matrix, format, n, pitch, fs) == HBD_OK; }
 
     // one wideband capture for all channels, each through its own NCO (frequency-offset channels)
     bool pushWideband(const IQVector& v) { return hbd_push_wideband(h_, reinterpret_cast<const float*>(v.data()), v.size(), v.samplingRate()) == HBD_OK; }
     bool pushWidebandDevice(const void* device_row, size_t n, double fs) { return hbd_push_wideband_device(h_, static_cast<const float*>(device_row), n, fs) == HBD_OK; }
+    bool pushWideband(const void* row, hbd_iq_format format, size_t n, double fs) { return hbd_push_iq_wideband(h_, row, format, n, fs) == HBD_OK; }
+    bool pushWidebandDevice(const void* device_row, hbd_iq_format format, size_t n, double fs) { return hbd_push_iq_wideband_device(h_, device_row, format, n, fs) == HBD_OK; }
     // NCO pre-mixer: replaces the SDR retune of code/websocketServer/main.cpp:247-265
     void nco(double freq_hz, int ch = -1) { hbd_set_nco(h_, ch, freq_hz); }
     double nco(int ch) const { return hbd_get_nco(h_, ch); }
@@ -223,6 +229,7 @@ class Decoder {
 public:
     explicit Decoder(int cuda_device = 0) : b_(1, cuda_device) {}
     bool pushSamples(const IQVector& v) { return b_.pushSamples(0, v); }
+    bool pushSamples(const void* iq, hbd_iq_format format, size_t n, double fs) { return b_.pushSamples(0, iq, format, n, fs); }   // integer IQ
     void lowpass_bw(float v) { b_.lowpass_bw(v, 0); }
     float lowpass_bw() const { return b_.lowpass_bw(0); }
     void lowpass_trans(float v) { b_.lowpass_trans(v, 0); }
