@@ -89,6 +89,14 @@ class ResultRecord(C.Structure):
 
 RECORD_BYTES = C.sizeof(ResultRecord)
 
+
+class ScanParams(C.Structure):
+    _fields_ = [("min_snr_db", C.c_double), ("min_shift_hz", C.c_double), ("max_shift_hz", C.c_double), ("max_tone_ratio_db", C.c_double)]
+
+
+class ScanSignal(C.Structure):
+    _fields_ = [("center_hz", C.c_double), ("shift_hz", C.c_double), ("snr_db", C.c_double), ("bin_lo", C.c_int), ("bin_hi", C.c_int)]
+
 TELEMETRY_CB = C.CFUNCTYPE(None, C.c_void_p, C.c_int, C.POINTER(Telemetry), C.c_char_p)
 SSDV_CB = C.CFUNCTYPE(None, C.c_void_p, C.c_int, C.POINTER(SsdvPacketInfo), C.POINTER(C.c_ubyte))
 SENTENCE_CB = C.CFUNCTYPE(None, C.c_void_p, C.c_int, C.c_char_p, C.c_char_p, C.c_char_p)
@@ -212,6 +220,17 @@ SIGNATURES = {
     "hbd_tracker_stats_payload": (C.c_size_t, [C.c_void_p, C.c_int, C.c_int, C.c_char_p, C.c_size_t]),
     "hbd_tracker_get_sentence": (C.c_size_t, [C.c_void_p, C.c_int, C.c_int, C.c_char_p, C.c_size_t]),
     "hbd_attach_tracker": (C.c_int, [_H, C.c_void_p, C.c_int]),
+    "hbd_scanner_create": (C.c_int, [C.c_int, C.c_size_t, C.POINTER(C.c_void_p)]),
+    "hbd_scanner_destroy": (None, [C.c_void_p]),
+    "hbd_scanner_last_error": (C.c_char_p, [C.c_void_p]),
+    "hbd_scanner_set_stream": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "hbd_scan_push": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_size_t, C.c_double]),
+    "hbd_scan_push_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_size_t, C.c_double]),
+    "hbd_scan_reset": (C.c_int, [C.c_void_p]),
+    "hbd_scan_get_psd": (C.c_size_t, [C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_ulonglong)]),
+    "hbd_scan_default_params": (None, [C.POINTER(ScanParams)]),
+    "hbd_scan_find": (C.c_int, [C.c_void_p, C.POINTER(ScanParams), C.c_void_p, C.c_size_t]),
+    "hbd_scan_detect": (C.c_int, [C.c_void_p, C.c_size_t, C.c_double, C.POINTER(ScanParams), C.c_void_p, C.c_size_t]),
     "hbd_debug_stage": (C.c_size_t, [_H, C.c_int, C.c_int, C.c_void_p, C.c_size_t]),
     "hbd_design_lowpass": (C.c_size_t, [C.c_float, C.c_float, C.c_size_t, C.c_size_t, C.c_void_p, C.c_size_t]),
     "hbd_extract_sentence": (C.c_int, [C.c_char_p, C.c_size_t, C.c_char_p, C.c_char_p, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]),
@@ -475,6 +494,109 @@ class Tracker:
         buf = C.create_string_buffer(1200)
         n = self._lib.hbd_tracker_get_sentence(self._t, ch, int(frame), buf, 1200)
         return buf.value if n else b""
+
+
+# ---- wideband scanner (hbd_scanner / hbd_scan_*): where the RTTY payloads of a capture are -------------------------
+def scan_default_params() -> dict:
+    p = ScanParams()
+    load().hbd_scan_default_params(C.byref(p))
+    return {name: getattr(p, name) for name, _ in ScanParams._fields_}
+
+
+def _scan_params(params: dict):
+    if not params:
+        return None
+    p = ScanParams(**scan_default_params())
+    for k, v in params.items():
+        if k not in scan_default_params():
+            raise TypeError("unknown scan parameter %r" % k)
+        setattr(p, k, float(v))
+    return C.byref(p)
+
+
+def _scan_signals(call) -> list[dict]:
+    arr = (ScanSignal * 16)()
+    n = call(arr, len(arr))
+    if n > len(arr):                  # more than the first guess: once more with room for all
+        arr = (ScanSignal * n)()
+        n = call(arr, n)
+    if n < 0:
+        raise HbdError("scan detection failed (%d)" % n)
+    return [{"center_hz": x.center_hz, "shift_hz": x.shift_hz, "snr_db": x.snr_db, "bin_lo": x.bin_lo, "bin_hi": x.bin_hi} for x in arr[:n]]
+
+
+def scan_detect(psd, fs: float, **params) -> list[dict]:
+    """Tone pairs in an fft-shifted float32 PSD (hbd_scan_detect, host only); params as hbd_scan_params (defaults when absent)."""
+    psd = np.ascontiguousarray(psd, dtype=np.float32)
+    lib, p = load(), _scan_params(params)
+    return _scan_signals(lambda out, cap: lib.hbd_scan_detect(psd.ctypes.data, psd.size, float(fs), p, out, cap))
+
+
+class Scanner:
+    """Averaged GPU spectrum of a wideband capture and the RTTY tone pairs in it (hbd_scanner).  Offsets are relative to the
+    capture centre, in the units BatchDecoder.set_nco takes."""
+
+    def __init__(self, n_fft: int, device: int = 0):
+        self._lib = load()
+        h = C.c_void_p()
+        rc = self._lib.hbd_scanner_create(int(device), int(n_fft), C.byref(h))
+        if rc != HBD_OK:
+            raise HbdError("hbd_scanner_create failed (%d): n_fft must be a power of two in [4096, 2^20], and a CUDA device "
+                           "(B200, sm_100a) is required" % rc)
+        self._s = h
+        self.n_fft = int(n_fft)
+        self.fs = None
+
+    def close(self):
+        if getattr(self, "_s", None):
+            self._lib.hbd_scanner_destroy(self._s)
+            self._s = None
+
+    __del__ = close
+
+    def _chk(self, rc):
+        if rc != HBD_OK:
+            raise HbdError("habdec_b200 scanner error %d: %s" % (rc, (self._lib.hbd_scanner_last_error(self._s) or b"").decode()))
+
+    def set_stream(self, cuda_stream_ptr: int): self._chk(self._lib.hbd_scanner_set_stream(self._s, cuda_stream_ptr))
+
+    def push(self, iq, fs: float, fmt: int = IQ_CF32):
+        """iq: complex64 [n] (IQ_CF32) or interleaved integers [2n] of the format's dtype"""
+        if fmt == IQ_CF32:
+            arr = np.ascontiguousarray(iq, dtype=np.complex64)
+            n = arr.size
+        else:
+            arr = BatchDecoder._iq_arr(iq, fmt, 1)
+            n = arr.size // 2
+        self._chk(self._lib.hbd_scan_push(self._s, arr.ctypes.data, int(fmt), n, float(fs)))
+        self.fs = float(fs)
+
+    def push_device(self, ptr: int, n: int, fs: float, fmt: int = IQ_CF32):
+        self._chk(self._lib.hbd_scan_push_device(self._s, ptr, int(fmt), int(n), float(fs)))
+        self.fs = float(fs)
+
+    def reset(self):
+        self._chk(self._lib.hbd_scan_reset(self._s))
+        self.fs = None
+
+    def psd(self):
+        """(float32 [n_fft] fft-shifted PSD, segments averaged)"""
+        out = np.empty(self.n_fft, dtype=np.float32)
+        seg = C.c_ulonglong(0)
+        if self._lib.hbd_scan_get_psd(self._s, out.ctypes.data, out.size, C.byref(seg)) != self.n_fft:
+            raise HbdError("hbd_scan_get_psd failed: %s" % (self._lib.hbd_scanner_last_error(self._s) or b"").decode())
+        return out, seg.value
+
+    def freqs(self) -> np.ndarray:
+        """Offset of every PSD bin from the capture centre in Hz (needs the sampling rate of a push)."""
+        if self.fs is None:
+            raise HbdError("no sampling rate latched yet: push first")
+        return (np.arange(self.n_fft, dtype=np.float64) - self.n_fft // 2) * (self.fs / self.n_fft)
+
+    def find(self, **params) -> list[dict]:
+        """[{center_hz, shift_hz, snr_db, bin_lo, bin_hi}] sorted by center_hz"""
+        p = _scan_params(params)
+        return _scan_signals(lambda out, cap: self._lib.hbd_scan_find(self._s, p, out, cap))
 
 
 class BatchDecoder:

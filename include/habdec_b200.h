@@ -333,6 +333,50 @@ size_t hbd_tracker_get_sentence(hbd_tracker* t, int ch, int frame, char* out, si
  * after the sentence callback; NULL detaches */
 int    hbd_attach_tracker(hbd_decoder* h, hbd_tracker* t, int ch_offset);
 
+/* ---- wideband scanner (new; in the reference a person reads the spectrum and retunes the radio) ----------------
+ * Finds 2-FSK (RTTY) payloads in a wideband capture and reports them as offsets from the capture centre, in the units
+ * hbd_set_nco takes: hbd_set_nco(h, ch, sig.center_hz) puts a found signal at 0 Hz in channel ch.  Independent of
+ * hbd_decoder; to scan the capture a decoder reads, give both the same stream and push the capture to both.
+ *
+ * Spectrum: N = n_fft (a power of two, 4096 .. 1048576), segments [s N/2, s N/2 + N) of the samples pushed since the last
+ * reset (a segment is used once all its samples have arrived; samples wait across pushes), 4-term Blackman-Harris window
+ * w (habdec_windows.h:27-53), P[k] = sum_s |X_s[k]|^2 / (S sum_n w[n]^2) with |X_s|^2 in float32 and the sum over
+ * segments in float64, in segment order: the result does not depend on how the capture was cut into pushes.  Returned
+ * fft-shifted as float32 (bin i = frequency (i - N/2) fs / N, the orientation of hbd_get_fft).  Integer formats are
+ * dequantised exactly like a decoder push, so an integer push gives the PSD of the cf32 push of its dequantised values.
+ * The first push latches fs; a push at another rate fails with HBD_ERR_STATE until hbd_scan_reset, which also clears
+ * the spectrum and the waiting samples.  A device capture (16-byte aligned) is read in place by work enqueued on the
+ * scanner's stream: it must stay valid and unchanged until that work has completed (work put on the stream later is
+ * ordered behind it).  A host push returns when the caller owns `iq` again.  All entry points take the scanner's mutex.
+ *
+ * Detection (hbd_scan_find on the scanner's PSD, hbd_scan_detect on any PSD; host, float64): noise floor nf = lower
+ * median of the 1024-bin block holding a bin; a tone candidate is a bin with P >= nf 10^(min_snr_db/10) that is the first
+ * maximum of P within +-max(1, floor(min_shift_hz / (2 fs/N))) bins.  Strongest candidate first, each takes as partner
+ * the strongest unused candidate between min_shift_hz and max_shift_hz away whose power is within max_tone_ratio_db of
+ * its own; a pair uses up every candidate within one shift of it.  Detection is promised for baud <= shift only: faster
+ * keying leaves no separate tones.  Signals come sorted by center_hz. */
+typedef struct hbd_scanner hbd_scanner;
+typedef struct hbd_scan_params {
+    double min_snr_db, min_shift_hz, max_shift_hz, max_tone_ratio_db;   /* defaults 10, 150, 1200, 15 */
+} hbd_scan_params;
+typedef struct hbd_scan_signal {
+    double center_hz, shift_hz, snr_db;   /* (f_a + f_b) / 2, |f_b - f_a|, 10 log10 min(P_a / nf_a, P_b / nf_b) */
+    int    bin_lo, bin_hi;                /* the two tones' bins in the fft-shifted PSD */
+} hbd_scan_signal;
+int    hbd_scanner_create(int cuda_device, size_t n_fft, hbd_scanner** out);
+void   hbd_scanner_destroy(hbd_scanner* s);
+const char* hbd_scanner_last_error(hbd_scanner* s);
+int    hbd_scanner_set_stream(hbd_scanner* s, void* cuda_stream);   /* share a decoder's stream to scan the same device capture */
+int    hbd_scan_push(hbd_scanner* s, const void* iq, int format, size_t n_complex, double sampling_rate);
+int    hbd_scan_push_device(hbd_scanner* s, const void* d_iq, int format, size_t n_complex, double sampling_rate);
+int    hbd_scan_reset(hbd_scanner* s);
+/* copies min(cap, N) floats of the PSD (zeros before the first complete segment); *n_segments = S; returns N */
+size_t hbd_scan_get_psd(hbd_scanner* s, float* out, size_t cap_floats, unsigned long long* n_segments);
+void   hbd_scan_default_params(hbd_scan_params* p);
+/* signals found (may exceed cap; the first cap are stored), < 0 on error; p NULL = defaults */
+int    hbd_scan_find(hbd_scanner* s, const hbd_scan_params* p, hbd_scan_signal* out, size_t cap);
+int    hbd_scan_detect(const float* psd, size_t n, double fs, const hbd_scan_params* p, hbd_scan_signal* out, size_t cap);   /* host only */
+
 /* ---- test hooks ------------------------------------------------------------------------------------------ */
 enum { HBD_STAGE_DECIMATED = 0, HBD_STAGE_FILTERED = 1, HBD_STAGE_DEMOD = 2, HBD_STAGE_LPTAPS = 5,
        HBD_STAGE_PENDING = 6, HBD_STAGE_BITS = 7 };
