@@ -132,6 +132,19 @@ struct Deferred {
 // what one thread of the drain records for its channel range (collect_locked)
 struct ReplayPart { std::vector<std::pair<unsigned, Deferred>> events; bool spilled = false; };
 
+// the samples of one hbd_push_* call (hbd_decoder::push)
+struct PushSrc {
+    enum Shape { kChannel, kMatrix, kRow };   // one channel's samples, [n_ch][pitch], one wideband row for all channels
+    const void* p;
+    bool device;
+    int format;     // HBD_IQ_*
+    Shape shape;
+    int ch;         // kChannel
+    size_t pitch;   // kMatrix, in samples
+    size_t n;
+    double fs;
+};
+
 struct hbd_decoder {
     std::mutex mtx;
     std::string err;
@@ -249,24 +262,23 @@ struct hbd_decoder {
     float2* d_rec_dec = nullptr; float2* d_rec_filt = nullptr; size_t rec_pitch = 0;
     unsigned char* d_rec_bits = nullptr; unsigned* d_rec_bits_n = nullptr; unsigned rec_bits_pitch = 0;
 
-    // input
+    // input (push)
     float2* d_stage = nullptr; size_t stage_pitch = 0;   // host pushes land here
-    const float2* ext = nullptr; size_t ext_pitch = 0; size_t ext_n = 0; // zero-copy device push
-    int ext_format = HBD_IQ_CF32;    // ... of integer samples that K1 reads itself (decim1_supports_native_iq); ext then points at them
-    // integer input that K1 does not read natively: host data is uploaded as integers to d_iq_up, device data is widened
-    // to cf32 into d_widen and pushed from there like a cf32 device matrix
+    // A device push that K1 reads in place at the next process call (p == nullptr: K1 reads the staging matrix).
+    // format: integers that K1 reads itself (decim1_supports_native_iq).  nco: raw samples that K1 mixes through the
+    // channels' NCOs (fused K0); pitch 0 is one wideband row shared by all channels.
+    struct DeviceInput { const void* p = nullptr; size_t pitch = 0, n = 0; int format = HBD_IQ_CF32; const NcoChan* nco = nullptr; } in;
+    int push(const PushSrc& s);
+    // Host integers are uploaded to d_iq_up.  d_widen holds cf32: widened device integers, and wideband rows that do not
+    // arrive as device cf32.
     unsigned char* d_iq_up = nullptr; size_t iq_up_bytes = 0;
     float2* d_widen = nullptr; size_t widen_bytes = 0;
-    int ensure_iq_up(size_t bytes);
-    int widen_device(const void* src, int format, size_t n, size_t pitch, size_t* out_pitch);
+    int ensure_scratch(void** p, size_t* cap, size_t bytes);
+    int widen(const void* src, size_t pitch, int format, int rows, size_t n, size_t* out_pitch);
     // fused-NCO parameter ring: pinned host slots + device slots, so a push never waits for the GPU
     static constexpr unsigned kNcoSlots = 16;
     NcoChan* h_nco_pin = nullptr; NcoChan* d_nco_ring = nullptr; cudaEvent_t ev_nco[kNcoSlots] = {}; unsigned nco_seq = 0;
-    const NcoChan* ext_nco_ptr = nullptr;
-    bool ext_nco = false;    // ... of RAW samples that K1 mixes through the channels' NCOs itself (fused K0; ext_pitch 0 = wideband row)
     bool nco_fused = true;   // HBD_NCO_FUSED=0 (measurement / test hook): always pre-mix with K0 into the staging matrix
-    int push_fused_nco(const float2* src, size_t pitch, size_t n);
-    float* h_pinned = nullptr; size_t pinned_bytes = 0;  // staging for pageable host memory
 
     // websocket wire formats (wire.cu)
     bool demod_acc_on = false;
@@ -277,9 +289,8 @@ struct hbd_decoder {
     int ensure_dacc();
     // NCO pre-mixer (nco.cu)
     NcoChan* d_nco = nullptr; std::vector<NcoChan> h_nco;
-    float2* d_wide = nullptr; size_t wide_cap = 0;       // wideband capture row shared by all channels
     bool nco_any = false;    // some channel has (had) a non-zero NCO frequency or phase (set by hbd_set_nco, never cleared)
-    bool nco_active() const { return nco_any; }
+    void nco_params(NcoChan* out, int c0, int nc, size_t n, bool k0_rotation);
     int mix_into_stage(const void* src, size_t src_pitch, int c0, int nc, size_t dst_off, size_t n, int format = HBD_IQ_CF32);
     int pending_marks = 0;   // async calls since the last collect
     int sv_override = -1;
@@ -544,10 +555,9 @@ void hbd_decoder::free_all()
     if (ev_in) cudaEventDestroy(ev_in);
     void* ptrs[] = {d_state, d_plan, d_carry2[0], d_carry2[1], d_s1x[0], d_s1x[1], d_decq, d_fftbuf, d_spectrum, d_power, d_lptaps, d_slicer, d_demod, d_uart_runs, d_maskc, d_log, d_log_ctl,
                     d_taps1, d_taps2, d_twiddle, d_cfg_baud, d_cfg_stops, d_cfg_bits, d_cfg_dc, d_cfg_ntaps,
-                    d_cfg_dirty, d_rec_dec, d_rec_filt, d_rec_bits, d_rec_bits_n, d_stage, d_nco, d_wide, d_iq_up, d_widen, d_dacc, d_dacc_n, d_frames, d_frame_sizes,
+                    d_cfg_dirty, d_rec_dec, d_rec_filt, d_rec_bits, d_rec_bits_n, d_stage, d_nco, d_iq_up, d_widen, d_dacc, d_dacc_n, d_frames, d_frame_sizes,
                     d_ssdv_ring, d_ssdv_total, d_ssdv_scanned, d_ssdv_log};
     for (void* p : ptrs) if (p) cudaFree(p);
-    if (h_pinned) cudaFreeHost(h_pinned);
     for (MidStage& m : mids) { if (m.d_taps) cudaFree(m.d_taps); if (m.d_out) cudaFree(m.d_out); }
     for (int i = 0; i < 2; ++i) if (d_midlast[i]) cudaFree(d_midlast[i]);
     if (dist_ctx) { internal_free_dist(dist_ctx); dist_ctx = nullptr; }
@@ -733,7 +743,7 @@ int hbd_decoder::process_async_locked()
     ChanPlan uplan{};
     if (uni) {
         ChanStep st;
-        const unsigned pushed = ext ? unsigned(ext_n) : hc[0].pushed;
+        const unsigned pushed = in.p ? unsigned(in.n) : hc[0].pushed;
         max_total = size_t(hc[0].in_r) + pushed;
         if (max_total > cap_n_in || !d_s1x[0]) { if (quiesce()) return HBD_ERR_CUDA; }   // buffers are about to be reallocated
         { const int rc = ensure_call_capacity(max_total); if (rc) return rc; }
@@ -768,13 +778,13 @@ int hbd_decoder::process_async_locked()
         }
     } else {
         h_plan.resize(n);
-        for (size_t c = 0; c < n; ++c) max_total = std::max<size_t>(max_total, size_t(hc[c].in_r) + (ext ? unsigned(ext_n) : hc[c].pushed));
+        for (size_t c = 0; c < n; ++c) max_total = std::max<size_t>(max_total, size_t(hc[c].in_r) + (in.p ? unsigned(in.n) : hc[c].pushed));
         if (max_total > cap_n_in || !d_s1x[0]) { if (quiesce()) return HBD_ERR_CUDA; }
         { const int rc = ensure_call_capacity(max_total); if (rc) return rc; }
         for (size_t c = 0; c < n; ++c) {
             HostChan& x = hc[c];
             ChanStep st;
-            const int rc = step_channel(this, x, ext ? unsigned(ext_n) : x.pushed, st, new_taps);
+            const int rc = step_channel(this, x, in.p ? unsigned(in.n) : x.pushed, st, new_taps);
             if (rc) return rc;   // channels below c have been stepped: their samples are gone (documented in the header)
             h_plan[c] = st.plan;
             any_work |= !(st.plan.flags & 1u); need_k4 |= st.frame_done;
@@ -850,14 +860,14 @@ int hbd_decoder::process_async_locked()
     int sv_want = int(std::min<double>(6144.0, 16.0 * max_spb_c + double(max_nf) + 64.0));
     if (sv_override >= 0) sv_want = sv_override;   // test hook (HBD_SV_WANT): 0 forces the slicer's HBM path
 
-    if (ext && ext_format != HBD_IQ_CF32 && !decim1_supports_native_iq(M1, T1)) {   // the plan changed after an integer device push
+    if (in.p && in.format != HBD_IQ_CF32 && !decim1_supports_native_iq(M1, T1)) {   // the plan changed after a native integer push
         size_t wp = 0;
-        const int rc = widen_device(ext, ext_format, ext_n, ext_pitch, &wp);
+        const int rc = widen(in.p, in.pitch, in.format, n_ch, in.n, &wp);
         if (rc) return rc;
-        ext = d_widen; ext_pitch = wp; ext_format = HBD_IQ_CF32;
+        in = DeviceInput{d_widen, wp, in.n};
     }
-    const float2* chunk = ext ? ext : d_stage;
-    const size_t chunk_pitch = ext ? ext_pitch : stage_pitch;
+    const float2* chunk = in.p ? static_cast<const float2*>(in.p) : d_stage;
+    const size_t chunk_pitch = in.p ? in.pitch : stage_pitch;
     int nl = 0;
     // everything the caller (and the host-side updates above) put on `stream` happens before the kernels start
     HBD_CUDA_CHECK(cudaEventRecord(ev_in, stream));
@@ -870,9 +880,9 @@ int hbd_decoder::process_async_locked()
         da.chunk = chunk; da.chunk_pitch = chunk_pitch; da.carry = d_carry2[carry_cur]; da.carry_next = d_carry2[carry_cur ^ 1]; da.carry_cap = carry_cap;
         da.s1 = d_s1x[s1_cur]; da.s1_pitch = s1_pitch; da.s1_hist = kS1Hist;
         da.plan = d_plan; da.uplan = uplan; da.uniform = plan_uniform ? 1 : 0; da.taps = d_taps1; da.ch0 = 0; da.n_channels = n_ch;
-        da.nco = ext_nco ? ext_nco_ptr : nullptr;
+        da.nco = in.nco;
         if (timing) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_k1, ev_used_k1), hi));
-        HBD_CUDA_CHECK(launch_decim1(da, M1, T1, max_n1, n_sms, hi, &nl, ext ? ext_format : HBD_IQ_CF32));
+        HBD_CUDA_CHECK(launch_decim1(da, M1, T1, max_n1, n_sms, hi, &nl, in.format));
         if (timing) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_k1, ev_used_k1), hi));
     }
     HBD_CUDA_CHECK(cudaEventRecord(ev_consumed, hi)); // input no longer needed; stage-1 output ready
@@ -945,7 +955,7 @@ int hbd_decoder::process_async_locked()
     HBD_CUDA_CHECK(cudaEventRecord(ev_call[slot], lo)); // everything of this call is done
     ++call_seq;
     ++pending_marks;
-    ext = nullptr; ext_n = 0; ext_nco = false; ext_format = HBD_IQ_CF32;
+    in = DeviceInput{};
     return HBD_OK;
 }
 
@@ -1489,37 +1499,31 @@ size_t hbd_setup_decimation_bw(hbd_decoder* h, double max_rate)
     return h->set_plan(plan, total) == HBD_OK ? total : 0;
 }
 
-static int latch_rate(hbd_decoder* h, double fs)
+// ---- input: the hbd_push_* entry points ---------------------------------------------------------------------------------
+// NCO parameters of channels [c0, c0 + nc) for a push of n samples into out[0, nc), and the channels' phases advanced past
+// the push.  k0_rotation: also the rotation over kNcoThreads samples that K0 steps by (K1's fused mixer does not use it).
+void hbd_decoder::nco_params(NcoChan* out, int c0, int nc, size_t n, bool k0_rotation)
 {
-    if (!h->fs_in) h->fs_in = double(float(fs)); // Decoder::init(const float)
-    return HBD_OK;
-}
-
-static int ensure_stage(hbd_decoder* h, size_t need)
-{
-    if (need <= h->stage_pitch && h->d_stage) return HBD_OK;
-    const size_t np = (std::max(need, h->stage_pitch) + 15) & ~size_t(15);
-    cudaError_t e = grow_rows(&h->d_stage, &h->stage_pitch, np, size_t(h->n_ch), h->stage_pitch, h->stream);
-    if (e != cudaSuccess) { h->set_error(std::string("staging alloc: ") + cudaGetErrorString(e)); return HBD_ERR_CUDA; }
-    return HBD_OK;
-}
-
-// Mix `n` samples per channel of channels [c0, c0+nc) from src into the staging rows at dst_off and advance the
-// channels' NCO phases.  src_pitch 0: one shared (wideband) row.  Integer src (format) is widened on the way; a channel
-// without an offset is then a plain widening copy.  Runs on the handle's stream.
-int hbd_decoder::mix_into_stage(const void* src, size_t src_pitch, int c0, int nc, size_t dst_off, size_t n, int format)
-{
-    if (!n) return HBD_OK;
-    for (int c = c0; c < c0 + nc; ++c) {
-        HostChan& x = hc[size_t(c)];
-        NcoChan& k = h_nco[size_t(c)];
+    for (int i = 0; i < nc; ++i) {
+        HostChan& x = hc[size_t(c0 + i)];
+        NcoChan& k = out[i];
         k.inc = x.nco_freq / fs_in;
         k.ph0 = x.nco_phase;
         const double a = -2.0 * M_PI * k.inc * double(kNcoThreads);
-        k.step_re = std::cos(a); k.step_im = std::sin(a);
-        double ph = x.nco_phase + double(n) * k.inc;
+        k.step_re = k0_rotation ? std::cos(a) : 1.0;
+        k.step_im = k0_rotation ? std::sin(a) : 0.0;
+        const double ph = x.nco_phase + double(n) * k.inc;
         x.nco_phase = ph - std::floor(ph);
     }
+}
+
+// K0: mix `n` samples per channel of channels [c0, c0+nc) from src into the staging rows at dst_off and advance the
+// channels' NCO phases.  src_pitch 0: one shared (wideband) row.  Integer src (format) is widened on the way; a channel
+// without an offset is then a plain widening copy.  Returns once the stream has caught up.
+int hbd_decoder::mix_into_stage(const void* src, size_t src_pitch, int c0, int nc, size_t dst_off, size_t n, int format)
+{
+    if (!n) return HBD_OK;
+    nco_params(h_nco.data() + c0, c0, nc, n, true);
     HBD_CUDA_CHECK(cudaMemcpyAsync(d_nco + c0, h_nco.data() + c0, sizeof(NcoChan) * size_t(nc), cudaMemcpyHostToDevice, stream));
     int nl = 0;
     HBD_CUDA_CHECK(launch_nco_mix(src, src_pitch, d_stage, stage_pitch, dst_off, n, d_nco, c0, nc, stream, &nl, format));
@@ -1528,143 +1532,158 @@ int hbd_decoder::mix_into_stage(const void* src, size_t src_pitch, int c0, int n
     return HBD_OK;
 }
 
-// Fused form of mix_into_stage for a whole-batch device push with nothing staged: the raw samples stay where they are
-// (src_pitch 0: one wideband row), the per-channel NCO parameters go to the device and K1 mixes while it decimates
-// (decim1.cu, DecimArgs::nco) -- no K0 launch, no 8-byte write + 8-byte read per channel-sample through HBM.
-int hbd_decoder::push_fused_nco(const float2* src, size_t pitch, size_t n)
+// grow d_iq_up / d_widen to `bytes`; what they held is dropped
+int hbd_decoder::ensure_scratch(void** p, size_t* cap, size_t bytes)
 {
-    if (!h_nco_pin) {
-        HBD_CUDA_CHECK(cudaHostAlloc((void**)&h_nco_pin, sizeof(NcoChan) * size_t(n_ch) * kNcoSlots, cudaHostAllocDefault));
-        HBD_CUDA_CHECK(dalloc(&d_nco_ring, size_t(n_ch) * kNcoSlots));
-        for (unsigned i = 0; i < kNcoSlots; ++i) HBD_CUDA_CHECK(cudaEventCreateWithFlags(&ev_nco[i], cudaEventDisableTiming));
+    if (bytes <= *cap) return HBD_OK;
+    HBD_CUDA_CHECK(cudaStreamSynchronize(stream));   // a kernel of an earlier push may still read the old buffer
+    cudaFree(*p); *p = nullptr; *cap = 0;
+    HBD_CUDA_CHECK(cudaMalloc(p, bytes));
+    *cap = bytes;
+    return HBD_OK;
+}
+
+// K0 without a mixer: `rows` rows of n samples of `format` (row pitch `pitch`) -> cf32 d_widen [rows][*out_pitch] (even
+// pitch: 16-byte rows), on the stream.  Work put on the stream after a process call waits for that call's K1
+// (process_async_locked), so d_widen is free again by then.
+int hbd_decoder::widen(const void* src, size_t pitch, int format, int rows, size_t n, size_t* out_pitch)
+{
+    *out_pitch = (n + 1) & ~size_t(1);
+    { const int rc = ensure_scratch((void**)&d_widen, &widen_bytes, std::max<size_t>(size_t(rows) * *out_pitch * sizeof(float2), 256)); if (rc) return rc; }
+    int nl = 0;
+    HBD_CUDA_CHECK(launch_nco_mix(src, pitch, d_widen, *out_pitch, 0, n, nullptr, 0, rows, stream, &nl, format));
+    launches += unsigned(nl);
+    return HBD_OK;
+}
+
+// One push, whichever entry point it came through: check the arguments, then, under the mutex, the state; latch the rate
+// and take the route that gets the samples to where K1 reads them.  `base`: samples already staged in the rows pushed to.
+//
+//   source                                condition                                  route
+//   host cf32, channel / matrix           -                                          copy into staging at base; K0 in place if
+//                                                                                    the channel's NCO is set (channel) / nco_any
+//   host integers, channel / matrix       -                                          upload to d_iq_up; K0 widens (and mixes)
+//                                                                                    into staging at base
+//   device cf32 matrix                    no nco_any                                 zero copy
+//   device integer matrix                 no nco_any, decim1_supports_native_iq      zero copy, K1 reads the integers
+//   device integer matrix                 otherwise                                  K0 widens into d_widen, then the device
+//                                                                                    cf32 route on d_widen
+//   device cf32 matrix with nco_any, or   nco_fused, base == 0, n > 0, 16-byte       fused NCO: K1 mixes while it decimates (a
+//   any wideband row (a host or integer   aligned, decim1_supports_fused_nco         host row synchronises before returning)
+//   row lands in d_widen as cf32 first)   otherwise                                  K0 mixes into staging at base
+int hbd_decoder::push(const PushSrc& s)
+{
+    const size_t bytes = size_t(iq_bytes(s.format)), n = s.n;
+    const bool channel = s.shape == PushSrc::kChannel, device_matrix = s.device && s.shape == PushSrc::kMatrix;
+    if (!bytes || (channel && (s.ch < 0 || s.ch >= n_ch)) || (!s.p && (n || device_matrix))) return HBD_ERR_ARG;
+    if (s.shape == PushSrc::kMatrix && s.pitch < n) return HBD_ERR_ARG;
+    if (device_matrix && ((s.pitch * bytes) % 16 || (reinterpret_cast<uintptr_t>(s.p) & 15))) return HBD_ERR_ARG;
+
+    std::lock_guard<std::mutex> l(mtx);
+    if (in.p) { set_error("device push pending"); return HBD_ERR_STATE; }
+    HBD_CUDA_CHECK(cudaSetDevice(device));
+    const bool zero_copy = device_matrix && !nco_any;   // K1 reads the caller's matrix (or its widened copy) in place
+    unsigned base = 0;
+    if (channel) {
+        if (n_ch > 1) leave_uniform();   // per-channel feeding: the counters are stepped channel by channel from here on
+        base = hc[size_t(s.ch)].pushed;
+    } else if (!queue_depth_equal(base) || (zero_copy && base)) {
+        set_error(s.shape == PushSrc::kRow ? "wideband push needs equal queue depth in all channels"
+                  : zero_copy              ? "host push pending"
+                                           : "batch push needs equal queue depth in all channels");
+        return HBD_ERR_STATE;
     }
-    const unsigned slot = nco_seq % kNcoSlots;
-    if (nco_seq >= kNcoSlots) HBD_CUDA_CHECK(cudaEventSynchronize(ev_nco[slot]));   // the upload that last used this pinned slot (16 pushes ago)
-    ++nco_seq;
-    NcoChan* hp = h_nco_pin + size_t(slot) * size_t(n_ch);
-    for (int c = 0; c < n_ch; ++c) {
-        HostChan& x = hc[size_t(c)];
-        NcoChan& k = hp[c];
-        k.inc = x.nco_freq / fs_in;
-        k.ph0 = x.nco_phase;
-        k.step_re = 1.0; k.step_im = 0.0;   // K0's rotation, unused by K1
-        double ph = x.nco_phase + double(n) * k.inc;
-        x.nco_phase = ph - std::floor(ph);
+    if (!fs_in) fs_in = double(float(s.fs));   // Decoder::init(const float)
+    auto ensure_stage = [&] {
+        return grow_rows(&d_stage, &stage_pitch, (std::max(size_t(base) + n, stage_pitch) + 15) & ~size_t(15), size_t(n_ch), stage_pitch, stream);
+    };
+
+    if (!s.device && s.shape != PushSrc::kRow) {   // host channel / matrix: into the staging rows
+        const int c0 = channel ? s.ch : 0, rows = channel ? 1 : n_ch;
+        const bool cf32 = s.format == HBD_IQ_CF32;
+        HBD_CUDA_CHECK(ensure_stage());
+        if (!cf32 && n) { const int rc = ensure_scratch((void**)&d_iq_up, &iq_up_bytes, size_t(rows) * n * bytes); if (rc) return rc; }
+        void* dst = cf32 ? (void*)(d_stage + size_t(c0) * stage_pitch + base) : (void*)d_iq_up;   // integers cross PCIe packed [rows][n]
+        const size_t dst_pitch = cf32 ? stage_pitch * sizeof(float2) : n * bytes;
+        if (n) HBD_CUDA_CHECK(cudaMemcpy2DAsync(dst, dst_pitch, s.p, (channel ? n : s.pitch) * bytes, n * bytes, size_t(rows), cudaMemcpyHostToDevice, stream));
+        const bool mix = channel ? hc[size_t(c0)].nco_freq != 0 || hc[size_t(c0)].nco_phase != 0 : nco_any;
+        int rc = HBD_OK;
+        if (!cf32) rc = mix_into_stage(d_iq_up, channel ? 0 : n, c0, rows, base, n, s.format);
+        else if (mix) rc = mix_into_stage(d_stage + base, stage_pitch, c0, rows, base, n);   // in place
+        else HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
+        if (rc) return rc;   // either way the stream has caught up: the caller owns `p` again (Decoder.h:209-213 copies)
+        if (channel) hc[size_t(c0)].pushed += unsigned(n); else add_pushed(unsigned(n));
+        return HBD_OK;
     }
-    NcoChan* dp = d_nco_ring + size_t(slot) * size_t(n_ch);
-    HBD_CUDA_CHECK(cudaMemcpyAsync(dp, hp, sizeof(NcoChan) * size_t(n_ch), cudaMemcpyHostToDevice, stream));
-    HBD_CUDA_CHECK(cudaEventRecord(ev_nco[slot], stream));
-    ext = src; ext_pitch = pitch; ext_n = n; ext_nco = true; ext_nco_ptr = dp;
+
+    const void* src = s.p;
+    size_t pitch = s.pitch;   // 0 for a row
+    if (s.shape == PushSrc::kRow && !(s.device && s.format == HBD_IQ_CF32)) {   // the row lands in d_widen as cf32
+        const bool cf32 = s.format == HBD_IQ_CF32;
+        if (!s.device && n) {   // upload: cf32 straight into d_widen, integers into d_iq_up
+            void** up = cf32 ? (void**)&d_widen : (void**)&d_iq_up;
+            { const int rc = ensure_scratch(up, cf32 ? &widen_bytes : &iq_up_bytes, n * bytes); if (rc) return rc; }
+            HBD_CUDA_CHECK(cudaMemcpyAsync(*up, s.p, n * bytes, cudaMemcpyHostToDevice, stream));
+            src = *up;
+        }
+        if (!cf32) { size_t wp = 0; const int rc = widen(src, 0, s.format, 1, n, &wp); if (rc) return rc; }
+        src = d_widen;
+    }
+    if (device_matrix && s.format != HBD_IQ_CF32) {
+        if (zero_copy && decim1_supports_native_iq(M1, T1)) { in = DeviceInput{s.p, s.pitch, n, s.format}; return HBD_OK; }
+        const int rc = widen(s.p, s.pitch, s.format, n_ch, n, &pitch);
+        if (rc) return rc;
+        src = d_widen;
+    }
+    if (zero_copy) { in = DeviceInput{src, pitch, n}; return HBD_OK; }
+    if (nco_fused && base == 0 && n && decim1_supports_fused_nco(M1, T1) && !(reinterpret_cast<uintptr_t>(src) & 15)) {
+        // the raw samples stay where they are and K1 mixes while it decimates (decim1.cu, DecimArgs::nco): no K0 launch, no
+        // 8-byte write + 8-byte read per channel-sample through HBM.  The parameters go through a ring of pinned slots, so
+        // the push does not wait for the GPU.
+        if (!s.device) HBD_CUDA_CHECK(cudaStreamSynchronize(stream));   // the caller owns `p` again on return
+        if (!h_nco_pin) {
+            HBD_CUDA_CHECK(cudaHostAlloc((void**)&h_nco_pin, sizeof(NcoChan) * size_t(n_ch) * kNcoSlots, cudaHostAllocDefault));
+            HBD_CUDA_CHECK(dalloc(&d_nco_ring, size_t(n_ch) * kNcoSlots));
+            for (unsigned i = 0; i < kNcoSlots; ++i) HBD_CUDA_CHECK(cudaEventCreateWithFlags(&ev_nco[i], cudaEventDisableTiming));
+        }
+        const unsigned slot = nco_seq % kNcoSlots;
+        if (nco_seq >= kNcoSlots) HBD_CUDA_CHECK(cudaEventSynchronize(ev_nco[slot]));   // the upload that last used this pinned slot (16 pushes ago)
+        ++nco_seq;
+        NcoChan* hp = h_nco_pin + size_t(slot) * size_t(n_ch);
+        NcoChan* dp = d_nco_ring + size_t(slot) * size_t(n_ch);
+        nco_params(hp, 0, n_ch, n, false);
+        HBD_CUDA_CHECK(cudaMemcpyAsync(dp, hp, sizeof(NcoChan) * size_t(n_ch), cudaMemcpyHostToDevice, stream));
+        HBD_CUDA_CHECK(cudaEventRecord(ev_nco[slot], stream));
+        in = DeviceInput{src, pitch, n, HBD_IQ_CF32, dp};
+        return HBD_OK;
+    }
+    HBD_CUDA_CHECK(ensure_stage());
+    const int rc = mix_into_stage(src, pitch, 0, n_ch, base, n);
+    if (rc) return rc;
+    add_pushed(unsigned(n));
     return HBD_OK;
 }
 
 int hbd_push_samples(hbd_decoder* h, int ch, const float* iq, size_t n, double fs)
-{
-    HBD_CHECK_CH(h, ch);
-    if (!iq && n) return HBD_ERR_ARG;
-    std::lock_guard<std::mutex> l(h->mtx);
-    if (h->ext) { h->set_error("device push pending"); return HBD_ERR_STATE; }
-    if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
-    if (h->n_ch > 1) h->leave_uniform();   // per-channel feeding: the counters are stepped channel by channel from here on
-    HostChan& x = h->hc[size_t(ch)];
-    const int rc = ensure_stage(h, size_t(x.pushed) + n);
-    if (rc) return rc;
-    if (n) {
-        cudaError_t e = cudaMemcpyAsync(h->d_stage + size_t(ch) * h->stage_pitch + x.pushed, iq, n * sizeof(float2), cudaMemcpyHostToDevice, h->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream); // the caller owns `iq` again on return (Decoder.h:209-213 copies)
-        if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
-    }
-    latch_rate(h, fs);
-    if (x.nco_freq != 0 || x.nco_phase != 0) {
-        const float2* row = h->d_stage + size_t(ch) * h->stage_pitch + x.pushed;
-        const int rc2 = h->mix_into_stage(row - size_t(ch) * h->stage_pitch, h->stage_pitch, ch, 1, x.pushed, n); // in place
-        if (rc2) return rc2;
-    }
-    x.pushed += unsigned(n);
-    return HBD_OK;
-}
-
+{ return h ? h->push({iq, false, HBD_IQ_CF32, PushSrc::kChannel, ch, 0, n, fs}) : HBD_ERR_ARG; }
 int hbd_push_samples_batch(hbd_decoder* h, const float* iq, size_t n, size_t pitch, double fs)
-{
-    HBD_CHECK_H(h);
-    if ((!iq && n) || pitch < n) return HBD_ERR_ARG;
-    std::lock_guard<std::mutex> l(h->mtx);
-    if (h->ext) { h->set_error("device push pending"); return HBD_ERR_STATE; }
-    if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
-    unsigned base = 0;
-    if (!h->queue_depth_equal(base)) { h->set_error("batch push needs equal queue depth in all channels"); return HBD_ERR_STATE; }
-    const int rc = ensure_stage(h, size_t(base) + n);
-    if (rc) return rc;
-    if (n) {
-        cudaError_t e = cudaMemcpy2DAsync(h->d_stage + base, h->stage_pitch * sizeof(float2), iq, pitch * sizeof(float2), n * sizeof(float2),
-                                          size_t(h->n_ch), cudaMemcpyHostToDevice, h->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-        if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
-    }
-    latch_rate(h, fs);
-    if (h->nco_active()) {
-        const int rc2 = h->mix_into_stage(h->d_stage + base, h->stage_pitch, 0, h->n_ch, base, n); // in place
-        if (rc2) return rc2;
-    }
-    h->add_pushed(unsigned(n));
-    return HBD_OK;
-}
-
-// One capture shared by every channel (frequency-offset channels of a wideband capture): each channel receives
-// iq * exp(-2 pi i f_nco t).  `device` != 0: iq is a device pointer.
-static int push_wideband(hbd_decoder* h, const void* iq, size_t n, double fs, bool device, int format = HBD_IQ_CF32)
-{
-    HBD_CHECK_H(h);
-    const size_t bytes = size_t(iq_bytes(format));
-    if (!bytes || (!iq && n)) return HBD_ERR_ARG;
-    std::lock_guard<std::mutex> l(h->mtx);
-    if (h->ext) { h->set_error("device push pending"); return HBD_ERR_STATE; }
-    if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
-    unsigned base = 0;
-    if (!h->queue_depth_equal(base)) { h->set_error("wideband push needs equal queue depth in all channels"); return HBD_ERR_STATE; }
-    latch_rate(h, fs);
-    const float2* src = reinterpret_cast<const float2*>(iq);
-    if (!device || format != HBD_IQ_CF32) {
-        if (n > h->wide_cap) {
-            if (h->d_wide) { cudaStreamSynchronize(h->stream); cudaFree(h->d_wide); h->d_wide = nullptr; }
-            if (cudaMalloc((void**)&h->d_wide, n * sizeof(float2)) != cudaSuccess) { h->set_error("wideband buffer alloc"); return HBD_ERR_NOMEM; }
-            h->wide_cap = n;
-        }
-        if (format == HBD_IQ_CF32) {
-            cudaError_t e = cudaMemcpyAsync(h->d_wide, iq, n * sizeof(float2), cudaMemcpyHostToDevice, h->stream);
-            if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
-        } else if (n) {   // integer capture: widened once into the row every channel reads, the rest is the cf32 path
-            const void* row = iq;
-            if (!device) {
-                const int rc = h->ensure_iq_up(n * bytes);
-                if (rc) return rc;
-                cudaError_t e = cudaMemcpyAsync(h->d_iq_up, iq, n * bytes, cudaMemcpyHostToDevice, h->stream);
-                if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
-                row = h->d_iq_up;
-            }
-            int nl = 0;
-            cudaError_t e = launch_nco_mix(row, 0, h->d_wide, 0, 0, n, nullptr, 0, 1, h->stream, &nl, format);
-            h->launches += unsigned(nl);
-            if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
-        }
-        src = h->d_wide;
-    }
-    if (h->nco_fused && base == 0 && n && decim1_supports_fused_nco(h->M1, h->T1) && !(reinterpret_cast<uintptr_t>(src) & 15)) {
-        // host capture: the caller owns `iq` again on return (Decoder.h:209-213 copies), so the upload has to be complete
-        if (!device && cudaStreamSynchronize(h->stream) != cudaSuccess) return HBD_ERR_CUDA;
-        return h->push_fused_nco(src, 0, n);
-    }
-    const int rc = ensure_stage(h, size_t(base) + n);
-    if (rc) return rc;
-    const int rc2 = h->mix_into_stage(src, 0, 0, h->n_ch, base, n);
-    if (rc2) return rc2;
-    h->add_pushed(unsigned(n));
-    return HBD_OK;
-}
-int hbd_push_wideband(hbd_decoder* h, const float* iq, size_t n, double fs) { return push_wideband(h, iq, n, fs, false); }
-int hbd_push_wideband_device(hbd_decoder* h, const float* d_iq, size_t n, double fs) { return push_wideband(h, d_iq, n, fs, true); }
-int hbd_push_iq_wideband(hbd_decoder* h, const void* iq, int format, size_t n, double fs) { return push_wideband(h, iq, n, fs, false, format); }
-int hbd_push_iq_wideband_device(hbd_decoder* h, const void* d_iq, int format, size_t n, double fs) { return push_wideband(h, d_iq, n, fs, true, format); }
+{ return h ? h->push({iq, false, HBD_IQ_CF32, PushSrc::kMatrix, 0, pitch, n, fs}) : HBD_ERR_ARG; }
+int hbd_push_samples_device(hbd_decoder* h, const float* d_iq, size_t n, size_t pitch, double fs)
+{ return h ? h->push({d_iq, true, HBD_IQ_CF32, PushSrc::kMatrix, 0, pitch, n, fs}) : HBD_ERR_ARG; }
+int hbd_push_wideband(hbd_decoder* h, const float* iq, size_t n, double fs)
+{ return h ? h->push({iq, false, HBD_IQ_CF32, PushSrc::kRow, 0, 0, n, fs}) : HBD_ERR_ARG; }
+int hbd_push_wideband_device(hbd_decoder* h, const float* d_iq, size_t n, double fs)
+{ return h ? h->push({d_iq, true, HBD_IQ_CF32, PushSrc::kRow, 0, 0, n, fs}) : HBD_ERR_ARG; }
+int hbd_push_iq(hbd_decoder* h, int ch, const void* iq, int format, size_t n, double fs)
+{ return h ? h->push({iq, false, format, PushSrc::kChannel, ch, 0, n, fs}) : HBD_ERR_ARG; }
+int hbd_push_iq_batch(hbd_decoder* h, const void* iq, int format, size_t n, size_t pitch, double fs)
+{ return h ? h->push({iq, false, format, PushSrc::kMatrix, 0, pitch, n, fs}) : HBD_ERR_ARG; }
+int hbd_push_iq_device(hbd_decoder* h, const void* d_iq, int format, size_t n, size_t pitch, double fs)
+{ return h ? h->push({d_iq, true, format, PushSrc::kMatrix, 0, pitch, n, fs}) : HBD_ERR_ARG; }
+int hbd_push_iq_wideband(hbd_decoder* h, const void* iq, int format, size_t n, double fs)
+{ return h ? h->push({iq, false, format, PushSrc::kRow, 0, 0, n, fs}) : HBD_ERR_ARG; }
+int hbd_push_iq_wideband_device(hbd_decoder* h, const void* d_iq, int format, size_t n, double fs)
+{ return h ? h->push({d_iq, true, format, PushSrc::kRow, 0, 0, n, fs}) : HBD_ERR_ARG; }
 
 int hbd_set_nco(hbd_decoder* h, int ch, double freq_hz)
 {
@@ -1679,137 +1698,6 @@ double hbd_get_nco(hbd_decoder* h, int ch)
     if (!h || ch < 0 || ch >= h->n_ch) return 0;
     std::lock_guard<std::mutex> l(h->mtx);
     return h->hc[size_t(ch)].nco_freq;
-}
-
-int hbd_push_samples_device(hbd_decoder* h, const float* d_iq, size_t n, size_t pitch, double fs)
-{
-    HBD_CHECK_H(h);
-    if (!d_iq || pitch < n || (pitch & 1) || (reinterpret_cast<uintptr_t>(d_iq) & 15)) return HBD_ERR_ARG;
-    std::lock_guard<std::mutex> l(h->mtx);
-    if (h->ext) { h->set_error("device push pending"); return HBD_ERR_STATE; }
-    latch_rate(h, fs);
-    if (h->nco_active()) { // zero copy is not possible: the mixed samples go through the staging matrix
-        if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
-        unsigned base = 0;
-        if (!h->queue_depth_equal(base)) { h->set_error("batch push needs equal queue depth in all channels"); return HBD_ERR_STATE; }
-        if (h->nco_fused && base == 0 && n && decim1_supports_fused_nco(h->M1, h->T1))
-            return h->push_fused_nco(reinterpret_cast<const float2*>(d_iq), pitch, n);   // zero copy after all: K1 mixes
-        const int rc = ensure_stage(h, size_t(base) + n);
-        if (rc) return rc;
-        const int rc2 = h->mix_into_stage(reinterpret_cast<const float2*>(d_iq), pitch, 0, h->n_ch, base, n);
-        if (rc2) return rc2;
-        h->add_pushed(unsigned(n));
-        return HBD_OK;
-    }
-    { unsigned base = 0; if (!h->queue_depth_equal(base) || base) { h->set_error("host push pending"); return HBD_ERR_STATE; } }
-    h->ext = reinterpret_cast<const float2*>(d_iq); h->ext_pitch = pitch; h->ext_n = n;
-    return HBD_OK;
-}
-
-// ---- integer IQ input (include/habdec_b200.h: hbd_push_iq*) -------------------------------------------------------------
-int hbd_decoder::ensure_iq_up(size_t bytes)
-{
-    if (bytes <= iq_up_bytes) return HBD_OK;
-    HBD_CUDA_CHECK(cudaStreamSynchronize(stream));   // a widen of the previous push may still read the old buffer
-    cudaFree(d_iq_up); d_iq_up = nullptr; iq_up_bytes = 0;
-    HBD_CUDA_CHECK(cudaMalloc((void**)&d_iq_up, bytes));
-    iq_up_bytes = bytes;
-    return HBD_OK;
-}
-
-// device matrix [n_ch][pitch] of `format` -> cf32 d_widen [n_ch][*out_pitch] (even pitch: 16-byte rows), on the stream.  Work
-// put on the stream after a call waits for that call's K1 (process_async_locked), so d_widen is free again by then.
-int hbd_decoder::widen_device(const void* src, int format, size_t n, size_t pitch, size_t* out_pitch)
-{
-    const size_t wp = (n + 1) & ~size_t(1);
-    const size_t bytes = std::max<size_t>(size_t(n_ch) * wp * sizeof(float2), 256);
-    if (bytes > widen_bytes) {
-        HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
-        cudaFree(d_widen); d_widen = nullptr; widen_bytes = 0;
-        HBD_CUDA_CHECK(cudaMalloc((void**)&d_widen, bytes));
-        widen_bytes = bytes;
-    }
-    int nl = 0;
-    HBD_CUDA_CHECK(launch_nco_mix(src, pitch, d_widen, wp, 0, n, nullptr, 0, n_ch, stream, &nl, format));
-    launches += unsigned(nl);
-    *out_pitch = wp;
-    return HBD_OK;
-}
-
-int hbd_push_iq(hbd_decoder* h, int ch, const void* iq, int format, size_t n, double fs)
-{
-    if (format == HBD_IQ_CF32) return hbd_push_samples(h, ch, static_cast<const float*>(iq), n, fs);
-    HBD_CHECK_CH(h, ch);
-    const size_t bytes = size_t(iq_bytes(format));
-    if (!bytes || (!iq && n)) return HBD_ERR_ARG;
-    std::lock_guard<std::mutex> l(h->mtx);
-    if (h->ext) { h->set_error("device push pending"); return HBD_ERR_STATE; }
-    if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
-    if (h->n_ch > 1) h->leave_uniform();
-    HostChan& x = h->hc[size_t(ch)];
-    int rc = ensure_stage(h, size_t(x.pushed) + n);
-    if (!rc && n) rc = h->ensure_iq_up(n * bytes);
-    if (rc) return rc;
-    if (n) {
-        cudaError_t e = cudaMemcpyAsync(h->d_iq_up, iq, n * bytes, cudaMemcpyHostToDevice, h->stream);
-        if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
-    }
-    latch_rate(h, fs);
-    // widened (and mixed, where the channel has an NCO offset) into the staging row; returns after the stream has caught up,
-    // so the caller owns `iq` again
-    rc = h->mix_into_stage(h->d_iq_up, 0, ch, 1, x.pushed, n, format);
-    if (rc) return rc;
-    x.pushed += unsigned(n);
-    return HBD_OK;
-}
-
-int hbd_push_iq_batch(hbd_decoder* h, const void* iq, int format, size_t n, size_t pitch, double fs)
-{
-    if (format == HBD_IQ_CF32) return hbd_push_samples_batch(h, static_cast<const float*>(iq), n, pitch, fs);
-    HBD_CHECK_H(h);
-    const size_t bytes = size_t(iq_bytes(format));
-    if (!bytes || (!iq && n) || pitch < n) return HBD_ERR_ARG;
-    std::lock_guard<std::mutex> l(h->mtx);
-    if (h->ext) { h->set_error("device push pending"); return HBD_ERR_STATE; }
-    if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
-    unsigned base = 0;
-    if (!h->queue_depth_equal(base)) { h->set_error("batch push needs equal queue depth in all channels"); return HBD_ERR_STATE; }
-    int rc = ensure_stage(h, size_t(base) + n);
-    if (!rc && n) rc = h->ensure_iq_up(size_t(h->n_ch) * n * bytes);
-    if (rc) return rc;
-    if (n) {   // the integers cross PCIe, packed [n_ch][n]
-        cudaError_t e = cudaMemcpy2DAsync(h->d_iq_up, n * bytes, iq, pitch * bytes, n * bytes, size_t(h->n_ch), cudaMemcpyHostToDevice, h->stream);
-        if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
-    }
-    latch_rate(h, fs);
-    rc = h->mix_into_stage(h->d_iq_up, n, 0, h->n_ch, base, n, format);   // synchronises: the caller owns `iq` again
-    if (rc) return rc;
-    h->add_pushed(unsigned(n));
-    return HBD_OK;
-}
-
-int hbd_push_iq_device(hbd_decoder* h, const void* d_iq, int format, size_t n, size_t pitch, double fs)
-{
-    if (format == HBD_IQ_CF32) return hbd_push_samples_device(h, static_cast<const float*>(d_iq), n, pitch, fs);
-    HBD_CHECK_H(h);
-    const size_t bytes = size_t(iq_bytes(format));
-    if (!bytes || !d_iq || pitch < n || (pitch * bytes) % 16 || (reinterpret_cast<uintptr_t>(d_iq) & 15)) return HBD_ERR_ARG;
-    size_t wp = 0;
-    {
-        std::lock_guard<std::mutex> l(h->mtx);
-        if (h->ext) { h->set_error("device push pending"); return HBD_ERR_STATE; }
-        if (!h->nco_active() && decim1_supports_native_iq(h->M1, h->T1)) {   // zero copy: K1 streams the integers itself
-            latch_rate(h, fs);
-            { unsigned base = 0; if (!h->queue_depth_equal(base) || base) { h->set_error("host push pending"); return HBD_ERR_STATE; } }
-            h->ext = reinterpret_cast<const float2*>(d_iq); h->ext_pitch = pitch; h->ext_n = n; h->ext_format = format;
-            return HBD_OK;
-        }
-        if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
-        const int rc = h->widen_device(d_iq, format, n, pitch, &wp);
-        if (rc) return rc;
-    }
-    // every other case: the widened matrix takes the cf32 device push's path (fused NCO, K0 pre-mix or zero copy)
-    return hbd_push_samples_device(h, reinterpret_cast<const float*>(h->d_widen), n, wp, fs);
 }
 
 int hbd_process_async(hbd_decoder* h) { HBD_CHECK_H(h); return locked_then_fire(h, [h] { return h->process_async_locked(); }); }
