@@ -28,7 +28,6 @@
 #include "telemetry_abi.h"
 #include "api_internal.h"
 #include "nco.cuh"
-#include "iq_format.cuh"
 #include "ssdv.cuh"
 #include "tail.cuh"
 #include "wire.cuh"
@@ -91,6 +90,29 @@ struct HostChan : ChanCtr {
     double nco_freq = 0, nco_phase = 0; // pre-mixer: frequency in Hz, phase (cycles) of the next pushed sample
     bool cfg_dirty = true;
     ChanCtr& ctr() { return *this; }
+};
+
+// What one channel's share of a process() call amounts to on the host: the reference's buffer arithmetic
+// (Decoder.h:426-436,492-542) stepped on the channel's counters (step_channel), and the side effects that
+// hbd_decoder::apply_step applies to that channel's rows -- or, in uniform mode, to the rows of every channel at once.
+struct ChanStep {
+    ChanPlan plan;
+    bool zero_carry = false;       // Decimator.h:74-79: the stage's work buffer grew -> its history is zeroed
+    bool zero_s1hist = false;      // ... of the LAST stage (the tail kernel's input buffer)
+    unsigned zero_mid = 0;         // bit k: ... of middle stage k (cascaded plans)
+    bool zero_lphist = false;      // FirFilter.h:141-147
+    bool taps_changed = false;     // low-pass redesigned: upload `taps`
+    size_t taps_old = 0, taps_new = 0;
+    bool frame_done = false;       // this call completes an FFT frame (K4 runs)
+    unsigned nf = 0;
+};
+
+// what the kernel launches of a process call read from its planning (plan_call -> enqueue_call)
+struct CallPlan {
+    ChanPlan uplan{};   // every channel's plan when plan_uniform, else channel 0's (d_plan holds them all)
+    bool plan_uniform = true, any_work = false, need_k4 = false;
+    unsigned max_n1 = 0;
+    int sv_want = 0;
 };
 
 constexpr unsigned kMaxCallsBetweenCollects = 256; // process_async forces a drain beyond this (log capacity)
@@ -167,18 +189,28 @@ struct hbd_decoder {
         if (lo && cudaStreamSynchronize(lo) != cudaSuccess) return HBD_ERR_CUDA;
         return HBD_OK;
     }
+    // plan_call: wait for the compute streams once, before the first host-side change a kernel in flight could see
+    bool groups_idle = false;
+    int quiesce() { if (!groups_idle) { if (sync_groups()) return HBD_ERR_CUDA; groups_idle = true; } return HBD_OK; }
     bool record = false;
     unsigned long long launches = 0;
 
     double fs_in = 0;
     int factor = 1;
     int M1 = 1, T1 = 1, M2 = 1, T2 = 1;   // first stage (K1) and last stage (tail kernel; M2 == 1: the plan has one stage)
-    std::vector<TapTable> stages;         // the whole plan (Decoder.h:286-320, cascaded by setupDecimationStagesBW :350-399)
     struct MidStage { int M = 1, T = 1; unsigned div_in = 1; float* d_taps = nullptr; float2* d_out = nullptr; size_t pitch = 0; };
-    std::vector<MidStage> mids;           // stages[1 .. size-2]
+    std::vector<MidStage> mids;           // stages[1 .. size-2] of the plan (Decoder.h:286-320, cascaded by setupDecimationStagesBW :350-399)
     float2* d_midlast[2] = {nullptr, nullptr}; size_t midlast_pitch = 0, midlast_pitch_b = 0;   // output of the last middle stage = the tail kernel's
                                           // input, ping-pong over calls like d_s1x
-    unsigned div_last_in = 1;             // samples entering the last stage per call = consumed / div_last_in
+    // The input buffer of middle stage k (k == mids.size(): of the tail kernel): history slots [0, hist), this call's
+    // samples from hist on; `next` receives the history for the next call (== p where the buffer is not ping-ponged).
+    struct StageRows { float2* p; float2* next; size_t pitch; int hist; };
+    StageRows stage_in(size_t k) const
+    {
+        if (k == 0) return {d_s1x[s1_cur], d_s1x[s1_cur ^ 1], s1_pitch, kS1Hist};
+        if (k < mids.size()) return {mids[k - 1].d_out, mids[k - 1].d_out, mids[k - 1].pitch, kMidHist};
+        return {d_midlast[s1_cur], d_midlast[s1_cur ^ 1], midlast_pitch, kS1Hist};
+    }
     int carry_cap = kCarryCapMin;
     int set_plan(const std::vector<TapTable>& st, size_t total_factor);
     int fft_n = kFftN;       // spectrum size: 4096 like the reference, or 16384 (hbd_set_fft_size)
@@ -292,7 +324,6 @@ struct hbd_decoder {
     bool nco_any = false;    // some channel has (had) a non-zero NCO frequency or phase (set by hbd_set_nco, never cleared)
     void nco_params(NcoChan* out, int c0, int nc, size_t n, bool k0_rotation);
     int mix_into_stage(const void* src, size_t src_pitch, int c0, int nc, size_t dst_off, size_t n, int format = HBD_IQ_CF32);
-    int pending_marks = 0;   // async calls since the last collect
     int sv_override = -1;
     bool mask_cache = true;      // HBD_MASK_CACHE=0 (test hook): the slicer's position masks are rebuilt from scratch in every call
     // optional per-kernel CUDA-event timing (bench roofline): one event pair per K1 launch / per rest-of-step
@@ -332,6 +363,9 @@ struct hbd_decoder {
     void set_error(const std::string& e) { err = e; }
     int ensure_call_capacity(size_t n_in_max);
     int alloc_fixed();
+    int apply_step(const ChanStep& st, size_t c0, size_t rows, const std::vector<float>& taps);
+    int plan_call(CallPlan& cp);
+    int enqueue_call(const CallPlan& cp);
     int process_async_locked();
     int collect_locked(unsigned lag);
     int log_pressure();
@@ -496,7 +530,6 @@ int hbd_decoder::set_plan(const std::vector<TapTable>& st, size_t total_factor)
     const size_t n = size_t(n_ch);
     sync_ctrs();
     const int old_cap = carry_cap;
-    stages = st;
     factor = int(total_factor);
     M1 = T1 = M2 = T2 = 1;
     if (!st.empty()) {
@@ -520,7 +553,6 @@ int hbd_decoder::set_plan(const std::vector<TapTable>& st, size_t total_factor)
         mids.push_back(m);
         div *= unsigned(m.M);
     }
-    div_last_in = div;
     // the carry holds T1-1 samples of history plus the unconsumed remainder (< total factor).  Fresh, zeroed rows (new
     // decimators have an empty history); the remainder queued under the old plan stays queued, as in the reference
     unsigned max_r = 0;
@@ -612,24 +644,7 @@ int hbd_decoder::ensure_call_capacity(size_t n_in_max)
     return HBD_OK;
 }
 
-namespace {
-// What one channel's share of a process() call amounts to on the host: the reference's buffer arithmetic
-// (Decoder.h:426-436,492-542) stepped on the channel's counters.  No CUDA calls in here; the caller applies the
-// side effects to that channel's rows -- or, in uniform mode, to the rows of every channel at once.
-struct ChanStep {
-    ChanPlan plan;
-    bool zero_carry = false;       // Decimator.h:74-79: the stage's work buffer grew -> its history is zeroed
-    bool zero_s1hist = false;      // ... of the LAST stage (the tail kernel's input buffer)
-    unsigned zero_mid = 0;         // bit k: ... of middle stage k (cascaded plans)
-    bool zero_lphist = false;      // FirFilter.h:141-147
-    bool taps_changed = false;     // low-pass redesigned: upload `taps`
-    size_t taps_old = 0, taps_new = 0;
-    bool frame_done = false;       // this call completes an FFT frame (K4 runs)
-    unsigned nf = 0;
-};
-} // namespace
-
-// returns HBD_OK or HBD_ERR_ARG (nothing has been changed in that case)
+// No CUDA calls in here.  Returns HBD_OK or HBD_ERR_ARG (nothing has been changed in that case)
 static int step_channel(hbd_decoder* h, HostChan& x, unsigned pushed, ChanStep& o, std::vector<float>& taps)
 {
     const int factor = h->factor, M1 = h->M1, T1 = h->T1, M2 = h->M2, T2 = h->T2, fft_n = h->fft_n;
@@ -692,7 +707,7 @@ static int step_channel(hbd_decoder* h, HostChan& x, unsigned pushed, ChanStep& 
     x.lp_input_size = nf; x.lp_dirty = false;
     if (redesign) {
         o.taps_changed = true; o.taps_old = x.lp_ntaps; o.taps_new = T;
-        x.lp_ntaps = T; x.cfg_dirty = true; h->cfg_dirty_any = true; h->derived_dirty = true;
+        x.lp_ntaps = T; h->derived_dirty = true;
     }
     p.lp_ntaps = unsigned(x.lp_ntaps);
     const size_t need = size_t(nf) + x.lp_ntaps;
@@ -723,94 +738,58 @@ int hbd_decoder::log_pressure()
     return collect_locked(call_seq - calls_collected > 2u ? 1u : 0u);
 }
 
-int hbd_decoder::process_async_locked()
+// One ChanStep's side effects on the rows [c0, c0 + rows) of the per-channel buffers: a uniform call applies channel 0's
+// step to every row (0, n_ch), a per-channel call each channel's step to its own row (c, 1).
+int hbd_decoder::apply_step(const ChanStep& st, size_t c0, size_t rows, const std::vector<float>& taps)
 {
-    if (!fs_in) return HBD_OK; // Decoder.h:418-419: uninitialised -> silently nothing
-    HBD_CUDA_CHECK(cudaSetDevice(device));
-    { const int rc = log_pressure(); if (rc) return rc; }
-    const size_t n = size_t(n_ch);
-    const double fs_dec = fs_in / factor;
-    bool groups_idle = false; // set once we had to wait for the compute streams (rare host-side state changes)
-    auto quiesce = [&]() -> int { if (!groups_idle) { if (sync_groups()) return HBD_ERR_CUDA; groups_idle = true; } return HBD_OK; };
+    if (!(st.zero_carry || st.zero_s1hist || st.zero_mid || st.zero_lphist || st.taps_changed)) return HBD_OK;
+    if (quiesce()) return HBD_ERR_CUDA;
+    auto zero = [&](float2* p, size_t pitch, size_t w) {   // w samples from p on, in each of the rows of a [n_ch][pitch] matrix
+        return cudaMemset2DAsync(p + c0 * pitch, pitch * sizeof(float2), 0, w * sizeof(float2), rows, stream);
+    };
+    if (st.zero_carry) HBD_CUDA_CHECK(zero(d_carry2[carry_cur] + (carry_cap - (T1 - 1) - int(st.plan.r)), size_t(carry_cap), size_t(T1 - 1)));
+    for (size_t k = 0; k < mids.size(); ++k)
+        if (st.zero_mid & (1u << k)) { const StageRows s = stage_in(k); HBD_CUDA_CHECK(zero(s.p, s.pitch, size_t(s.hist))); }
+    if (st.zero_s1hist) { const StageRows s = stage_in(mids.size()); HBD_CUDA_CHECK(zero(s.p, s.pitch, size_t(s.hist))); }
+    if (st.taps_changed) {
+        std::vector<float> all(rows * st.taps_new);
+        for (size_t c = 0; c < rows; ++c) memcpy(all.data() + c * st.taps_new, taps.data(), 4 * st.taps_new);
+        HBD_CUDA_CHECK(cudaMemcpy2DAsync(d_lptaps + c0 * kLpMaxTaps, kLpMaxTaps * sizeof(float), all.data(), st.taps_new * sizeof(float), st.taps_new * sizeof(float), rows,
+                                         cudaMemcpyHostToDevice, stream));
+        HBD_CUDA_CHECK(cudaStreamSynchronize(stream)); // `all` goes out of scope
+        for (size_t c = c0; c < c0 + rows; ++c) hc[c].cfg_dirty = true;   // lp_ntaps travels with the configuration upload
+        cfg_dirty_any = true;
+    }
+    if (st.zero_lphist) HBD_CUDA_CHECK(zero(d_decq, dq_pitch, std::min<size_t>(st.plan.lp_ntaps, kLpHist)));
+    return HBD_OK;
+}
 
-    // ---- plan ------------------------------------------------------------------------------------------------
+// The host half of a process call: step the counters of the channels (channel 0 alone in uniform mode), size the per-call
+// buffers, apply the side effects, upload configuration and plans.  Everything in a call that may wait for the GPU is here.
+int hbd_decoder::plan_call(CallPlan& cp)
+{
+    const size_t n = size_t(n_ch);
+    groups_idle = false;
     // uniform mode (whole-batch pushes only, one low-pass setting): channel 0 stands for all of them, O(1) per call
     const bool uni = ctr_uniform && lp_cfg_uniform;
-    if (!uni) sync_ctrs();
-    size_t max_total = 0; unsigned max_n1 = 0, max_nf = 0;
-    bool any_work = false, need_k4 = false;
+    if (!uni) { sync_ctrs(); h_plan.resize(n); }
+    const size_t stepped = uni ? 1 : n;
+    auto pushed = [&](size_t c) { return in.p ? unsigned(in.n) : hc[c].pushed; };
+    size_t max_total = 0;
+    for (size_t c = 0; c < stepped; ++c) max_total = std::max<size_t>(max_total, size_t(hc[c].in_r) + pushed(c));
+    if (max_total > cap_n_in || !d_s1x[0]) { if (quiesce()) return HBD_ERR_CUDA; }   // buffers are about to be reallocated
+    { const int rc = ensure_call_capacity(max_total); if (rc) return rc; }
+    unsigned max_nf = 0;
     std::vector<float> new_taps;
-    ChanPlan uplan{};
-    if (uni) {
+    for (size_t c = 0; c < stepped; ++c) {
         ChanStep st;
-        const unsigned pushed = in.p ? unsigned(in.n) : hc[0].pushed;
-        max_total = size_t(hc[0].in_r) + pushed;
-        if (max_total > cap_n_in || !d_s1x[0]) { if (quiesce()) return HBD_ERR_CUDA; }   // buffers are about to be reallocated
-        { const int rc = ensure_call_capacity(max_total); if (rc) return rc; }
-        const int rc = step_channel(this, hc[0], pushed, st, new_taps);
-        if (rc) return rc;   // nothing has been stepped
-        ctr_stale = true;
-        uplan = st.plan;
-        any_work = !(st.plan.flags & 1u); need_k4 = st.frame_done; max_n1 = st.plan.n1; max_nf = st.nf;
-        if (st.zero_carry || st.zero_s1hist || st.zero_mid || st.zero_lphist || st.taps_changed) {
-            if (quiesce()) return HBD_ERR_CUDA;
-            if (st.zero_carry)
-                HBD_CUDA_CHECK(cudaMemset2DAsync(d_carry2[carry_cur] + (carry_cap - (T1 - 1) - int(st.plan.r)), size_t(carry_cap) * sizeof(float2), 0,
-                                                 sizeof(float2) * size_t(T1 - 1), n, stream));
-            for (size_t k = 0; k < mids.size(); ++k)
-                if (st.zero_mid & (1u << k)) {
-                    if (k == 0) HBD_CUDA_CHECK(cudaMemset2DAsync(d_s1x[s1_cur], s1_pitch * sizeof(float2), 0, sizeof(float2) * kS1Hist, n, stream));
-                    else HBD_CUDA_CHECK(cudaMemset2DAsync(mids[k - 1].d_out, mids[k - 1].pitch * sizeof(float2), 0, sizeof(float2) * kMidHist, n, stream));
-                }
-            if (st.zero_s1hist) {
-                if (mids.empty()) HBD_CUDA_CHECK(cudaMemset2DAsync(d_s1x[s1_cur], s1_pitch * sizeof(float2), 0, sizeof(float2) * kS1Hist, n, stream));
-                else HBD_CUDA_CHECK(cudaMemset2DAsync(d_midlast[s1_cur], midlast_pitch * sizeof(float2), 0, sizeof(float2) * kS1Hist, n, stream));
-            }
-            if (st.taps_changed) {
-                std::vector<float> all(n * st.taps_new);
-                for (size_t c = 0; c < n; ++c) memcpy(all.data() + c * st.taps_new, new_taps.data(), 4 * st.taps_new);
-                HBD_CUDA_CHECK(cudaMemcpy2DAsync(d_lptaps, kLpMaxTaps * sizeof(float), all.data(), st.taps_new * sizeof(float), st.taps_new * sizeof(float), n,
-                                                 cudaMemcpyHostToDevice, stream));
-                HBD_CUDA_CHECK(cudaStreamSynchronize(stream)); // `all` goes out of scope
-                for (size_t c = 1; c < n; ++c) hc[c].cfg_dirty = true;   // lp_ntaps travels with the configuration upload
-            }
-            if (st.zero_lphist) HBD_CUDA_CHECK(cudaMemset2DAsync(d_decq, dq_pitch * sizeof(float2), 0, sizeof(float2) * std::min<size_t>(hc[0].lp_ntaps, kLpHist), n, stream));
-        }
-    } else {
-        h_plan.resize(n);
-        for (size_t c = 0; c < n; ++c) max_total = std::max<size_t>(max_total, size_t(hc[c].in_r) + (in.p ? unsigned(in.n) : hc[c].pushed));
-        if (max_total > cap_n_in || !d_s1x[0]) { if (quiesce()) return HBD_ERR_CUDA; }
-        { const int rc = ensure_call_capacity(max_total); if (rc) return rc; }
-        for (size_t c = 0; c < n; ++c) {
-            HostChan& x = hc[c];
-            ChanStep st;
-            const int rc = step_channel(this, x, in.p ? unsigned(in.n) : x.pushed, st, new_taps);
-            if (rc) return rc;   // channels below c have been stepped: their samples are gone (documented in the header)
-            h_plan[c] = st.plan;
-            any_work |= !(st.plan.flags & 1u); need_k4 |= st.frame_done;
-            max_n1 = std::max(max_n1, st.plan.n1); max_nf = std::max(max_nf, st.nf);
-            if (!(st.zero_carry || st.zero_s1hist || st.zero_mid || st.zero_lphist || st.taps_changed)) continue;
-            if (quiesce()) return HBD_ERR_CUDA;
-            if (st.zero_carry) HBD_CUDA_CHECK(cudaMemsetAsync(d_carry2[carry_cur] + c * size_t(carry_cap) + (carry_cap - (T1 - 1) - int(st.plan.r)), 0, sizeof(float2) * size_t(T1 - 1), stream));
-            for (size_t k = 0; k < mids.size(); ++k)
-                if (st.zero_mid & (1u << k)) {
-                    if (k == 0) HBD_CUDA_CHECK(cudaMemsetAsync(d_s1x[s1_cur] + c * s1_pitch, 0, sizeof(float2) * kS1Hist, stream));
-                    else HBD_CUDA_CHECK(cudaMemsetAsync(mids[k - 1].d_out + c * mids[k - 1].pitch, 0, sizeof(float2) * kMidHist, stream));
-                }
-            if (st.zero_s1hist) {
-                if (mids.empty()) HBD_CUDA_CHECK(cudaMemsetAsync(d_s1x[s1_cur] + c * s1_pitch, 0, sizeof(float2) * kS1Hist, stream));
-                else HBD_CUDA_CHECK(cudaMemsetAsync(d_midlast[s1_cur] + c * midlast_pitch, 0, sizeof(float2) * kS1Hist, stream));
-            }
-            if (st.taps_changed) {
-                HBD_CUDA_CHECK(cudaMemcpyAsync(d_lptaps + c * kLpMaxTaps, new_taps.data(), 4 * st.taps_new, cudaMemcpyHostToDevice, stream));
-                HBD_CUDA_CHECK(cudaStreamSynchronize(stream)); // new_taps is reused
-            }
-            if (st.zero_lphist) HBD_CUDA_CHECK(cudaMemsetAsync(d_decq + c * dq_pitch, 0, sizeof(float2) * std::min<size_t>(x.lp_ntaps, kLpHist), stream));
-        }
-        // back to uniform mode as soon as the channels agree again (e.g. after a round of per-channel pushes of one size)
-        bool same = true;
-        for (size_t c = 1; c < n && same; ++c) same = hc[c].same(hc[0]);
-        ctr_uniform = same;
+        int rc = step_channel(this, hc[c], pushed(c), st, new_taps);
+        if (rc) return rc;   // channels below c have been stepped: their samples are gone (documented in the header)
+        if (uni) { ctr_stale = true; cp.uplan = st.plan; } else h_plan[c] = st.plan;
+        cp.any_work |= !(st.plan.flags & 1u); cp.need_k4 |= st.frame_done;
+        cp.max_n1 = std::max(cp.max_n1, st.plan.n1); max_nf = std::max(max_nf, st.nf);
+        rc = apply_step(st, c, uni ? n : 1, new_taps);
+        if (rc) return rc;
     }
     if (demod_acc_on) { const int rc = ensure_dacc(); if (rc) return rc; }
 
@@ -833,12 +812,13 @@ int hbd_decoder::process_async_locked()
         HBD_CUDA_CHECK(cudaStreamSynchronize(stream)); // host vectors go out of scope
         cfg_dirty_any = false;
     }
-    bool plan_uniform = uni;
     if (!uni) {
-        plan_uniform = true;
-        for (size_t c = 1; c < n && plan_uniform; ++c) plan_uniform = memcmp(&h_plan[c], &h_plan[0], sizeof(ChanPlan)) == 0;
-        uplan = h_plan[0];
-        if (!plan_uniform && (h_plan_uploaded.size() != n || memcmp(h_plan.data(), h_plan_uploaded.data(), n * sizeof(ChanPlan)) != 0)) {
+        // back to uniform mode as soon as the channels agree again (e.g. after a round of per-channel pushes of one size)
+        ctr_uniform = true;
+        for (size_t c = 1; c < n && ctr_uniform; ++c) ctr_uniform = hc[c].same(hc[0]);
+        for (size_t c = 1; c < n && cp.plan_uniform; ++c) cp.plan_uniform = memcmp(&h_plan[c], &h_plan[0], sizeof(ChanPlan)) == 0;
+        cp.uplan = h_plan[0];
+        if (!cp.plan_uniform && (h_plan_uploaded.size() != n || memcmp(h_plan.data(), h_plan_uploaded.data(), n * sizeof(ChanPlan)) != 0)) {
             if (quiesce()) return HBD_ERR_CUDA;
             HBD_CUDA_CHECK(cudaMemcpyAsync(d_plan, h_plan.data(), n * sizeof(ChanPlan), cudaMemcpyHostToDevice, stream));
             HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
@@ -849,6 +829,7 @@ int hbd_decoder::process_async_locked()
     // what the tail kernel stages in shared memory: sized from host-side knowledge of all channels
     if (derived_dirty) {
         sync_ctrs();
+        const double fs_dec = fs_in / factor;
         max_lp_taps_c = 1; max_spb_c = 1;
         for (size_t c = 0; c < n; ++c) {
             max_lp_taps_c = std::max(max_lp_taps_c, hc[c].lp_ntaps);
@@ -857,19 +838,20 @@ int hbd_decoder::process_async_locked()
         derived_dirty = false;
     }
     // a channel normally holds < ~12 symbols of pending samples after a slicer pass (plus this call's batch)
-    int sv_want = int(std::min<double>(6144.0, 16.0 * max_spb_c + double(max_nf) + 64.0));
-    if (sv_override >= 0) sv_want = sv_override;   // test hook (HBD_SV_WANT): 0 forces the slicer's HBM path
+    cp.sv_want = int(std::min<double>(6144.0, 16.0 * max_spb_c + double(max_nf) + 64.0));
+    if (sv_override >= 0) cp.sv_want = sv_override;   // test hook (HBD_SV_WANT): 0 forces the slicer's HBM path
+    return HBD_OK;
+}
 
-    if (in.p && in.format != HBD_IQ_CF32 && !decim1_supports_native_iq(M1, T1)) {   // the plan changed after a native integer push
-        size_t wp = 0;
-        const int rc = widen(in.p, in.pitch, in.format, n_ch, in.n, &wp);
-        if (rc) return rc;
-        in = DeviceInput{d_widen, wp, in.n};
-    }
+// The device half of a process call: the kernel sequence on the hi / lo streams, the commit of the log heads and the
+// ping-pong flips.  No allocation, no synchronisation.
+int hbd_decoder::enqueue_call(const CallPlan& cp)
+{
+    const double fs_dec = fs_in / factor;
     const float2* chunk = in.p ? static_cast<const float2*>(in.p) : d_stage;
     const size_t chunk_pitch = in.p ? in.pitch : stage_pitch;
     int nl = 0;
-    // everything the caller (and the host-side updates above) put on `stream` happens before the kernels start
+    // everything the caller (and the host-side updates of plan_call) put on `stream` happens before the kernels start
     HBD_CUDA_CHECK(cudaEventRecord(ev_in, stream));
     HBD_CUDA_CHECK(cudaStreamWaitEvent(hi, ev_in, 0));
     bool tail_recorded = false;
@@ -879,35 +861,34 @@ int hbd_decoder::process_async_locked()
         DecimArgs da{};
         da.chunk = chunk; da.chunk_pitch = chunk_pitch; da.carry = d_carry2[carry_cur]; da.carry_next = d_carry2[carry_cur ^ 1]; da.carry_cap = carry_cap;
         da.s1 = d_s1x[s1_cur]; da.s1_pitch = s1_pitch; da.s1_hist = kS1Hist;
-        da.plan = d_plan; da.uplan = uplan; da.uniform = plan_uniform ? 1 : 0; da.taps = d_taps1; da.ch0 = 0; da.n_channels = n_ch;
+        da.plan = d_plan; da.uplan = cp.uplan; da.uniform = cp.plan_uniform ? 1 : 0; da.taps = d_taps1; da.ch0 = 0; da.n_channels = n_ch;
         da.nco = in.nco;
         if (timing) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_k1, ev_used_k1), hi));
-        HBD_CUDA_CHECK(launch_decim1(da, M1, T1, max_n1, n_sms, hi, &nl, in.format));
+        HBD_CUDA_CHECK(launch_decim1(da, M1, T1, cp.max_n1, n_sms, hi, &nl, in.format));
         if (timing) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_k1, ev_used_k1), hi));
     }
     HBD_CUDA_CHECK(cudaEventRecord(ev_consumed, hi)); // input no longer needed; stage-1 output ready
     HBD_CUDA_CHECK(cudaStreamWaitEvent(lo, ev_consumed, 0));
     if (timing > 1) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_rest, ev_used_rest), lo));
-    if (any_work) {
+    if (cp.any_work) {
         // cascaded plan: the stages between K1's and the tail kernel's (1/64 of the input rate or less)
         for (size_t k = 0; k < mids.size(); ++k) {
+            const StageRows in_k = stage_in(k), out_k = stage_in(k + 1);
             MidArgs ma{};
-            ma.plan = d_plan; ma.uplan = uplan; ma.uniform = plan_uniform ? 1 : 0;
-            if (k == 0) { ma.in = d_s1x[s1_cur]; ma.in_next = d_s1x[s1_cur ^ 1]; ma.in_pitch = s1_pitch; ma.in_hist = kS1Hist; }
-            else { ma.in = mids[k - 1].d_out; ma.in_next = mids[k - 1].d_out; ma.in_pitch = mids[k - 1].pitch; ma.in_hist = kMidHist; }
-            if (k + 1 < mids.size()) { ma.out = mids[k].d_out; ma.out_pitch = mids[k].pitch; ma.out_hist = kMidHist; }
-            else { ma.out = d_midlast[s1_cur]; ma.out_pitch = midlast_pitch; ma.out_hist = kS1Hist; }
+            ma.plan = d_plan; ma.uplan = cp.uplan; ma.uniform = cp.plan_uniform ? 1 : 0;
+            ma.in = in_k.p; ma.in_next = in_k.next; ma.in_pitch = in_k.pitch; ma.in_hist = in_k.hist;
+            ma.out = out_k.p; ma.out_pitch = out_k.pitch; ma.out_hist = out_k.hist;
             ma.taps = mids[k].d_taps; ma.M = mids[k].M; ma.T = mids[k].T; ma.div_in = mids[k].div_in;
             HBD_CUDA_CHECK(launch_mid_stage(ma, n_ch, lo, &nl));
         }
+        const StageRows s1 = stage_in(mids.size());
         TailArgs ta{};
-        ta.plan = d_plan; ta.uplan = uplan; ta.uniform = plan_uniform ? 1 : 0; ta.state = d_state; ta.ch0 = 0;
-        if (mids.empty()) { ta.s1 = d_s1x[s1_cur]; ta.s1_next = d_s1x[s1_cur ^ 1]; ta.s1_pitch = s1_pitch; }
-        else { ta.s1 = d_midlast[s1_cur]; ta.s1_next = d_midlast[s1_cur ^ 1]; ta.s1_pitch = midlast_pitch; }
+        ta.plan = d_plan; ta.uplan = cp.uplan; ta.uniform = cp.plan_uniform ? 1 : 0; ta.state = d_state; ta.ch0 = 0;
+        ta.s1 = s1.p; ta.s1_next = s1.next; ta.s1_pitch = s1.pitch;
         ta.taps2 = d_taps2; ta.M2 = M2; ta.T2 = T2;
         ta.decq = d_decq; ta.dq_pitch = dq_pitch; ta.fs_dec = fs_dec; ta.fftbuf = d_fftbuf; ta.fft_n = fft_n; ta.lptaps = d_lptaps;
         ta.max_lp_taps = int(max_lp_taps_c);
-        ta.slicer = d_slicer; ta.slicer_pitch = slicer_pitch; ta.sv_want = sv_want;
+        ta.slicer = d_slicer; ta.slicer_pitch = slicer_pitch; ta.sv_want = cp.sv_want;
         ta.log = d_log; ta.log_ctl = d_log_ctl; ta.log_mask = log_cap - 1u; ta.call_seq = call_seq & 0xffffffu;
         ta.uart_runs = d_uart_runs;
         ta.maskc = mask_cache ? d_maskc : nullptr;
@@ -922,7 +903,7 @@ int hbd_decoder::process_async_locked()
         FftArgs fa{};
         fa.state = d_state; fa.fftbuf = d_fftbuf; fa.spectrum = d_spectrum; fa.power = d_power; fa.twiddle = d_twiddle; fa.fs_dec = fs_dec;
         fa.ch0 = 0; fa.fft_n = fft_n;
-        if (need_k4) HBD_CUDA_CHECK(launch_fft_afc(fa, n_ch, lo, &nl));   // other calls: K2 has stepped the AFC itself
+        if (cp.need_k4) HBD_CUDA_CHECK(launch_fft_afc(fa, n_ch, lo, &nl));   // other calls: K2 has stepped the AFC itself
         if (ssdv_on) {   // test every 0x55-started window the new characters completed
             SsdvScanArgs sa{};
             sa.ring = d_ssdv_ring; sa.total = d_ssdv_total; sa.scanned = d_ssdv_scanned; sa.log = d_ssdv_log;
@@ -942,10 +923,10 @@ int hbd_decoder::process_async_locked()
     // the caller's stream resumes once the input has been consumed (it does not wait for the tail kernels)
     HBD_CUDA_CHECK(cudaStreamWaitEvent(stream, ev_consumed, 0));
     carry_cur ^= 1;
-    if (any_work) s1_cur ^= 1; // the tail (which moves the stage-2 history to the other buffer) ran
+    if (cp.any_work) s1_cur ^= 1; // the tail (which moves the stage-2 history to the other buffer) ran
     launches += unsigned(nl);
     if (snap_on) {
-        stats_snap_kernel<<<(n_ch + 127) / 128, 128, 0, lo>>>(d_state, d_snap + size_t(call_seq % kSnapSlots) * n * 6, n_ch);
+        stats_snap_kernel<<<(n_ch + 127) / 128, 128, 0, lo>>>(d_state, d_snap + size_t(call_seq % kSnapSlots) * size_t(n_ch) * 6, n_ch);
         ++launches;
     }
     // commit: the log control words as they stand after this call, into the call's pinned slot (stream order: every
@@ -954,7 +935,23 @@ int hbd_decoder::process_async_locked()
     HBD_CUDA_CHECK(cudaMemcpyAsync(h_heads + slot * kCtlWords, d_log_ctl, kCtlWords * sizeof(unsigned), cudaMemcpyDeviceToHost, lo));
     HBD_CUDA_CHECK(cudaEventRecord(ev_call[slot], lo)); // everything of this call is done
     ++call_seq;
-    ++pending_marks;
+    return HBD_OK;
+}
+
+int hbd_decoder::process_async_locked()
+{
+    if (!fs_in) return HBD_OK; // Decoder.h:418-419: uninitialised -> silently nothing
+    HBD_CUDA_CHECK(cudaSetDevice(device));
+    { const int rc = log_pressure(); if (rc) return rc; }
+    CallPlan cp;
+    { const int rc = plan_call(cp); if (rc) return rc; }
+    if (in.p && in.format != HBD_IQ_CF32 && !decim1_supports_native_iq(M1, T1)) {   // the plan changed after a native integer push
+        size_t wp = 0;
+        const int rc = widen(in.p, in.pitch, in.format, n_ch, in.n, &wp);
+        if (rc) return rc;
+        in = DeviceInput{d_widen, wp, in.n};
+    }
+    { const int rc = enqueue_call(cp); if (rc) return rc; }
     in = DeviceInput{};
     return HBD_OK;
 }
@@ -989,7 +986,6 @@ int hbd_decoder::collect_locked(unsigned lag)
     unsigned heads[kCtlWords];
     memcpy(heads, h_heads + size_t((upto - 1) % ev_call.size()) * kCtlWords, sizeof(heads));
     const unsigned head = heads[kCtlCharHead];
-    const unsigned upto24 = upto & 0xffffffu;
     int result = HBD_OK;
     if (ssdv_on) {
         // accepted SSDV packets of the calls being drained go to their channels first: the buffer automaton below
@@ -1167,11 +1163,9 @@ int hbd_decoder::collect_locked(unsigned lag)
             for (auto& e : all) deferred.push_back(std::move(e.second));
         }
     }
-    (void)upto24;
     drain_host_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_replay0).count();
     drain_calls += upto - calls_collected;
     calls_collected = upto;
-    pending_marks = int(call_seq - calls_collected);
     return result;
 }
 
