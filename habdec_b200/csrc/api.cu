@@ -27,6 +27,7 @@
 #include "range_pool.h"
 #include "telemetry_abi.h"
 #include "api_internal.h"
+#include "cuda_res.h"
 #include "nco.cuh"
 #include "ssdv.cuh"
 #include "tail.cuh"
@@ -171,23 +172,32 @@ struct hbd_decoder {
     std::mutex mtx;
     std::string err;
     int n_ch = 0, device = 0, n_sms = 148;
+    // The streams come first: members are destroyed in reverse order, so the streams outlive the buffers and events.
     cudaStream_t stream = nullptr;   // the caller's stream: inputs are ordered on it, it waits until inputs are consumed
-    bool own_stream = false;
+    Stream own_stream;               // the private stream `stream` is until hbd_set_stream
     // Two streams: the HBM-bound K1 of call s+1 overlaps the FP32/latency-bound tail kernels of call s (the stage-1
     // stream and the carry are double buffered over calls, so K1 only ever waits for the tail of call s-1).
     //   hi (high priority): K1 (+ carry) of every call
     //   lo (low priority):  K2 tail / K4 fft_afc; they fill the SM resources K1 leaves free
-    cudaStream_t hi = nullptr, lo = nullptr;
-    cudaEvent_t ev_consumed = nullptr;      // K1 + carry done (input consumed, stage-1 output ready)
-    cudaEvent_t ev_tail[2] = {nullptr, nullptr};   // per stage-1 buffer: tail done, that buffer may be overwritten by K1
+    Stream hi, lo;
+    Stream copy_stream;              // result read-back, independent of the compute streams
+    Event ev_consumed;               // K1 + carry done (input consumed, stage-1 output ready)
+    Event ev_tail[2];                // per stage-1 buffer: tail done, that buffer may be overwritten by K1
     bool tail_pending[2] = {false, false};
     bool tail_ev_late = false;              // HBD_TAIL_EV_LATE=1 (measurement hook): record ev_tail after the whole lo-stream sequence
-    cudaEvent_t ev_in = nullptr;
+    Event ev_in;
     int sync_groups()
     {
-        if (hi && cudaStreamSynchronize(hi) != cudaSuccess) return HBD_ERR_CUDA;
-        if (lo && cudaStreamSynchronize(lo) != cudaSuccess) return HBD_ERR_CUDA;
+        if (hi && cudaStreamSynchronize(hi.get()) != cudaSuccess) return HBD_ERR_CUDA;
+        if (lo && cudaStreamSynchronize(lo.get()) != cudaSuccess) return HBD_ERR_CUDA;
         return HBD_OK;
+    }
+    ~hbd_decoder()
+    {
+        cudaSetDevice(device);
+        sync_groups();
+        if (stream) cudaStreamSynchronize(stream);
+        dist_ctx.reset();
     }
     // plan_call: wait for the compute streams once, before the first host-side change a kernel in flight could see
     bool groups_idle = false;
@@ -198,23 +208,23 @@ struct hbd_decoder {
     double fs_in = 0;
     int factor = 1;
     int M1 = 1, T1 = 1, M2 = 1, T2 = 1;   // first stage (K1) and last stage (tail kernel; M2 == 1: the plan has one stage)
-    struct MidStage { int M = 1, T = 1; unsigned div_in = 1; float* d_taps = nullptr; float2* d_out = nullptr; size_t pitch = 0; };
+    struct MidStage { int M = 1, T = 1; unsigned div_in = 1; DevPtr<float> d_taps; Rows<float2> out; };
     std::vector<MidStage> mids;           // stages[1 .. size-2] of the plan (Decoder.h:286-320, cascaded by setupDecimationStagesBW :350-399)
-    float2* d_midlast[2] = {nullptr, nullptr}; size_t midlast_pitch = 0, midlast_pitch_b = 0;   // output of the last middle stage = the tail kernel's
-                                          // input, ping-pong over calls like d_s1x
+    Rows<float2, 2> midlast;              // output of the last middle stage = the tail kernel's input, ping-pong over calls like s1x
     // The input buffer of middle stage k (k == mids.size(): of the tail kernel): history slots [0, hist), this call's
     // samples from hist on; `next` receives the history for the next call (== p where the buffer is not ping-ponged).
     struct StageRows { float2* p; float2* next; size_t pitch; int hist; };
     StageRows stage_in(size_t k) const
     {
-        if (k == 0) return {d_s1x[s1_cur], d_s1x[s1_cur ^ 1], s1_pitch, kS1Hist};
-        if (k < mids.size()) return {mids[k - 1].d_out, mids[k - 1].d_out, mids[k - 1].pitch, kMidHist};
-        return {d_midlast[s1_cur], d_midlast[s1_cur ^ 1], midlast_pitch, kS1Hist};
+        if (k == 0) return {s1x.get(s1_cur), s1x.get(s1_cur ^ 1), s1x.pitch, kS1Hist};
+        if (k < mids.size()) return {mids[k - 1].out.get(), mids[k - 1].out.get(), mids[k - 1].out.pitch, kMidHist};
+        return {midlast.get(s1_cur), midlast.get(s1_cur ^ 1), midlast.pitch, kS1Hist};
     }
     int carry_cap = kCarryCapMin;
     int set_plan(const std::vector<TapTable>& st, size_t total_factor);
     int fft_n = kFftN;       // spectrum size: 4096 like the reference, or 16384 (hbd_set_fft_size)
-    int alloc_fft();
+    struct FftBufs { DevPtr<float2> buf, spectrum, twiddle; DevPtr<float> power; } fft;
+    int make_fft(int N, FftBufs& out);
     std::vector<HostChan> hc;        // per-channel configuration + counters (see ChanCtr)
     // Uniform mode: every channel has been fed the same way since creation (whole-batch pushes only), so all ChanCtr are
     // equal and only hc[0]'s is stepped per call; hc[1..] lag behind (ctr_stale) until sync_ctrs() copies them.
@@ -243,30 +253,26 @@ struct hbd_decoder {
     std::vector<hbd_result_record> pend;   // per channel: characters / sentence bytes waiting for a poll or the next gather (host_tail.h)
 
     // device state
-    ChanState* d_state = nullptr;
-    ChanPlan* d_plan = nullptr;
+    DevPtr<ChanState> d_state;
+    DevPtr<ChanPlan> d_plan;
     std::vector<ChanPlan> h_plan, h_plan_uploaded;
-    float2* d_carry2[2] = {nullptr, nullptr}; // stage-1 carry, ping-pong: K1 reads [carry_cur], writes [carry_cur ^ 1]
+    DevPtr<float2> d_carry2[2];  // stage-1 carry, ping-pong: K1 reads [carry_cur], writes [carry_cur ^ 1]
     int carry_cur = 0;
-    float2* d_s1x[2] = {nullptr, nullptr}; size_t s1_pitch = 0, s1_pitch_b = 0; // stage-1 stream, ping-pong over calls:
+    Rows<float2, 2> s1x;         // stage-1 stream, ping-pong over calls:
     int s1_cur = 0;              // K1 + tail of a call use [s1_cur]; the tail leaves the stage-2 history in [s1_cur ^ 1]
-    float2* d_decq = nullptr;    size_t dq_pitch = 0;
-    float2* d_fftbuf = nullptr;
-    float2* d_spectrum = nullptr;
-    float* d_power = nullptr;
-    float* d_lptaps = nullptr;
-    float* d_slicer = nullptr;   size_t slicer_pitch = 0;
-    float* d_demod = nullptr;    size_t demod_pitch = 0;
-    unsigned* d_maskc = nullptr;             // cached slicer position masks [n][2][kMaskWords] (tail.cu)
-    unsigned short* d_uart_runs = nullptr;   // UART backlog [n][kUartRunsCap] (slicer_dev.cuh)
+    Rows<float2> decq;
+    DevPtr<float> d_lptaps;
+    Rows<float> slicer, demod;
+    DevPtr<unsigned> d_maskc;                // cached slicer position masks [n][2][kMaskWords] (tail.cu)
+    DevPtr<unsigned short> d_uart_runs;      // UART backlog [n][kUartRunsCap] (slicer_dev.cuh)
     // Decoded-character log: ring of log_cap entries appended by the tail kernels (monotonic head in d_log_ctl[0]).
     // After the kernels of a call the control words are copied to that call's slot of h_heads (pinned), in stream order:
     // the host only ever reads a COMMITTED head, never the live one (entries below it are completely written).
-    uint2* d_log = nullptr;
+    DevPtr<uint2> d_log;
     unsigned log_cap = 0;                // power of two, sized from the channel count
-    unsigned* d_log_ctl = nullptr;       // kCtlWords control words (see LogCtl in hbd_common.cuh)
-    unsigned* h_heads = nullptr;         // pinned, [ev_call.size()][kCtlWords]
-    unsigned* h_tail_pin = nullptr;      // pinned, [2]: char log tail, SSDV log tail (source of the async upload)
+    DevPtr<unsigned> d_log_ctl;          // kCtlWords control words (see LogCtl in hbd_common.cuh)
+    HostPtr<unsigned> h_heads;           // pinned, [ev_call.size()][kCtlWords]
+    HostPtr<unsigned> h_tail_pin;        // pinned, [2]: char log tail, SSDV log tail (source of the async upload)
     unsigned log_tail = 0;               // host: entries below this index are already processed
     unsigned call_seq = 0;               // calls enqueued so far (24 bits travel in the log entries)
     unsigned calls_collected = 0;        // calls whose characters went through the sentence layer
@@ -275,9 +281,8 @@ struct hbd_decoder {
     unsigned per_call_max = 0;           // largest number of characters one completed call appended so far
     unsigned long long chars_lost = 0;   // characters dropped by log overflows (reported by hbd_collect*)
     unsigned ovf_seen[3] = {0, 0, 0};    // last seen kCtlSsdvRingOvf / kCtlSsdvOvf / kCtlCharOvf (monotonic counters)
-    std::vector<cudaEvent_t> ev_call;    // ring: completion of call (seq % size)
-    cudaStream_t copy_stream = nullptr;  // result read-back, independent of the compute streams
-    std::vector<uint2> h_log;            // host staging
+    std::vector<Event> ev_call;          // ring: completion of call (seq % size)
+    std::vector<uint2> h_log;           // host staging
     std::vector<std::string> call_chars; // per channel: raw chars of the call being replayed
     std::vector<unsigned> seg_start;     // collect_locked: first log entry of every (call, channel) segment
     static constexpr int kCharBufHost = 64;   // == kCharBuf (slicer_dev.cuh): characters per device-side flush
@@ -285,42 +290,41 @@ struct hbd_decoder {
     hbd::RangePool pool;                 // the drain's worker threads (part t of a drain / a pack runs on the same thread every time)
     int host_threads = 1;                // threads the drain may use (hbd_set_host_threads; default: min(4, half the cores this process may run on))
     bool keep_raw = true;                // hbd_set_raw_chars: retain the raw (unfiltered) characters for hbd_poll_raw_chars
-    float* d_taps1 = nullptr; float* d_taps2 = nullptr;
-    float2* d_twiddle = nullptr;
+    DevPtr<float> d_taps1, d_taps2;
     // config upload scratch
-    double* d_cfg_baud = nullptr; float* d_cfg_stops = nullptr; int* d_cfg_bits = nullptr; int* d_cfg_dc = nullptr;
-    int* d_cfg_ntaps = nullptr; unsigned char* d_cfg_dirty = nullptr;
+    DevPtr<double> d_cfg_baud; DevPtr<float> d_cfg_stops; DevPtr<int> d_cfg_bits, d_cfg_dc, d_cfg_ntaps; DevPtr<unsigned char> d_cfg_dirty;
     // recordings
-    float2* d_rec_dec = nullptr; float2* d_rec_filt = nullptr; size_t rec_pitch = 0;
-    unsigned char* d_rec_bits = nullptr; unsigned* d_rec_bits_n = nullptr; unsigned rec_bits_pitch = 0;
+    Rows<float2, 2> rec;         // [0] decimated, [1] filtered
+    DevPtr<unsigned char> d_rec_bits; DevPtr<unsigned> d_rec_bits_n; unsigned rec_bits_pitch = 0;
 
     // input (push)
-    float2* d_stage = nullptr; size_t stage_pitch = 0;   // host pushes land here
+    Rows<float2> stage;          // host pushes land here
     // A device push that K1 reads in place at the next process call (p == nullptr: K1 reads the staging matrix).
     // format: integers that K1 reads itself (decim1_supports_native_iq).  nco: raw samples that K1 mixes through the
     // channels' NCOs (fused K0); pitch 0 is one wideband row shared by all channels.
     struct DeviceInput { const void* p = nullptr; size_t pitch = 0, n = 0; int format = HBD_IQ_CF32; const NcoChan* nco = nullptr; } in;
     int push(const PushSrc& s);
-    // Host integers are uploaded to d_iq_up.  d_widen holds cf32: widened device integers, and wideband rows that do not
+    // Host integers are uploaded to iq_up.  d_widen() holds cf32: widened device integers, and wideband rows that do not
     // arrive as device cf32.
-    unsigned char* d_iq_up = nullptr; size_t iq_up_bytes = 0;
-    float2* d_widen = nullptr; size_t widen_bytes = 0;
-    int ensure_scratch(void** p, size_t* cap, size_t bytes);
+    // One row of `pitch` bytes each, grown with grow(bytes, 1, 0, stream): what they held is dropped, and the old buffer is
+    // released only after `stream` has caught up (a kernel of an earlier push may still read it).
+    Rows<unsigned char> iq_up, widen_buf;
+    float2* d_widen() const { return reinterpret_cast<float2*>(widen_buf.get()); }
     int widen(const void* src, size_t pitch, int format, int rows, size_t n, size_t* out_pitch);
     // fused-NCO parameter ring: pinned host slots + device slots, so a push never waits for the GPU
     static constexpr unsigned kNcoSlots = 16;
-    NcoChan* h_nco_pin = nullptr; NcoChan* d_nco_ring = nullptr; cudaEvent_t ev_nco[kNcoSlots] = {}; unsigned nco_seq = 0;
+    HostPtr<NcoChan> h_nco_pin; DevPtr<NcoChan> d_nco_ring; Event ev_nco[kNcoSlots]; unsigned nco_seq = 0;
     bool nco_fused = true;   // HBD_NCO_FUSED=0 (measurement / test hook): always pre-mix with K0 into the staging matrix
 
     // websocket wire formats (wire.cu)
     bool demod_acc_on = false;
-    float* d_dacc = nullptr; size_t dacc_pitch = 0; unsigned* d_dacc_n = nullptr;
-    unsigned char* d_frames = nullptr; size_t frames_pitch = 0; unsigned* d_frame_sizes = nullptr;
+    Rows<float> dacc; DevPtr<unsigned> d_dacc_n;
+    DevPtr<unsigned char> d_frames; size_t frames_pitch = 0; DevPtr<unsigned> d_frame_sizes;
     std::vector<unsigned> h_frame_sizes;
     int ensure_frames(size_t pitch);
     int ensure_dacc();
     // NCO pre-mixer (nco.cu)
-    NcoChan* d_nco = nullptr; std::vector<NcoChan> h_nco;
+    DevPtr<NcoChan> d_nco; std::vector<NcoChan> h_nco;
     bool nco_any = false;    // some channel has (had) a non-zero NCO frequency or phase (set by hbd_set_nco, never cleared)
     void nco_params(NcoChan* out, int c0, int nc, size_t n, bool k0_rotation);
     int mix_into_stage(const void* src, size_t src_pitch, int c0, int nc, size_t dst_off, size_t n, int format = HBD_IQ_CF32);
@@ -328,19 +332,19 @@ struct hbd_decoder {
     bool mask_cache = true;      // HBD_MASK_CACHE=0 (test hook): the slicer's position masks are rebuilt from scratch in every call
     // optional per-kernel CUDA-event timing (bench roofline): one event pair per K1 launch / per rest-of-step
     int timing = 0;          // 0 off, 1: events around K1 only (what the roofline needs), 2: also around the rest of the step (pipeline diagnostics)
-    std::vector<cudaEvent_t> ev_k1, ev_rest; // pairs: [2i] start, [2i+1] stop
+    std::vector<Event> ev_k1, ev_rest;   // pairs: [2i] start, [2i+1] stop
     size_t ev_used_k1 = 0, ev_used_rest = 0;
-    cudaEvent_t next_event(std::vector<cudaEvent_t>& pool, size_t& used)
+    cudaEvent_t next_event(std::vector<Event>& pool, size_t& used)
     {
-        if (used == pool.size()) { cudaEvent_t e; cudaEventCreate(&e); pool.push_back(e); }
-        return pool[used++];
+        if (used == pool.size()) { pool.emplace_back(); event_create(pool.back(), cudaEventDefault); }
+        return pool[used++].get();
     }
     size_t cap_n_in = 0;     // largest (r + n) the per-call buffers are sized for
 
     // SSDV packet sync (ssdv.cu + host_tail.cpp SsdvChannel); off until hbd_set_ssdv / hbd_set_ssdv_callback
     bool ssdv_on = false;
-    unsigned char* d_ssdv_ring = nullptr; unsigned* d_ssdv_total = nullptr; unsigned* d_ssdv_scanned = nullptr;
-    SsdvLogEntry* d_ssdv_log = nullptr; unsigned ssdv_log_tail = 0;
+    DevPtr<unsigned char> d_ssdv_ring; DevPtr<unsigned> d_ssdv_total, d_ssdv_scanned;
+    DevPtr<SsdvLogEntry> d_ssdv_log; unsigned ssdv_log_tail = 0;
     std::vector<SsdvLogEntry> h_ssdv_log;
     std::vector<SsdvChannel> ssdv;
     hbd_ssdv_cb ssdv_cb = nullptr; void* ssdv_user = nullptr;
@@ -354,10 +358,10 @@ struct hbd_decoder {
     // ring, so that a drain can read the values that belong to the calls it drains without stopping the pipeline
     static constexpr unsigned kSnapSlots = 32;
     bool snap_on = false;
-    float* d_snap = nullptr;         // [kSnapSlots][n][6]
-    float* h_snap = nullptr;         // pinned, [n][6]: snapshot of the newest drained call
+    DevPtr<float> d_snap;            // [kSnapSlots][n][6]
+    HostPtr<float> h_snap;           // pinned, [n][6]: snapshot of the newest drained call
     bool h_snap_valid = false;
-    void* dist_ctx = nullptr;        // dist.cu
+    DistSlot dist_ctx;               // dist.cu
     int enable_snap();
 
     void set_error(const std::string& e) { err = e; }
@@ -369,7 +373,6 @@ struct hbd_decoder {
     int process_async_locked();
     int collect_locked(unsigned lag);
     int log_pressure();
-    void free_all();
 };
 
 // Runs `body` (a lambda returning int) under the handle's mutex, then fires the callbacks it recorded with the mutex
@@ -419,36 +422,10 @@ static void fill_ssdv_info(hbd_ssdv_packet_info& info, const SsdvEvent& ev)
 #define HBD_CHECK_H(h)  if (!(h)) return HBD_ERR_ARG
 #define HBD_CHECK_CH(h, ch) if (!(h) || (ch) < 0 || (ch) >= (h)->n_ch) return HBD_ERR_ARG
 
-template <typename T>
-static cudaError_t dalloc(T** p, size_t count) { return cudaMalloc((void**)p, std::max<size_t>(count, 1) * sizeof(T)); }
-
-// grow a [rows][pitch] device matrix, keeping the first `keep` elements of every row
-template <typename T>
-static cudaError_t grow_rows(T** p, size_t* pitch, size_t new_pitch, size_t rows, size_t keep, cudaStream_t s)
-{
-    if (new_pitch <= *pitch && *p) return cudaSuccess;
-    T* np = nullptr;
-    cudaError_t e = cudaMalloc((void**)&np, rows * new_pitch * sizeof(T));
-    if (e != cudaSuccess) return e;
-    e = cudaMemsetAsync(np, 0, rows * new_pitch * sizeof(T), s);
-    if (e != cudaSuccess) return e;
-    if (*p && keep) {
-        e = cudaMemcpy2DAsync(np, new_pitch * sizeof(T), *p, *pitch * sizeof(T), std::min(keep, *pitch) * sizeof(T), rows,
-                              cudaMemcpyDeviceToDevice, s);
-        if (e != cudaSuccess) return e;
-    }
-    e = cudaStreamSynchronize(s);
-    if (e != cudaSuccess) return e;
-    if (*p) cudaFree(*p);
-    *p = np;
-    *pitch = new_pitch;
-    return cudaSuccess;
-}
-
 int hbd_decoder::alloc_fixed()
 {
     const size_t n = size_t(n_ch);
-    HBD_CUDA_CHECK(dalloc(&d_state, n));
+    HBD_CUDA_CHECK(dev_alloc(d_state, n));
     {
         // Average<T>'s constructor add()s one 0: count starts at 1 (Average.h:34-37)
         ChanState init;
@@ -456,72 +433,75 @@ int hbd_decoder::alloc_fixed()
         init.baud = 1; // SymbolExtractor.h:96
         init.nf_cnt = init.nv_cnt = init.pl_cnt = init.pr_cnt = 1;
         std::vector<ChanState> all(n, init);
-        HBD_CUDA_CHECK(cudaMemcpy(d_state, all.data(), n * sizeof(ChanState), cudaMemcpyHostToDevice));
+        HBD_CUDA_CHECK(cudaMemcpy(d_state.get(), all.data(), n * sizeof(ChanState), cudaMemcpyHostToDevice));
     }
-    HBD_CUDA_CHECK(dalloc(&d_plan, n));
-    for (int i = 0; i < 2; ++i) {
-        HBD_CUDA_CHECK(dalloc(&d_carry2[i], n * size_t(carry_cap)));
-        HBD_CUDA_CHECK(cudaMemset(d_carry2[i], 0, n * size_t(carry_cap) * sizeof(float2)));
+    HBD_CUDA_CHECK(dev_alloc(d_plan, n));
+    for (DevPtr<float2>& c : d_carry2) {
+        HBD_CUDA_CHECK(dev_alloc(c, n * size_t(carry_cap)));
+        HBD_CUDA_CHECK(cudaMemset(c.get(), 0, n * size_t(carry_cap) * sizeof(float2)));
     }
-    { const int rc = alloc_fft(); if (rc) return rc; }
-    HBD_CUDA_CHECK(dalloc(&d_uart_runs, n * size_t(kUartRunsCap)));
-    HBD_CUDA_CHECK(dalloc(&d_maskc, n * size_t(2 * kMaskWords)));
-    HBD_CUDA_CHECK(dalloc(&d_lptaps, n * kLpMaxTaps));
-    HBD_CUDA_CHECK(cudaMemset(d_lptaps, 0, n * kLpMaxTaps * sizeof(float)));
+    { const int rc = make_fft(fft_n, fft); if (rc) return rc; }
+    HBD_CUDA_CHECK(dev_alloc(d_uart_runs, n * size_t(kUartRunsCap)));
+    HBD_CUDA_CHECK(dev_alloc(d_maskc, n * size_t(2 * kMaskWords)));
+    HBD_CUDA_CHECK(dev_alloc(d_lptaps, n * kLpMaxTaps));
+    HBD_CUDA_CHECK(cudaMemset(d_lptaps.get(), 0, n * kLpMaxTaps * sizeof(float)));
     // character log: at least 512 entries per channel (a 600 baud channel decodes ~2 characters per 65 536-sample call,
     // so that is > 250 calls between drains even when every channel is noise); log_pressure() drains before it fills
     log_cap = kLogCapMin;
     while (size_t(log_cap) < 512 * n && log_cap < (1u << 30)) log_cap <<= 1;
-    HBD_CUDA_CHECK(dalloc(&d_log, size_t(log_cap)));
-    HBD_CUDA_CHECK(dalloc(&d_log_ctl, size_t(kCtlWords)));
-    HBD_CUDA_CHECK(cudaMemset(d_log_ctl, 0, kCtlWords * sizeof(unsigned)));
-    HBD_CUDA_CHECK(cudaStreamCreateWithFlags(&copy_stream, cudaStreamNonBlocking));
+    HBD_CUDA_CHECK(dev_alloc(d_log, size_t(log_cap)));
+    HBD_CUDA_CHECK(dev_alloc(d_log_ctl, size_t(kCtlWords)));
+    HBD_CUDA_CHECK(cudaMemset(d_log_ctl.get(), 0, kCtlWords * sizeof(unsigned)));
+    HBD_CUDA_CHECK(stream_create(copy_stream));
     ev_call.resize(kMaxCallsBetweenCollects * 2);
-    for (auto& e : ev_call) HBD_CUDA_CHECK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    HBD_CUDA_CHECK(cudaHostAlloc((void**)&h_heads, ev_call.size() * kCtlWords * sizeof(unsigned), cudaHostAllocDefault));
-    memset(h_heads, 0, ev_call.size() * kCtlWords * sizeof(unsigned));
-    HBD_CUDA_CHECK(cudaHostAlloc((void**)&h_tail_pin, 2 * sizeof(unsigned), cudaHostAllocDefault));
+    for (Event& e : ev_call) HBD_CUDA_CHECK(event_create(e));
+    HBD_CUDA_CHECK(host_alloc(h_heads, ev_call.size() * kCtlWords));
+    memset(h_heads.get(), 0, ev_call.size() * kCtlWords * sizeof(unsigned));
+    HBD_CUDA_CHECK(host_alloc(h_tail_pin, 2));
     call_chars.resize(n);
-    HBD_CUDA_CHECK(dalloc(&d_taps1, 512));
-    HBD_CUDA_CHECK(dalloc(&d_taps2, 512));
-    HBD_CUDA_CHECK(dalloc(&d_cfg_baud, n));
-    HBD_CUDA_CHECK(dalloc(&d_cfg_stops, n));
-    HBD_CUDA_CHECK(dalloc(&d_cfg_bits, n));
-    HBD_CUDA_CHECK(dalloc(&d_cfg_dc, n));
-    HBD_CUDA_CHECK(dalloc(&d_cfg_ntaps, n));
-    HBD_CUDA_CHECK(dalloc(&d_cfg_dirty, n));
-    HBD_CUDA_CHECK(dalloc(&d_nco, n));
+    HBD_CUDA_CHECK(dev_alloc(d_taps1, 512));
+    HBD_CUDA_CHECK(dev_alloc(d_taps2, 512));
+    HBD_CUDA_CHECK(dev_alloc(d_cfg_baud, n));
+    HBD_CUDA_CHECK(dev_alloc(d_cfg_stops, n));
+    HBD_CUDA_CHECK(dev_alloc(d_cfg_bits, n));
+    HBD_CUDA_CHECK(dev_alloc(d_cfg_dc, n));
+    HBD_CUDA_CHECK(dev_alloc(d_cfg_ntaps, n));
+    HBD_CUDA_CHECK(dev_alloc(d_cfg_dirty, n));
+    HBD_CUDA_CHECK(dev_alloc(d_nco, n));
     h_nco.resize(n);
+    HBD_CUDA_CHECK(dev_alloc(d_dacc_n, n));
+    HBD_CUDA_CHECK(cudaMemset(d_dacc_n.get(), 0, n * sizeof(unsigned)));
+    HBD_CUDA_CHECK(dev_alloc(d_frame_sizes, n));
+    h_frame_sizes.resize(n);
     return HBD_OK;
 }
 
-// spectrum buffers + twiddle table for the current fft_n (also called by hbd_set_fft_size)
-int hbd_decoder::alloc_fft()
+// spectrum buffers + twiddle table of an N-point spectrum into `f` (hbd_create, hbd_set_fft_size)
+int hbd_decoder::make_fft(int N_, FftBufs& f)
 {
-    const size_t n = size_t(n_ch), N = size_t(fft_n);
-    for (void* p : {(void*)d_fftbuf, (void*)d_spectrum, (void*)d_power, (void*)d_twiddle}) if (p) cudaFree(p);
-    d_fftbuf = d_spectrum = nullptr; d_power = nullptr; d_twiddle = nullptr;
-    HBD_CUDA_CHECK(dalloc(&d_fftbuf, n * N));
-    HBD_CUDA_CHECK(cudaMemset(d_fftbuf, 0, n * N * sizeof(float2)));
-    HBD_CUDA_CHECK(dalloc(&d_spectrum, n * N));
-    HBD_CUDA_CHECK(cudaMemset(d_spectrum, 0, n * N * sizeof(float2)));
-    HBD_CUDA_CHECK(dalloc(&d_power, n * N));
-    HBD_CUDA_CHECK(cudaMemset(d_power, 0, n * N * sizeof(float)));
+    const size_t n = size_t(n_ch), N = size_t(N_);
+    HBD_CUDA_CHECK(dev_alloc(f.buf, n * N));
+    HBD_CUDA_CHECK(cudaMemset(f.buf.get(), 0, n * N * sizeof(float2)));
+    HBD_CUDA_CHECK(dev_alloc(f.spectrum, n * N));
+    HBD_CUDA_CHECK(cudaMemset(f.spectrum.get(), 0, n * N * sizeof(float2)));
+    HBD_CUDA_CHECK(dev_alloc(f.power, n * N));
+    HBD_CUDA_CHECK(cudaMemset(f.power.get(), 0, n * N * sizeof(float)));
     // [0, N): exp(-2 pi i e / N); behind it the twiddles of the 4096-point (sub-)transform in the order its threads read
     // them: pass 1 [k1][t] = W_4096^(t k1) (16 x 256), pass 2 [j1][m2] = W_256^(m2 j1) (16 x 16); all evaluated in float64
-    HBD_CUDA_CHECK(dalloc(&d_twiddle, N + 4096 + 256));
+    HBD_CUDA_CHECK(dev_alloc(f.twiddle, N + 4096 + 256));
     std::vector<float2> tw(N + 4096 + 256);
     auto w = [](double num, double den) { const double ang = -2.0 * M_PI * num / den; return make_float2(float(std::cos(ang)), float(std::sin(ang))); };
     for (size_t e = 0; e < N; ++e) tw[e] = w(double(e), double(N));
     for (size_t k1 = 0; k1 < 16; ++k1) for (size_t t = 0; t < 256; ++t) tw[N + k1 * 256 + t] = w(double(t * k1), 4096.0);
     for (size_t j1 = 0; j1 < 16; ++j1) for (size_t m2 = 0; m2 < 16; ++m2) tw[N + 4096 + j1 * 16 + m2] = w(double(16 * m2 * j1), 4096.0);
-    HBD_CUDA_CHECK(cudaMemcpy(d_twiddle, tw.data(), sizeof(float2) * tw.size(), cudaMemcpyHostToDevice));
+    HBD_CUDA_CHECK(cudaMemcpy(f.twiddle.get(), tw.data(), sizeof(float2) * tw.size(), cudaMemcpyHostToDevice));
     return HBD_OK;
 }
 
 // Install a decimation plan (a list of (M, taps) stages with the given total factor): K1 runs stages[0], the tail kernel the
 // last stage, mid.cu the ones in between.  A new plan starts from fresh decimators (Decoder.h:283-284,347-348:
 // decimation_stages_.clear()); unconsumed input stays queued (iq_in_buffer_ is untouched) -- it sits at the end of the carry.
+// Taps and carry of the new plan go into locals first: on failure the previous plan stays in force.
 int hbd_decoder::set_plan(const std::vector<TapTable>& st, size_t total_factor)
 {
     HBD_CUDA_CHECK(cudaSetDevice(device));
@@ -529,117 +509,97 @@ int hbd_decoder::set_plan(const std::vector<TapTable>& st, size_t total_factor)
     HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
     const size_t n = size_t(n_ch);
     sync_ctrs();
-    const int old_cap = carry_cap;
-    factor = int(total_factor);
-    M1 = T1 = M2 = T2 = 1;
-    if (!st.empty()) {
-        M1 = st[0].M; T1 = st[0].len;
-        HBD_CUDA_CHECK(cudaMemcpy(d_taps1, st[0].bits, 4 * size_t(T1), cudaMemcpyHostToDevice));
-    }
-    if (st.size() >= 2) {
-        M2 = st.back().M; T2 = st.back().len;
-        HBD_CUDA_CHECK(cudaMemcpy(d_taps2, st.back().bits, 4 * size_t(T2), cudaMemcpyHostToDevice));
-    }
-    for (MidStage& m : mids) { if (m.d_taps) cudaFree(m.d_taps); if (m.d_out) cudaFree(m.d_out); }
-    mids.clear();
-    for (int i = 0; i < 2; ++i) { if (d_midlast[i]) cudaFree(d_midlast[i]); d_midlast[i] = nullptr; }
-    midlast_pitch = midlast_pitch_b = 0;
-    unsigned div = unsigned(M1);
+    const TapTable none{1, nullptr, 1};   // M == 1: no such stage (a plan without one keeps the tap buffer it has)
+    const TapTable &first = st.empty() ? none : st[0], &last = st.size() >= 2 ? st.back() : none;
+    auto upload = [](DevPtr<float>& d, const TapTable& t, size_t cap) {
+        cudaError_t e = t.bits ? dev_alloc(d, cap) : cudaSuccess;
+        if (e == cudaSuccess && t.bits) e = cudaMemcpy(d.get(), t.bits, 4 * size_t(t.len), cudaMemcpyHostToDevice);
+        return e;
+    };
+    DevPtr<float> taps1, taps2;
+    HBD_CUDA_CHECK(upload(taps1, first, 512));
+    HBD_CUDA_CHECK(upload(taps2, last, 512));
+    std::vector<MidStage> new_mids;
+    unsigned div = unsigned(first.M);
     for (size_t k = 1; k + 1 < st.size(); ++k) {
         MidStage m;
         m.M = st[k].M; m.T = st[k].len; m.div_in = div;
-        HBD_CUDA_CHECK(dalloc(&m.d_taps, size_t(m.T)));
-        HBD_CUDA_CHECK(cudaMemcpy(m.d_taps, st[k].bits, 4 * size_t(m.T), cudaMemcpyHostToDevice));
-        mids.push_back(m);
-        div *= unsigned(m.M);
+        HBD_CUDA_CHECK(upload(m.d_taps, st[k], size_t(m.T)));
+        new_mids.push_back(std::move(m));
+        div *= unsigned(st[k].M);
     }
     // the carry holds T1-1 samples of history plus the unconsumed remainder (< total factor).  Fresh, zeroed rows (new
     // decimators have an empty history); the remainder queued under the old plan stays queued, as in the reference
     unsigned max_r = 0;
     for (const auto& x : hc) max_r = std::max(max_r, x.in_r);
-    carry_cap = std::max(kCarryCapMin, int((size_t(T1) + std::max<size_t>(total_factor, max_r) + 64 + 63) & ~size_t(63)));
-    float2* fresh[2] = {nullptr, nullptr};
-    for (int i = 0; i < 2; ++i) {
-        HBD_CUDA_CHECK(cudaMalloc((void**)&fresh[i], n * size_t(carry_cap) * sizeof(float2)));
-        HBD_CUDA_CHECK(cudaMemset(fresh[i], 0, n * size_t(carry_cap) * sizeof(float2)));
+    const int cap = std::max(kCarryCapMin, int((size_t(first.len) + std::max<size_t>(total_factor, max_r) + 64 + 63) & ~size_t(63)));
+    DevPtr<float2> fresh[2];
+    for (DevPtr<float2>& f : fresh) {
+        HBD_CUDA_CHECK(dev_alloc(f, n * size_t(cap)));
+        HBD_CUDA_CHECK(cudaMemset(f.get(), 0, n * size_t(cap) * sizeof(float2)));
     }
     for (size_t c = 0; c < n; ++c)
         if (hc[c].in_r)
-            HBD_CUDA_CHECK(cudaMemcpy(fresh[carry_cur] + c * size_t(carry_cap) + size_t(carry_cap) - hc[c].in_r,
-                                      d_carry2[carry_cur] + c * size_t(old_cap) + size_t(old_cap) - hc[c].in_r, sizeof(float2) * hc[c].in_r, cudaMemcpyDeviceToDevice));
-    for (int i = 0; i < 2; ++i) { cudaFree(d_carry2[i]); d_carry2[i] = fresh[i]; }
-    for (int i = 0; i < 2; ++i) if (d_s1x[i]) HBD_CUDA_CHECK(cudaMemset(d_s1x[i], 0, n * s1_pitch * sizeof(float2)));
+            HBD_CUDA_CHECK(cudaMemcpy(fresh[carry_cur].get() + c * size_t(cap) + size_t(cap) - hc[c].in_r,
+                                      d_carry2[carry_cur].get() + c * size_t(carry_cap) + size_t(carry_cap) - hc[c].in_r, sizeof(float2) * hc[c].in_r,
+                                      cudaMemcpyDeviceToDevice));
+    for (int i = 0; i < 2; ++i) if (s1x.get(i)) HBD_CUDA_CHECK(cudaMemset(s1x.get(i), 0, n * s1x.pitch * sizeof(float2)));
+    // commit
+    factor = int(total_factor);
+    M1 = first.M; T1 = first.len; M2 = last.M; T2 = last.len;
+    if (taps1) d_taps1 = std::move(taps1);
+    if (taps2) d_taps2 = std::move(taps2);
+    mids = std::move(new_mids);
+    midlast = {};
+    carry_cap = cap;
+    for (int i = 0; i < 2; ++i) d_carry2[i] = std::move(fresh[i]);
     for (auto& x : hc) { x.grown1 = x.grown2 = 0; for (size_t& g : x.grown_mid) g = 0; }
     cap_n_in = 0;
     h_plan_uploaded.clear();
     return HBD_OK;
 }
 
-void hbd_decoder::free_all()
-{
-    cudaSetDevice(device);
-    sync_groups();
-    if (stream) cudaStreamSynchronize(stream);
-    if (hi) cudaStreamDestroy(hi);
-    if (lo) cudaStreamDestroy(lo);
-    if (ev_consumed) cudaEventDestroy(ev_consumed);
-    for (cudaEvent_t e : ev_tail) if (e) cudaEventDestroy(e);
-    if (ev_in) cudaEventDestroy(ev_in);
-    void* ptrs[] = {d_state, d_plan, d_carry2[0], d_carry2[1], d_s1x[0], d_s1x[1], d_decq, d_fftbuf, d_spectrum, d_power, d_lptaps, d_slicer, d_demod, d_uart_runs, d_maskc, d_log, d_log_ctl,
-                    d_taps1, d_taps2, d_twiddle, d_cfg_baud, d_cfg_stops, d_cfg_bits, d_cfg_dc, d_cfg_ntaps,
-                    d_cfg_dirty, d_rec_dec, d_rec_filt, d_rec_bits, d_rec_bits_n, d_stage, d_nco, d_iq_up, d_widen, d_dacc, d_dacc_n, d_frames, d_frame_sizes,
-                    d_ssdv_ring, d_ssdv_total, d_ssdv_scanned, d_ssdv_log};
-    for (void* p : ptrs) if (p) cudaFree(p);
-    for (MidStage& m : mids) { if (m.d_taps) cudaFree(m.d_taps); if (m.d_out) cudaFree(m.d_out); }
-    for (int i = 0; i < 2; ++i) if (d_midlast[i]) cudaFree(d_midlast[i]);
-    if (dist_ctx) { internal_free_dist(dist_ctx); dist_ctx = nullptr; }
-    if (d_snap) cudaFree(d_snap);
-    if (h_snap) cudaFreeHost(h_snap);
-    if (h_heads) cudaFreeHost(h_heads);
-    if (h_tail_pin) cudaFreeHost(h_tail_pin);
-    for (cudaEvent_t e : ev_call) cudaEventDestroy(e);
-    if (copy_stream) cudaStreamDestroy(copy_stream);
-    for (cudaEvent_t e : ev_k1) cudaEventDestroy(e);
-    for (cudaEvent_t e : ev_rest) cudaEventDestroy(e);
-    if (h_nco_pin) { cudaFreeHost(h_nco_pin); h_nco_pin = nullptr; }
-    if (d_nco_ring) { cudaFree(d_nco_ring); d_nco_ring = nullptr; }
-    for (cudaEvent_t& e : ev_nco) if (e) { cudaEventDestroy(e); e = nullptr; }
-    if (own_stream && stream) cudaStreamDestroy(stream);
-}
-
-// size the per-call buffers for pushes of up to n_in_max (carried + new) samples per channel
+// size the per-call buffers for pushes of up to n_in_max (carried + new) samples per channel.  Every matrix that grows is
+// filled into a local first; they are swapped in together once all of them are ready.
 int hbd_decoder::ensure_call_capacity(size_t n_in_max)
 {
-    if (n_in_max <= cap_n_in && d_s1x[0]) return HBD_OK;
+    if (n_in_max <= cap_n_in && s1x.get()) return HBD_OK;
     const size_t n = size_t(n_ch);
     const size_t grow_to = std::max(n_in_max, cap_n_in);
     const size_t n1_max = grow_to / size_t(M1) + 2, n2_max = grow_to / size_t(factor) + 2;
-    HBD_CUDA_CHECK(grow_rows(&d_s1x[0], &s1_pitch, (kS1Hist + n1_max + 15) & ~size_t(15), n, kS1Hist, stream));
-    HBD_CUDA_CHECK(grow_rows(&d_s1x[1], &s1_pitch_b, (kS1Hist + n1_max + 15) & ~size_t(15), n, kS1Hist, stream));
+    bool grown = false;
+    auto regrow = [&](const auto& cur, auto& next, size_t width, size_t keep) {
+        const cudaError_t e = cur.regrow(next, (width + 15) & ~size_t(15), n, keep, stream);
+        grown = grown || next.p[0];
+        return e;
+    };
+    Rows<float2, 2> s1, ml, rc;
+    std::vector<Rows<float2>> mo(mids.size());
+    Rows<float2> dq; Rows<float> sl, dm;
+    HBD_CUDA_CHECK(regrow(s1x, s1, kS1Hist + n1_max, kS1Hist));
     for (size_t k = 0; k < mids.size(); ++k) {   // cascaded plan: the buffers between the stages
         const size_t n_out_max = grow_to / (size_t(mids[k].div_in) * size_t(mids[k].M)) + 2;
-        if (k + 1 < mids.size()) HBD_CUDA_CHECK(grow_rows(&mids[k].d_out, &mids[k].pitch, (kMidHist + n_out_max + 15) & ~size_t(15), n, kMidHist, stream));
-        else {
-            HBD_CUDA_CHECK(grow_rows(&d_midlast[0], &midlast_pitch, (kS1Hist + n_out_max + 15) & ~size_t(15), n, kS1Hist, stream));
-            HBD_CUDA_CHECK(grow_rows(&d_midlast[1], &midlast_pitch_b, (kS1Hist + n_out_max + 15) & ~size_t(15), n, kS1Hist, stream));
-        }
+        if (k + 1 < mids.size()) HBD_CUDA_CHECK(regrow(mids[k].out, mo[k], kMidHist + n_out_max, kMidHist));
+        else HBD_CUDA_CHECK(regrow(midlast, ml, kS1Hist + n_out_max, kS1Hist));
     }
-    HBD_CUDA_CHECK(grow_rows(&d_decq, &dq_pitch, (kLpHist + kLpBatch + n2_max + 15) & ~size_t(15), n, kLpHist + kLpBatch, stream));
-    HBD_CUDA_CHECK(grow_rows(&d_slicer, &slicer_pitch, (size_t(kSlicerVent) + 1 + kLpBatch + n2_max + 15) & ~size_t(15), n,
-                             slicer_pitch, stream));
-    HBD_CUDA_CHECK(grow_rows(&d_demod, &demod_pitch, (kLpBatch + n2_max + 15) & ~size_t(15), n, 0, stream));
+    HBD_CUDA_CHECK(regrow(decq, dq, kLpHist + kLpBatch + n2_max, kLpHist + kLpBatch));
+    HBD_CUDA_CHECK(regrow(slicer, sl, size_t(kSlicerVent) + 1 + kLpBatch + n2_max, slicer.pitch));
+    HBD_CUDA_CHECK(regrow(demod, dm, kLpBatch + n2_max, 0));
+    DevPtr<unsigned char> bits; DevPtr<unsigned> bits_n;
     if (record) {
-        HBD_CUDA_CHECK(grow_rows(&d_rec_dec, &rec_pitch, (kLpBatch + n2_max + 15) & ~size_t(15), n, 0, stream));
-        size_t p2 = 0;
-        if (d_rec_filt) { cudaFree(d_rec_filt); d_rec_filt = nullptr; }
-        HBD_CUDA_CHECK(grow_rows(&d_rec_filt, &p2, rec_pitch, n, 0, stream));
+        HBD_CUDA_CHECK(regrow(rec, rc, kLpBatch + n2_max, 0));
         if (!d_rec_bits) {
-            rec_bits_pitch = 1u << 16;
-            HBD_CUDA_CHECK(dalloc(&d_rec_bits, n * rec_bits_pitch));
-            HBD_CUDA_CHECK(dalloc(&d_rec_bits_n, n));
-            HBD_CUDA_CHECK(cudaMemset(d_rec_bits_n, 0, n * sizeof(unsigned)));
+            HBD_CUDA_CHECK(dev_alloc(bits, n * (size_t(1) << 16)));
+            HBD_CUDA_CHECK(dev_alloc(bits_n, n));
+            HBD_CUDA_CHECK(cudaMemset(bits_n.get(), 0, n * sizeof(unsigned)));
         }
     }
+    if (grown) HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
+    s1x.commit(s1);
+    for (size_t k = 0; k < mids.size(); ++k) mids[k].out.commit(mo[k]);
+    midlast.commit(ml);
+    decq.commit(dq); slicer.commit(sl); demod.commit(dm); rec.commit(rc);
+    if (bits) { d_rec_bits = std::move(bits); d_rec_bits_n = std::move(bits_n); rec_bits_pitch = 1u << 16; }
     cap_n_in = grow_to;
     return HBD_OK;
 }
@@ -720,8 +680,8 @@ static int step_channel(hbd_decoder* h, HostChan& x, unsigned pushed, ChanStep& 
 // flight could exhaust the space that is left.
 int hbd_decoder::log_pressure()
 {
-    while (done_seq != call_seq && cudaEventQuery(ev_call[done_seq % ev_call.size()]) == cudaSuccess) {
-        const unsigned head = h_heads[size_t(done_seq % ev_call.size()) * kCtlWords + kCtlCharHead];
+    while (done_seq != call_seq && cudaEventQuery(ev_call[done_seq % ev_call.size()].get()) == cudaSuccess) {
+        const unsigned head = h_heads.get()[size_t(done_seq % ev_call.size()) * kCtlWords + kCtlCharHead];
         per_call_max = std::max(per_call_max, head - done_head);
         done_head = head;
         ++done_seq;
@@ -730,7 +690,7 @@ int hbd_decoder::log_pressure()
     const unsigned long long worst = (unsigned long long)(done_head - log_tail) + 2ull * in_flight * std::max(per_call_max, unsigned(n_ch));
     bool drain = worst > log_cap;
     if (ssdv_on && done_seq) {
-        const unsigned sh = h_heads[size_t((done_seq - 1u) % ev_call.size()) * kCtlWords + kCtlSsdvHead];
+        const unsigned sh = h_heads.get()[size_t((done_seq - 1u) % ev_call.size()) * kCtlWords + kCtlSsdvHead];
         if (sh - ssdv_log_tail > kSsdvLogCap / 2u) drain = true;
     }
     if (call_seq - calls_collected >= ev_call.size() / 2u) drain = true;   // event / head slots are about to be reused
@@ -747,20 +707,20 @@ int hbd_decoder::apply_step(const ChanStep& st, size_t c0, size_t rows, const st
     auto zero = [&](float2* p, size_t pitch, size_t w) {   // w samples from p on, in each of the rows of a [n_ch][pitch] matrix
         return cudaMemset2DAsync(p + c0 * pitch, pitch * sizeof(float2), 0, w * sizeof(float2), rows, stream);
     };
-    if (st.zero_carry) HBD_CUDA_CHECK(zero(d_carry2[carry_cur] + (carry_cap - (T1 - 1) - int(st.plan.r)), size_t(carry_cap), size_t(T1 - 1)));
+    if (st.zero_carry) HBD_CUDA_CHECK(zero(d_carry2[carry_cur].get() + (carry_cap - (T1 - 1) - int(st.plan.r)), size_t(carry_cap), size_t(T1 - 1)));
     for (size_t k = 0; k < mids.size(); ++k)
         if (st.zero_mid & (1u << k)) { const StageRows s = stage_in(k); HBD_CUDA_CHECK(zero(s.p, s.pitch, size_t(s.hist))); }
     if (st.zero_s1hist) { const StageRows s = stage_in(mids.size()); HBD_CUDA_CHECK(zero(s.p, s.pitch, size_t(s.hist))); }
     if (st.taps_changed) {
         std::vector<float> all(rows * st.taps_new);
         for (size_t c = 0; c < rows; ++c) memcpy(all.data() + c * st.taps_new, taps.data(), 4 * st.taps_new);
-        HBD_CUDA_CHECK(cudaMemcpy2DAsync(d_lptaps + c0 * kLpMaxTaps, kLpMaxTaps * sizeof(float), all.data(), st.taps_new * sizeof(float), st.taps_new * sizeof(float), rows,
+        HBD_CUDA_CHECK(cudaMemcpy2DAsync(d_lptaps.get() + c0 * kLpMaxTaps, kLpMaxTaps * sizeof(float), all.data(), st.taps_new * sizeof(float), st.taps_new * sizeof(float), rows,
                                          cudaMemcpyHostToDevice, stream));
         HBD_CUDA_CHECK(cudaStreamSynchronize(stream)); // `all` goes out of scope
         for (size_t c = c0; c < c0 + rows; ++c) hc[c].cfg_dirty = true;   // lp_ntaps travels with the configuration upload
         cfg_dirty_any = true;
     }
-    if (st.zero_lphist) HBD_CUDA_CHECK(zero(d_decq, dq_pitch, std::min<size_t>(st.plan.lp_ntaps, kLpHist)));
+    if (st.zero_lphist) HBD_CUDA_CHECK(zero(decq.get(), decq.pitch, std::min<size_t>(st.plan.lp_ntaps, kLpHist)));
     return HBD_OK;
 }
 
@@ -777,7 +737,7 @@ int hbd_decoder::plan_call(CallPlan& cp)
     auto pushed = [&](size_t c) { return in.p ? unsigned(in.n) : hc[c].pushed; };
     size_t max_total = 0;
     for (size_t c = 0; c < stepped; ++c) max_total = std::max<size_t>(max_total, size_t(hc[c].in_r) + pushed(c));
-    if (max_total > cap_n_in || !d_s1x[0]) { if (quiesce()) return HBD_ERR_CUDA; }   // buffers are about to be reallocated
+    if (max_total > cap_n_in || !s1x.get()) { if (quiesce()) return HBD_ERR_CUDA; }   // buffers are about to be reallocated
     { const int rc = ensure_call_capacity(max_total); if (rc) return rc; }
     unsigned max_nf = 0;
     std::vector<float> new_taps;
@@ -801,13 +761,13 @@ int hbd_decoder::plan_call(CallPlan& cp)
             b[c] = hc[c].baud; s[c] = hc[c].rtty_stops; bi[c] = int(hc[c].rtty_bits); dc[c] = hc[c].dc_remove; nt[c] = int(hc[c].lp_ntaps);
             d[c] = hc[c].cfg_dirty; hc[c].cfg_dirty = false;
         }
-        HBD_CUDA_CHECK(cudaMemcpyAsync(d_cfg_baud, b.data(), 8 * n, cudaMemcpyHostToDevice, stream));
-        HBD_CUDA_CHECK(cudaMemcpyAsync(d_cfg_stops, s.data(), 4 * n, cudaMemcpyHostToDevice, stream));
-        HBD_CUDA_CHECK(cudaMemcpyAsync(d_cfg_bits, bi.data(), 4 * n, cudaMemcpyHostToDevice, stream));
-        HBD_CUDA_CHECK(cudaMemcpyAsync(d_cfg_dc, dc.data(), 4 * n, cudaMemcpyHostToDevice, stream));
-        HBD_CUDA_CHECK(cudaMemcpyAsync(d_cfg_ntaps, nt.data(), 4 * n, cudaMemcpyHostToDevice, stream));
-        HBD_CUDA_CHECK(cudaMemcpyAsync(d_cfg_dirty, d.data(), n, cudaMemcpyHostToDevice, stream));
-        init_cfg_kernel<<<(n_ch + 127) / 128, 128, 0, stream>>>(d_state, d_cfg_baud, d_cfg_stops, d_cfg_bits, d_cfg_dc, d_cfg_ntaps, d_cfg_dirty, n_ch);
+        HBD_CUDA_CHECK(cudaMemcpyAsync(d_cfg_baud.get(), b.data(), 8 * n, cudaMemcpyHostToDevice, stream));
+        HBD_CUDA_CHECK(cudaMemcpyAsync(d_cfg_stops.get(), s.data(), 4 * n, cudaMemcpyHostToDevice, stream));
+        HBD_CUDA_CHECK(cudaMemcpyAsync(d_cfg_bits.get(), bi.data(), 4 * n, cudaMemcpyHostToDevice, stream));
+        HBD_CUDA_CHECK(cudaMemcpyAsync(d_cfg_dc.get(), dc.data(), 4 * n, cudaMemcpyHostToDevice, stream));
+        HBD_CUDA_CHECK(cudaMemcpyAsync(d_cfg_ntaps.get(), nt.data(), 4 * n, cudaMemcpyHostToDevice, stream));
+        HBD_CUDA_CHECK(cudaMemcpyAsync(d_cfg_dirty.get(), d.data(), n, cudaMemcpyHostToDevice, stream));
+        init_cfg_kernel<<<(n_ch + 127) / 128, 128, 0, stream>>>(d_state.get(), d_cfg_baud.get(), d_cfg_stops.get(), d_cfg_bits.get(), d_cfg_dc.get(), d_cfg_ntaps.get(), d_cfg_dirty.get(), n_ch);
         ++launches;
         HBD_CUDA_CHECK(cudaStreamSynchronize(stream)); // host vectors go out of scope
         cfg_dirty_any = false;
@@ -820,7 +780,7 @@ int hbd_decoder::plan_call(CallPlan& cp)
         cp.uplan = h_plan[0];
         if (!cp.plan_uniform && (h_plan_uploaded.size() != n || memcmp(h_plan.data(), h_plan_uploaded.data(), n * sizeof(ChanPlan)) != 0)) {
             if (quiesce()) return HBD_ERR_CUDA;
-            HBD_CUDA_CHECK(cudaMemcpyAsync(d_plan, h_plan.data(), n * sizeof(ChanPlan), cudaMemcpyHostToDevice, stream));
+            HBD_CUDA_CHECK(cudaMemcpyAsync(d_plan.get(), h_plan.data(), n * sizeof(ChanPlan), cudaMemcpyHostToDevice, stream));
             HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
             h_plan_uploaded = h_plan;
         }
@@ -848,92 +808,92 @@ int hbd_decoder::plan_call(CallPlan& cp)
 int hbd_decoder::enqueue_call(const CallPlan& cp)
 {
     const double fs_dec = fs_in / factor;
-    const float2* chunk = in.p ? static_cast<const float2*>(in.p) : d_stage;
-    const size_t chunk_pitch = in.p ? in.pitch : stage_pitch;
+    const float2* chunk = in.p ? static_cast<const float2*>(in.p) : stage.get();
+    const size_t chunk_pitch = in.p ? in.pitch : stage.pitch;
     int nl = 0;
     // everything the caller (and the host-side updates of plan_call) put on `stream` happens before the kernels start
-    HBD_CUDA_CHECK(cudaEventRecord(ev_in, stream));
-    HBD_CUDA_CHECK(cudaStreamWaitEvent(hi, ev_in, 0));
+    HBD_CUDA_CHECK(cudaEventRecord(ev_in.get(), stream));
+    HBD_CUDA_CHECK(cudaStreamWaitEvent(hi.get(), ev_in.get(), 0));
     bool tail_recorded = false;
     // K1 overwrites the stage-1 buffer: the tail of the call before the previous one must be done with it
-    if (tail_pending[s1_cur]) HBD_CUDA_CHECK(cudaStreamWaitEvent(hi, ev_tail[s1_cur], 0));
+    if (tail_pending[s1_cur]) HBD_CUDA_CHECK(cudaStreamWaitEvent(hi.get(), ev_tail[s1_cur].get(), 0));
     {   // K1 also writes the next call's carry (even when no channel has a full decimation block yet)
         DecimArgs da{};
-        da.chunk = chunk; da.chunk_pitch = chunk_pitch; da.carry = d_carry2[carry_cur]; da.carry_next = d_carry2[carry_cur ^ 1]; da.carry_cap = carry_cap;
-        da.s1 = d_s1x[s1_cur]; da.s1_pitch = s1_pitch; da.s1_hist = kS1Hist;
-        da.plan = d_plan; da.uplan = cp.uplan; da.uniform = cp.plan_uniform ? 1 : 0; da.taps = d_taps1; da.ch0 = 0; da.n_channels = n_ch;
+        da.chunk = chunk; da.chunk_pitch = chunk_pitch; da.carry = d_carry2[carry_cur].get(); da.carry_next = d_carry2[carry_cur ^ 1].get(); da.carry_cap = carry_cap;
+        da.s1 = s1x.get(s1_cur); da.s1_pitch = s1x.pitch; da.s1_hist = kS1Hist;
+        da.plan = d_plan.get(); da.uplan = cp.uplan; da.uniform = cp.plan_uniform ? 1 : 0; da.taps = d_taps1.get(); da.ch0 = 0; da.n_channels = n_ch;
         da.nco = in.nco;
-        if (timing) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_k1, ev_used_k1), hi));
-        HBD_CUDA_CHECK(launch_decim1(da, M1, T1, cp.max_n1, n_sms, hi, &nl, in.format));
-        if (timing) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_k1, ev_used_k1), hi));
+        if (timing) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_k1, ev_used_k1), hi.get()));
+        HBD_CUDA_CHECK(launch_decim1(da, M1, T1, cp.max_n1, n_sms, hi.get(), &nl, in.format));
+        if (timing) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_k1, ev_used_k1), hi.get()));
     }
-    HBD_CUDA_CHECK(cudaEventRecord(ev_consumed, hi)); // input no longer needed; stage-1 output ready
-    HBD_CUDA_CHECK(cudaStreamWaitEvent(lo, ev_consumed, 0));
-    if (timing > 1) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_rest, ev_used_rest), lo));
+    HBD_CUDA_CHECK(cudaEventRecord(ev_consumed.get(), hi.get())); // input no longer needed; stage-1 output ready
+    HBD_CUDA_CHECK(cudaStreamWaitEvent(lo.get(), ev_consumed.get(), 0));
+    if (timing > 1) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_rest, ev_used_rest), lo.get()));
     if (cp.any_work) {
         // cascaded plan: the stages between K1's and the tail kernel's (1/64 of the input rate or less)
         for (size_t k = 0; k < mids.size(); ++k) {
             const StageRows in_k = stage_in(k), out_k = stage_in(k + 1);
             MidArgs ma{};
-            ma.plan = d_plan; ma.uplan = cp.uplan; ma.uniform = cp.plan_uniform ? 1 : 0;
+            ma.plan = d_plan.get(); ma.uplan = cp.uplan; ma.uniform = cp.plan_uniform ? 1 : 0;
             ma.in = in_k.p; ma.in_next = in_k.next; ma.in_pitch = in_k.pitch; ma.in_hist = in_k.hist;
             ma.out = out_k.p; ma.out_pitch = out_k.pitch; ma.out_hist = out_k.hist;
-            ma.taps = mids[k].d_taps; ma.M = mids[k].M; ma.T = mids[k].T; ma.div_in = mids[k].div_in;
-            HBD_CUDA_CHECK(launch_mid_stage(ma, n_ch, lo, &nl));
+            ma.taps = mids[k].d_taps.get(); ma.M = mids[k].M; ma.T = mids[k].T; ma.div_in = mids[k].div_in;
+            HBD_CUDA_CHECK(launch_mid_stage(ma, n_ch, lo.get(), &nl));
         }
         const StageRows s1 = stage_in(mids.size());
         TailArgs ta{};
-        ta.plan = d_plan; ta.uplan = cp.uplan; ta.uniform = cp.plan_uniform ? 1 : 0; ta.state = d_state; ta.ch0 = 0;
+        ta.plan = d_plan.get(); ta.uplan = cp.uplan; ta.uniform = cp.plan_uniform ? 1 : 0; ta.state = d_state.get(); ta.ch0 = 0;
         ta.s1 = s1.p; ta.s1_next = s1.next; ta.s1_pitch = s1.pitch;
-        ta.taps2 = d_taps2; ta.M2 = M2; ta.T2 = T2;
-        ta.decq = d_decq; ta.dq_pitch = dq_pitch; ta.fs_dec = fs_dec; ta.fftbuf = d_fftbuf; ta.fft_n = fft_n; ta.lptaps = d_lptaps;
+        ta.taps2 = d_taps2.get(); ta.M2 = M2; ta.T2 = T2;
+        ta.decq = decq.get(); ta.dq_pitch = decq.pitch; ta.fs_dec = fs_dec; ta.fftbuf = fft.buf.get(); ta.fft_n = fft_n; ta.lptaps = d_lptaps.get();
         ta.max_lp_taps = int(max_lp_taps_c);
-        ta.slicer = d_slicer; ta.slicer_pitch = slicer_pitch; ta.sv_want = cp.sv_want;
-        ta.log = d_log; ta.log_ctl = d_log_ctl; ta.log_mask = log_cap - 1u; ta.call_seq = call_seq & 0xffffffu;
-        ta.uart_runs = d_uart_runs;
-        ta.maskc = mask_cache ? d_maskc : nullptr;
-        ta.ssdv_ring = ssdv_on ? d_ssdv_ring : nullptr; ta.ssdv_total = d_ssdv_total;
-        ta.demod_last = d_demod; ta.demod_pitch = demod_pitch;
-        ta.rec_decimated = record ? d_rec_dec : nullptr; ta.rec_filtered = record ? d_rec_filt : nullptr; ta.rec_pitch = rec_pitch;
-        ta.rec_bits = record ? d_rec_bits : nullptr; ta.rec_bits_n = d_rec_bits_n; ta.rec_bits_pitch = rec_bits_pitch;
-        HBD_CUDA_CHECK(launch_tail(ta, n_ch, lo, &nl));
+        ta.slicer = slicer.get(); ta.slicer_pitch = slicer.pitch; ta.sv_want = cp.sv_want;
+        ta.log = d_log.get(); ta.log_ctl = d_log_ctl.get(); ta.log_mask = log_cap - 1u; ta.call_seq = call_seq & 0xffffffu;
+        ta.uart_runs = d_uart_runs.get();
+        ta.maskc = mask_cache ? d_maskc.get() : nullptr;
+        ta.ssdv_ring = ssdv_on ? d_ssdv_ring.get() : nullptr; ta.ssdv_total = d_ssdv_total.get();
+        ta.demod_last = demod.get(); ta.demod_pitch = demod.pitch;
+        ta.rec_decimated = record ? rec.get(0) : nullptr; ta.rec_filtered = record ? rec.get(1) : nullptr; ta.rec_pitch = rec.pitch;
+        ta.rec_bits = record ? d_rec_bits.get() : nullptr; ta.rec_bits_n = d_rec_bits_n.get(); ta.rec_bits_pitch = rec_bits_pitch;
+        HBD_CUDA_CHECK(launch_tail(ta, n_ch, lo.get(), &nl));
         // only the tail kernel reads the stage-1 buffer: K1 of the call after next may overwrite it as soon as the
         // tail is done, without waiting for the FFT / SSDV / demod kernels behind it on this stream
-        if (!tail_ev_late) { HBD_CUDA_CHECK(cudaEventRecord(ev_tail[s1_cur], lo)); tail_recorded = true; }
+        if (!tail_ev_late) { HBD_CUDA_CHECK(cudaEventRecord(ev_tail[s1_cur].get(), lo.get())); tail_recorded = true; }
         FftArgs fa{};
-        fa.state = d_state; fa.fftbuf = d_fftbuf; fa.spectrum = d_spectrum; fa.power = d_power; fa.twiddle = d_twiddle; fa.fs_dec = fs_dec;
+        fa.state = d_state.get(); fa.fftbuf = fft.buf.get(); fa.spectrum = fft.spectrum.get(); fa.power = fft.power.get(); fa.twiddle = fft.twiddle.get(); fa.fs_dec = fs_dec;
         fa.ch0 = 0; fa.fft_n = fft_n;
-        if (cp.need_k4) HBD_CUDA_CHECK(launch_fft_afc(fa, n_ch, lo, &nl));   // other calls: K2 has stepped the AFC itself
+        if (cp.need_k4) HBD_CUDA_CHECK(launch_fft_afc(fa, n_ch, lo.get(), &nl));   // other calls: K2 has stepped the AFC itself
         if (ssdv_on) {   // test every 0x55-started window the new characters completed
             SsdvScanArgs sa{};
-            sa.ring = d_ssdv_ring; sa.total = d_ssdv_total; sa.scanned = d_ssdv_scanned; sa.log = d_ssdv_log;
-            sa.ctl = d_log_ctl; sa.call_seq = call_seq & 0xffffffu; sa.ch0 = 0;
-            HBD_CUDA_CHECK(launch_ssdv_scan(sa, n_ch, lo, &nl));
+            sa.ring = d_ssdv_ring.get(); sa.total = d_ssdv_total.get(); sa.scanned = d_ssdv_scanned.get(); sa.log = d_ssdv_log.get();
+            sa.ctl = d_log_ctl.get(); sa.call_seq = call_seq & 0xffffffu; sa.ch0 = 0;
+            HBD_CUDA_CHECK(launch_ssdv_scan(sa, n_ch, lo.get(), &nl));
         }
     }
-    if (demod_acc_on && d_demod) { // main.cpp:267-282 runs after EVERY process(), also when nothing new was demodulated
+    if (demod_acc_on && demod.get()) { // main.cpp:267-282 runs after EVERY process(), also when nothing new was demodulated
         DemodAccArgs aa{};
-        aa.state = d_state; aa.demod = d_demod; aa.demod_pitch = demod_pitch; aa.acc = d_dacc; aa.acc_pitch = dacc_pitch; aa.acc_n = d_dacc_n;
+        aa.state = d_state.get(); aa.demod = demod.get(); aa.demod_pitch = demod.pitch; aa.acc = dacc.get(); aa.acc_pitch = dacc.pitch; aa.acc_n = d_dacc_n.get();
         aa.fs_dec = fs_dec; aa.ch0 = 0;
-        HBD_CUDA_CHECK(launch_demod_accumulate(aa, n_ch, lo, &nl));
+        HBD_CUDA_CHECK(launch_demod_accumulate(aa, n_ch, lo.get(), &nl));
     }
-    if (timing > 1) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_rest, ev_used_rest), lo));
-    if (!tail_recorded) HBD_CUDA_CHECK(cudaEventRecord(ev_tail[s1_cur], lo));
+    if (timing > 1) HBD_CUDA_CHECK(cudaEventRecord(next_event(ev_rest, ev_used_rest), lo.get()));
+    if (!tail_recorded) HBD_CUDA_CHECK(cudaEventRecord(ev_tail[s1_cur].get(), lo.get()));
     tail_pending[s1_cur] = true;
     // the caller's stream resumes once the input has been consumed (it does not wait for the tail kernels)
-    HBD_CUDA_CHECK(cudaStreamWaitEvent(stream, ev_consumed, 0));
+    HBD_CUDA_CHECK(cudaStreamWaitEvent(stream, ev_consumed.get(), 0));
     carry_cur ^= 1;
     if (cp.any_work) s1_cur ^= 1; // the tail (which moves the stage-2 history to the other buffer) ran
     launches += unsigned(nl);
     if (snap_on) {
-        stats_snap_kernel<<<(n_ch + 127) / 128, 128, 0, lo>>>(d_state, d_snap + size_t(call_seq % kSnapSlots) * size_t(n_ch) * 6, n_ch);
+        stats_snap_kernel<<<(n_ch + 127) / 128, 128, 0, lo.get()>>>(d_state.get(), d_snap.get() + size_t(call_seq % kSnapSlots) * size_t(n_ch) * 6, n_ch);
         ++launches;
     }
     // commit: the log control words as they stand after this call, into the call's pinned slot (stream order: every
     // entry below these heads is completely written when ev_call fires)
     const size_t slot = call_seq % ev_call.size();
-    HBD_CUDA_CHECK(cudaMemcpyAsync(h_heads + slot * kCtlWords, d_log_ctl, kCtlWords * sizeof(unsigned), cudaMemcpyDeviceToHost, lo));
-    HBD_CUDA_CHECK(cudaEventRecord(ev_call[slot], lo)); // everything of this call is done
+    HBD_CUDA_CHECK(cudaMemcpyAsync(h_heads.get() + slot * kCtlWords, d_log_ctl.get(), kCtlWords * sizeof(unsigned), cudaMemcpyDeviceToHost, lo.get()));
+    HBD_CUDA_CHECK(cudaEventRecord(ev_call[slot].get(), lo.get())); // everything of this call is done
     ++call_seq;
     return HBD_OK;
 }
@@ -949,7 +909,7 @@ int hbd_decoder::process_async_locked()
         size_t wp = 0;
         const int rc = widen(in.p, in.pitch, in.format, n_ch, in.n, &wp);
         if (rc) return rc;
-        in = DeviceInput{d_widen, wp, in.n};
+        in = DeviceInput{d_widen(), wp, in.n};
     }
     { const int rc = enqueue_call(cp); if (rc) return rc; }
     in = DeviceInput{};
@@ -980,11 +940,11 @@ int hbd_decoder::collect_locked(unsigned lag)
         if (sync_groups()) { set_error("stream sync failed"); return HBD_ERR_CUDA; }
         HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
     } else {
-        HBD_CUDA_CHECK(cudaEventSynchronize(ev_call[(upto - 1) % ev_call.size()]));
+        HBD_CUDA_CHECK(cudaEventSynchronize(ev_call[(upto - 1) % ev_call.size()].get()));
     }
     // the COMMITTED control words of call upto-1 (never the live head: newer calls may be appending right now)
     unsigned heads[kCtlWords];
-    memcpy(heads, h_heads + size_t((upto - 1) % ev_call.size()) * kCtlWords, sizeof(heads));
+    memcpy(heads, h_heads.get() + size_t((upto - 1) % ev_call.size()) * kCtlWords, sizeof(heads));
     const unsigned head = heads[kCtlCharHead];
     int result = HBD_OK;
     if (ssdv_on) {
@@ -1006,10 +966,10 @@ int hbd_decoder::collect_locked(unsigned lag)
         if (avail_p) {
             const unsigned i0 = ssdv_log_tail & (kSsdvLogCap - 1u);
             const unsigned first = std::min(avail_p, kSsdvLogCap - i0);
-            HBD_CUDA_CHECK(cudaMemcpyAsync(h_ssdv_log.data(), d_ssdv_log + i0, size_t(first) * sizeof(SsdvLogEntry), cudaMemcpyDeviceToHost, copy_stream));
+            HBD_CUDA_CHECK(cudaMemcpyAsync(h_ssdv_log.data(), d_ssdv_log.get() + i0, size_t(first) * sizeof(SsdvLogEntry), cudaMemcpyDeviceToHost, copy_stream.get()));
             if (avail_p > first)
-                HBD_CUDA_CHECK(cudaMemcpyAsync(h_ssdv_log.data() + first, d_ssdv_log, size_t(avail_p - first) * sizeof(SsdvLogEntry), cudaMemcpyDeviceToHost, copy_stream));
-            HBD_CUDA_CHECK(cudaStreamSynchronize(copy_stream));
+                HBD_CUDA_CHECK(cudaMemcpyAsync(h_ssdv_log.data() + first, d_ssdv_log.get(), size_t(avail_p - first) * sizeof(SsdvLogEntry), cudaMemcpyDeviceToHost, copy_stream.get()));
+            HBD_CUDA_CHECK(cudaStreamSynchronize(copy_stream.get()));
         }
         for (unsigned k = 0; k < avail_p; ++k) {
             const SsdvLogEntry& e = h_ssdv_log[k];
@@ -1030,8 +990,8 @@ int hbd_decoder::collect_locked(unsigned lag)
         result = HBD_ERR_STATE;
     }
     if (snap_on && call_seq - (upto - 1u) < kSnapSlots - 1u) {   // the slot of call upto-1 has not been reused yet
-        HBD_CUDA_CHECK(cudaMemcpyAsync(h_snap, d_snap + size_t((upto - 1u) % kSnapSlots) * size_t(n_ch) * 6, sizeof(float) * 6 * size_t(n_ch),
-                                       cudaMemcpyDeviceToHost, copy_stream));
+        HBD_CUDA_CHECK(cudaMemcpyAsync(h_snap.get(), d_snap.get() + size_t((upto - 1u) % kSnapSlots) * size_t(n_ch) * 6, sizeof(float) * 6 * size_t(n_ch),
+                                       cudaMemcpyDeviceToHost, copy_stream.get()));
         h_snap_valid = true;
     }
     const unsigned avail = head - log_tail;
@@ -1039,17 +999,17 @@ int hbd_decoder::collect_locked(unsigned lag)
     if (avail) {
         const unsigned i0 = log_tail & (log_cap - 1u);
         const unsigned first = std::min(avail, log_cap - i0);
-        HBD_CUDA_CHECK(cudaMemcpyAsync(h_log.data(), d_log + i0, size_t(first) * sizeof(uint2), cudaMemcpyDeviceToHost, copy_stream));
+        HBD_CUDA_CHECK(cudaMemcpyAsync(h_log.data(), d_log.get() + i0, size_t(first) * sizeof(uint2), cudaMemcpyDeviceToHost, copy_stream.get()));
         if (avail > first)
-            HBD_CUDA_CHECK(cudaMemcpyAsync(h_log.data() + first, d_log, size_t(avail - first) * sizeof(uint2), cudaMemcpyDeviceToHost, copy_stream));
-        HBD_CUDA_CHECK(cudaStreamSynchronize(copy_stream));
+            HBD_CUDA_CHECK(cudaMemcpyAsync(h_log.data() + first, d_log.get(), size_t(avail - first) * sizeof(uint2), cudaMemcpyDeviceToHost, copy_stream.get()));
+        HBD_CUDA_CHECK(cudaStreamSynchronize(copy_stream.get()));
     }
     // the writers may reuse everything below the new tail
     log_tail = head;
-    h_tail_pin[0] = log_tail; h_tail_pin[1] = ssdv_log_tail;
-    HBD_CUDA_CHECK(cudaMemcpyAsync(d_log_ctl + kCtlCharTail, h_tail_pin, sizeof(unsigned), cudaMemcpyHostToDevice, copy_stream));
-    HBD_CUDA_CHECK(cudaMemcpyAsync(d_log_ctl + kCtlSsdvTail, h_tail_pin + 1, sizeof(unsigned), cudaMemcpyHostToDevice, copy_stream));
-    HBD_CUDA_CHECK(cudaStreamSynchronize(copy_stream));   // h_tail_pin is rewritten by the next drain
+    h_tail_pin.get()[0] = log_tail; h_tail_pin.get()[1] = ssdv_log_tail;
+    HBD_CUDA_CHECK(cudaMemcpyAsync(d_log_ctl.get() + kCtlCharTail, h_tail_pin.get(), sizeof(unsigned), cudaMemcpyHostToDevice, copy_stream.get()));
+    HBD_CUDA_CHECK(cudaMemcpyAsync(d_log_ctl.get() + kCtlSsdvTail, h_tail_pin.get() + 1, sizeof(unsigned), cudaMemcpyHostToDevice, copy_stream.get()));
+    HBD_CUDA_CHECK(cudaStreamSynchronize(copy_stream.get()));   // h_tail_pin is rewritten by the next drain
 
     // The log is sorted by call, and within a call a channel's characters form ONE contiguous segment (one reservation per
     // flush; only a channel that decodes more than kCharBuf = 64 characters in a call flushes twice).  Replay segment by
@@ -1178,19 +1138,21 @@ int hbd_decoder::enable_ssdv(bool on)
     { const int rc = collect_locked(0); if (rc) return rc; }
     const size_t n = size_t(n_ch);
     if (on) {
-        if (!d_ssdv_ring) {
-            HBD_CUDA_CHECK(dalloc(&d_ssdv_ring, n * kSsdvRing));
-            HBD_CUDA_CHECK(dalloc(&d_ssdv_total, n));
-            HBD_CUDA_CHECK(dalloc(&d_ssdv_scanned, n));
-            HBD_CUDA_CHECK(dalloc(&d_ssdv_log, size_t(kSsdvLogCap)));
+        if (!d_ssdv_ring) {   // the four buffers are allocated together
+            DevPtr<unsigned char> ring; DevPtr<unsigned> total, scanned; DevPtr<SsdvLogEntry> log;
+            HBD_CUDA_CHECK(dev_alloc(ring, n * kSsdvRing));
+            HBD_CUDA_CHECK(dev_alloc(total, n));
+            HBD_CUDA_CHECK(dev_alloc(scanned, n));
+            HBD_CUDA_CHECK(dev_alloc(log, size_t(kSsdvLogCap)));
+            d_ssdv_ring = std::move(ring); d_ssdv_total = std::move(total); d_ssdv_scanned = std::move(scanned); d_ssdv_log = std::move(log);
         }
-        HBD_CUDA_CHECK(cudaMemset(d_ssdv_ring, 0, n * kSsdvRing));
-        HBD_CUDA_CHECK(cudaMemset(d_ssdv_total, 0, n * sizeof(unsigned)));
-        HBD_CUDA_CHECK(cudaMemset(d_ssdv_scanned, 0, n * sizeof(unsigned)));
+        HBD_CUDA_CHECK(cudaMemset(d_ssdv_ring.get(), 0, n * kSsdvRing));
+        HBD_CUDA_CHECK(cudaMemset(d_ssdv_total.get(), 0, n * sizeof(unsigned)));
+        HBD_CUDA_CHECK(cudaMemset(d_ssdv_scanned.get(), 0, n * sizeof(unsigned)));
         // the SSDV log keeps its (monotonic) head: nothing below it is of interest any more
-        ssdv_log_tail = h_heads[size_t((call_seq ? call_seq - 1u : 0u) % ev_call.size()) * kCtlWords + kCtlSsdvHead];
-        h_tail_pin[1] = ssdv_log_tail;
-        HBD_CUDA_CHECK(cudaMemcpy(d_log_ctl + kCtlSsdvTail, h_tail_pin + 1, sizeof(unsigned), cudaMemcpyHostToDevice));
+        ssdv_log_tail = h_heads.get()[size_t((call_seq ? call_seq - 1u : 0u) % ev_call.size()) * kCtlWords + kCtlSsdvHead];
+        h_tail_pin.get()[1] = ssdv_log_tail;
+        HBD_CUDA_CHECK(cudaMemcpy(d_log_ctl.get() + kCtlSsdvTail, h_tail_pin.get() + 1, sizeof(unsigned), cudaMemcpyHostToDevice));
         ssdv.assign(n, SsdvChannel());
     }
     ssdv_on = on;
@@ -1201,11 +1163,13 @@ int hbd_decoder::enable_snap()
 {
     if (snap_on) return HBD_OK;
     HBD_CUDA_CHECK(cudaSetDevice(device));
-    if (!d_snap) {
-        HBD_CUDA_CHECK(dalloc(&d_snap, size_t(kSnapSlots) * size_t(n_ch) * 6));
-        HBD_CUDA_CHECK(cudaMemset(d_snap, 0, sizeof(float) * size_t(kSnapSlots) * size_t(n_ch) * 6));
-        HBD_CUDA_CHECK(cudaHostAlloc((void**)&h_snap, sizeof(float) * 6 * size_t(n_ch), cudaHostAllocDefault));
-        memset(h_snap, 0, sizeof(float) * 6 * size_t(n_ch));
+    if (!d_snap) {   // both buffers are allocated together
+        DevPtr<float> d; HostPtr<float> hp;
+        HBD_CUDA_CHECK(dev_alloc(d, size_t(kSnapSlots) * size_t(n_ch) * 6));
+        HBD_CUDA_CHECK(cudaMemset(d.get(), 0, sizeof(float) * size_t(kSnapSlots) * size_t(n_ch) * 6));
+        HBD_CUDA_CHECK(host_alloc(hp, 6 * size_t(n_ch)));
+        memset(hp.get(), 0, sizeof(float) * 6 * size_t(n_ch));
+        d_snap = std::move(d); h_snap = std::move(hp);
     }
     snap_on = true;
     return HBD_OK;
@@ -1214,7 +1178,7 @@ int hbd_decoder::enable_snap()
 namespace hbd {
 int internal_device(hbd_decoder* h) { return h->device; }
 void internal_set_error(hbd_decoder* h, const std::string& what) { std::lock_guard<std::mutex> l(h->mtx); h->set_error(what); }
-void** internal_dist_slot(hbd_decoder* h) { return &h->dist_ctx; }
+DistSlot& internal_dist_slot(hbd_decoder* h) { return h->dist_ctx; }
 }
 
 // =====================================================================================================
@@ -1229,14 +1193,14 @@ size_t hbd_pack_results(hbd_decoder* h, int ch_offset, hbd_result_record* out, s
     const size_t n = size_t(h->n_ch);
     if (!out || cap_records < n) return n;
     std::vector<float> live;     // AFC scalars when no snapshot has been taken yet
-    const float* st = h->h_snap;
+    const float* st = h->h_snap.get();
     if (!(h->snap_on && h->h_snap_valid)) {   // read the live state (waits for the calls in flight)
         if (h->enable_snap() != HBD_OK) return 0;
         cudaSetDevice(h->device);
         h->sync_groups();
         cudaStreamSynchronize(h->stream);
         std::vector<ChanState> cs(n);
-        if (cudaMemcpy(cs.data(), h->d_state, n * sizeof(ChanState), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
+        if (cudaMemcpy(cs.data(), h->d_state.get(), n * sizeof(ChanState), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
         live.resize(6 * n);
         for (size_t c = 0; c < n; ++c) {
             live[6 * c + 0] = float(cs[c].afc_correction); live[6 * c + 1] = float(cs[c].afc_shift_hz); live[6 * c + 2] = float(cs[c].afc_noise_floor);
@@ -1295,7 +1259,7 @@ int hbd_create(int n_channels, int cuda_device, hbd_decoder** out)
     int count = 0;
     if (cudaGetDeviceCount(&count) != cudaSuccess || cuda_device < 0 || cuda_device >= count) return HBD_ERR_CUDA;
     if (cudaSetDevice(cuda_device) != cudaSuccess) return HBD_ERR_CUDA;
-    hbd_decoder* h = new (std::nothrow) hbd_decoder;
+    std::unique_ptr<hbd_decoder> h(new (std::nothrow) hbd_decoder);
     if (!h) return HBD_ERR_NOMEM;
     h->n_ch = n_channels; h->device = cuda_device;
     cudaDeviceProp prop;
@@ -1304,8 +1268,8 @@ int hbd_create(int n_channels, int cuda_device, hbd_decoder** out)
     h->text.resize(size_t(n_channels));
     for (auto& tc : h->text) { tc.text_stream.reserve(120); tc.last_sentence.reserve(96); }   // no allocation on the drain path in steady state
     { hbd_result_record z; memset(&z, 0, sizeof(z)); h->pend.assign(size_t(n_channels), z); }
-    if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess) { delete h; return HBD_ERR_CUDA; }
-    h->own_stream = true;
+    if (stream_create(h->own_stream) != cudaSuccess) return HBD_ERR_CUDA;
+    h->stream = h->own_stream.get();
     {
         if (const char* sv = getenv("HBD_SV_WANT")) h->sv_override = atoi(sv);
         if (const char* mc = getenv("HBD_MASK_CACHE")) h->mask_cache = atoi(mc) != 0;
@@ -1320,25 +1284,17 @@ int hbd_create(int n_channels, int cuda_device, hbd_decoder** out)
         }
         int prio_lo = 0, prio_hi = 0;
         cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi); // numerically lower = higher priority
-        if (cudaStreamCreateWithPriority(&h->hi, cudaStreamNonBlocking, prio_hi) != cudaSuccess ||
-            cudaStreamCreateWithPriority(&h->lo, cudaStreamNonBlocking, prio_lo) != cudaSuccess) { h->free_all(); delete h; return HBD_ERR_CUDA; }
-        if (cudaEventCreateWithFlags(&h->ev_consumed, cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&h->ev_tail[0], cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&h->ev_tail[1], cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&h->ev_in, cudaEventDisableTiming) != cudaSuccess) { h->free_all(); delete h; return HBD_ERR_CUDA; }
+        if (stream_create(h->hi, prio_hi) != cudaSuccess || stream_create(h->lo, prio_lo) != cudaSuccess) return HBD_ERR_CUDA;
+        if (event_create(h->ev_consumed) != cudaSuccess || event_create(h->ev_tail[0]) != cudaSuccess || event_create(h->ev_tail[1]) != cudaSuccess ||
+            event_create(h->ev_in) != cudaSuccess) return HBD_ERR_CUDA;
     }
     const int rc = h->alloc_fixed();
-    if (rc) { h->free_all(); delete h; return rc; }
-    *out = h;
+    if (rc) return rc;
+    *out = h.release();
     return HBD_OK;
 }
 
-void hbd_destroy(hbd_decoder* h)
-{
-    if (!h) return;
-    h->free_all();
-    delete h;
-}
+void hbd_destroy(hbd_decoder* h) { delete h; }
 
 const char* hbd_last_error(hbd_decoder* h) { return h ? h->err.c_str() : "null handle"; }
 
@@ -1349,8 +1305,8 @@ int hbd_set_stream(hbd_decoder* h, void* s)
     cudaSetDevice(h->device);
     h->sync_groups();
     cudaStreamSynchronize(h->stream);
-    if (h->own_stream) cudaStreamDestroy(h->stream);
-    h->stream = (cudaStream_t)s; h->own_stream = false;
+    h->own_stream.reset();
+    h->stream = (cudaStream_t)s;
     return HBD_OK;
 }
 
@@ -1363,21 +1319,23 @@ int hbd_set_fft_size(hbd_decoder* h, size_t n_bins)
     cudaSetDevice(h->device);
     if (h->sync_groups() || cudaStreamSynchronize(h->stream) != cudaSuccess) return HBD_ERR_CUDA;
     if (int(n_bins) == h->fft_n) return HBD_OK;
-    h->fft_n = int(n_bins);
-    const int rc = h->alloc_fft();
+    hbd_decoder::FftBufs f;   // swapped in after the state reset below: on failure the old size and spectra stay
+    const int rc = h->make_fft(int(n_bins), f);
     if (rc) return rc;
     // spectrum / AFC state back to a freshly constructed decoder's (Average<T> starts with one 0 sample)
     std::vector<ChanState> st(size_t(h->n_ch));
-    if (cudaMemcpy(st.data(), h->d_state, st.size() * sizeof(ChanState), cudaMemcpyDeviceToHost) != cudaSuccess) return HBD_ERR_CUDA;
-    h->sync_ctrs();
-    for (auto& x : h->hc) x.fft_have = 0;
+    if (cudaMemcpy(st.data(), h->d_state.get(), st.size() * sizeof(ChanState), cudaMemcpyDeviceToHost) != cudaSuccess) return HBD_ERR_CUDA;
     for (auto& s : st) {
         s.fft_have = s.fft_ready = s.have_spectrum = 0;
         s.afc_correction = s.afc_noise_floor = s.afc_noise_var = s.afc_shift_hz = 0;
         s.nf_sum = s.nv_sum = 0; s.pl_sum = s.pr_sum = 0; s.nf_cnt = s.nv_cnt = s.pl_cnt = s.pr_cnt = 1;
         s.gui_left = s.gui_right = 0; s.spec_ok = 0;
     }
-    if (cudaMemcpy(h->d_state, st.data(), st.size() * sizeof(ChanState), cudaMemcpyHostToDevice) != cudaSuccess) return HBD_ERR_CUDA;
+    if (cudaMemcpy(h->d_state.get(), st.data(), st.size() * sizeof(ChanState), cudaMemcpyHostToDevice) != cudaSuccess) return HBD_ERR_CUDA;
+    h->fft = std::move(f);
+    h->fft_n = int(n_bins);
+    h->sync_ctrs();
+    for (auto& x : h->hc) x.fft_have = 0;
     return HBD_OK;
 }
 
@@ -1430,7 +1388,7 @@ static int set_lp(hbd_decoder* h, int ch, float bw, float trans, bool set_bw)
         const size_t T = design_lowpass(float(x.lp_bw / fs_dec), x.lp_trans, x.lp_input_size, x.lp_ntaps, taps);
         if (T != x.lp_ntaps && T <= size_t(kLpMaxTaps)) {
             x.lp_ntaps = T; x.cfg_dirty = true; h->cfg_dirty_any = h->derived_dirty = true;
-            if (cudaMemcpy(h->d_lptaps + size_t(c) * kLpMaxTaps, taps.data(), 4 * T, cudaMemcpyHostToDevice) != cudaSuccess) return HBD_ERR_CUDA;
+            if (cudaMemcpy(h->d_lptaps.get() + size_t(c) * kLpMaxTaps, taps.data(), 4 * T, cudaMemcpyHostToDevice) != cudaSuccess) return HBD_ERR_CUDA;
         }
     }
     bool cfg_same = true, ctr_same = true;
@@ -1518,22 +1476,11 @@ int hbd_decoder::mix_into_stage(const void* src, size_t src_pitch, int c0, int n
 {
     if (!n) return HBD_OK;
     nco_params(h_nco.data() + c0, c0, nc, n, true);
-    HBD_CUDA_CHECK(cudaMemcpyAsync(d_nco + c0, h_nco.data() + c0, sizeof(NcoChan) * size_t(nc), cudaMemcpyHostToDevice, stream));
+    HBD_CUDA_CHECK(cudaMemcpyAsync(d_nco.get() + c0, h_nco.data() + c0, sizeof(NcoChan) * size_t(nc), cudaMemcpyHostToDevice, stream));
     int nl = 0;
-    HBD_CUDA_CHECK(launch_nco_mix(src, src_pitch, d_stage, stage_pitch, dst_off, n, d_nco, c0, nc, stream, &nl, format));
+    HBD_CUDA_CHECK(launch_nco_mix(src, src_pitch, stage.get(), stage.pitch, dst_off, n, d_nco.get(), c0, nc, stream, &nl, format));
     launches += unsigned(nl);
     HBD_CUDA_CHECK(cudaStreamSynchronize(stream)); // h_nco is rewritten by the next push
-    return HBD_OK;
-}
-
-// grow d_iq_up / d_widen to `bytes`; what they held is dropped
-int hbd_decoder::ensure_scratch(void** p, size_t* cap, size_t bytes)
-{
-    if (bytes <= *cap) return HBD_OK;
-    HBD_CUDA_CHECK(cudaStreamSynchronize(stream));   // a kernel of an earlier push may still read the old buffer
-    cudaFree(*p); *p = nullptr; *cap = 0;
-    HBD_CUDA_CHECK(cudaMalloc(p, bytes));
-    *cap = bytes;
     return HBD_OK;
 }
 
@@ -1543,9 +1490,9 @@ int hbd_decoder::ensure_scratch(void** p, size_t* cap, size_t bytes)
 int hbd_decoder::widen(const void* src, size_t pitch, int format, int rows, size_t n, size_t* out_pitch)
 {
     *out_pitch = (n + 1) & ~size_t(1);
-    { const int rc = ensure_scratch((void**)&d_widen, &widen_bytes, std::max<size_t>(size_t(rows) * *out_pitch * sizeof(float2), 256)); if (rc) return rc; }
+    HBD_CUDA_CHECK(widen_buf.grow(std::max<size_t>(size_t(rows) * *out_pitch * sizeof(float2), 256), 1, 0, stream));
     int nl = 0;
-    HBD_CUDA_CHECK(launch_nco_mix(src, pitch, d_widen, *out_pitch, 0, n, nullptr, 0, rows, stream, &nl, format));
+    HBD_CUDA_CHECK(launch_nco_mix(src, pitch, d_widen(), *out_pitch, 0, n, nullptr, 0, rows, stream, &nl, format));
     launches += unsigned(nl);
     return HBD_OK;
 }
@@ -1556,7 +1503,7 @@ int hbd_decoder::widen(const void* src, size_t pitch, int format, int rows, size
 //   source                                condition                                  route
 //   host cf32, channel / matrix           -                                          copy into staging at base; K0 in place if
 //                                                                                    the channel's NCO is set (channel) / nco_any
-//   host integers, channel / matrix       -                                          upload to d_iq_up; K0 widens (and mixes)
+//   host integers, channel / matrix       -                                          upload to iq_up; K0 widens (and mixes)
 //                                                                                    into staging at base
 //   device cf32 matrix                    no nco_any                                 zero copy
 //   device integer matrix                 no nco_any, decim1_supports_native_iq      zero copy, K1 reads the integers
@@ -1589,21 +1536,21 @@ int hbd_decoder::push(const PushSrc& s)
     }
     if (!fs_in) fs_in = double(float(s.fs));   // Decoder::init(const float)
     auto ensure_stage = [&] {
-        return grow_rows(&d_stage, &stage_pitch, (std::max(size_t(base) + n, stage_pitch) + 15) & ~size_t(15), size_t(n_ch), stage_pitch, stream);
+        return stage.grow((std::max(size_t(base) + n, stage.pitch) + 15) & ~size_t(15), size_t(n_ch), stage.pitch, stream);
     };
 
     if (!s.device && s.shape != PushSrc::kRow) {   // host channel / matrix: into the staging rows
         const int c0 = channel ? s.ch : 0, rows = channel ? 1 : n_ch;
         const bool cf32 = s.format == HBD_IQ_CF32;
         HBD_CUDA_CHECK(ensure_stage());
-        if (!cf32 && n) { const int rc = ensure_scratch((void**)&d_iq_up, &iq_up_bytes, size_t(rows) * n * bytes); if (rc) return rc; }
-        void* dst = cf32 ? (void*)(d_stage + size_t(c0) * stage_pitch + base) : (void*)d_iq_up;   // integers cross PCIe packed [rows][n]
-        const size_t dst_pitch = cf32 ? stage_pitch * sizeof(float2) : n * bytes;
+        if (!cf32 && n) HBD_CUDA_CHECK(iq_up.grow(size_t(rows) * n * bytes, 1, 0, stream));
+        void* dst = cf32 ? (void*)(stage.get() + size_t(c0) * stage.pitch + base) : (void*)iq_up.get();   // integers cross PCIe packed [rows][n]
+        const size_t dst_pitch = cf32 ? stage.pitch * sizeof(float2) : n * bytes;
         if (n) HBD_CUDA_CHECK(cudaMemcpy2DAsync(dst, dst_pitch, s.p, (channel ? n : s.pitch) * bytes, n * bytes, size_t(rows), cudaMemcpyHostToDevice, stream));
         const bool mix = channel ? hc[size_t(c0)].nco_freq != 0 || hc[size_t(c0)].nco_phase != 0 : nco_any;
         int rc = HBD_OK;
-        if (!cf32) rc = mix_into_stage(d_iq_up, channel ? 0 : n, c0, rows, base, n, s.format);
-        else if (mix) rc = mix_into_stage(d_stage + base, stage_pitch, c0, rows, base, n);   // in place
+        if (!cf32) rc = mix_into_stage(iq_up.get(), channel ? 0 : n, c0, rows, base, n, s.format);
+        else if (mix) rc = mix_into_stage(stage.get() + base, stage.pitch, c0, rows, base, n);   // in place
         else HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
         if (rc) return rc;   // either way the stream has caught up: the caller owns `p` again (Decoder.h:209-213 copies)
         if (channel) hc[size_t(c0)].pushed += unsigned(n); else add_pushed(unsigned(n));
@@ -1614,20 +1561,20 @@ int hbd_decoder::push(const PushSrc& s)
     size_t pitch = s.pitch;   // 0 for a row
     if (s.shape == PushSrc::kRow && !(s.device && s.format == HBD_IQ_CF32)) {   // the row lands in d_widen as cf32
         const bool cf32 = s.format == HBD_IQ_CF32;
-        if (!s.device && n) {   // upload: cf32 straight into d_widen, integers into d_iq_up
-            void** up = cf32 ? (void**)&d_widen : (void**)&d_iq_up;
-            { const int rc = ensure_scratch(up, cf32 ? &widen_bytes : &iq_up_bytes, n * bytes); if (rc) return rc; }
-            HBD_CUDA_CHECK(cudaMemcpyAsync(*up, s.p, n * bytes, cudaMemcpyHostToDevice, stream));
-            src = *up;
+        if (!s.device && n) {   // upload: cf32 straight into d_widen, integers into iq_up
+            Rows<unsigned char>& up = cf32 ? widen_buf : iq_up;
+            HBD_CUDA_CHECK(up.grow(n * bytes, 1, 0, stream));
+            HBD_CUDA_CHECK(cudaMemcpyAsync(up.get(), s.p, n * bytes, cudaMemcpyHostToDevice, stream));
+            src = up.get();
         }
         if (!cf32) { size_t wp = 0; const int rc = widen(src, 0, s.format, 1, n, &wp); if (rc) return rc; }
-        src = d_widen;
+        src = d_widen();
     }
     if (device_matrix && s.format != HBD_IQ_CF32) {
         if (zero_copy && decim1_supports_native_iq(M1, T1)) { in = DeviceInput{s.p, s.pitch, n, s.format}; return HBD_OK; }
         const int rc = widen(s.p, s.pitch, s.format, n_ch, n, &pitch);
         if (rc) return rc;
-        src = d_widen;
+        src = d_widen();
     }
     if (zero_copy) { in = DeviceInput{src, pitch, n}; return HBD_OK; }
     if (nco_fused && base == 0 && n && decim1_supports_fused_nco(M1, T1) && !(reinterpret_cast<uintptr_t>(src) & 15)) {
@@ -1635,19 +1582,22 @@ int hbd_decoder::push(const PushSrc& s)
         // 8-byte write + 8-byte read per channel-sample through HBM.  The parameters go through a ring of pinned slots, so
         // the push does not wait for the GPU.
         if (!s.device) HBD_CUDA_CHECK(cudaStreamSynchronize(stream));   // the caller owns `p` again on return
-        if (!h_nco_pin) {
-            HBD_CUDA_CHECK(cudaHostAlloc((void**)&h_nco_pin, sizeof(NcoChan) * size_t(n_ch) * kNcoSlots, cudaHostAllocDefault));
-            HBD_CUDA_CHECK(dalloc(&d_nco_ring, size_t(n_ch) * kNcoSlots));
-            for (unsigned i = 0; i < kNcoSlots; ++i) HBD_CUDA_CHECK(cudaEventCreateWithFlags(&ev_nco[i], cudaEventDisableTiming));
+        if (!h_nco_pin) {   // the ring's buffers and events are created together
+            HostPtr<NcoChan> hp; DevPtr<NcoChan> dp; Event ev[kNcoSlots];
+            HBD_CUDA_CHECK(host_alloc(hp, size_t(n_ch) * kNcoSlots));
+            HBD_CUDA_CHECK(dev_alloc(dp, size_t(n_ch) * kNcoSlots));
+            for (Event& e : ev) HBD_CUDA_CHECK(event_create(e));
+            h_nco_pin = std::move(hp); d_nco_ring = std::move(dp);
+            for (unsigned i = 0; i < kNcoSlots; ++i) ev_nco[i] = std::move(ev[i]);
         }
         const unsigned slot = nco_seq % kNcoSlots;
-        if (nco_seq >= kNcoSlots) HBD_CUDA_CHECK(cudaEventSynchronize(ev_nco[slot]));   // the upload that last used this pinned slot (16 pushes ago)
+        if (nco_seq >= kNcoSlots) HBD_CUDA_CHECK(cudaEventSynchronize(ev_nco[slot].get()));   // the upload that last used this pinned slot (16 pushes ago)
         ++nco_seq;
-        NcoChan* hp = h_nco_pin + size_t(slot) * size_t(n_ch);
-        NcoChan* dp = d_nco_ring + size_t(slot) * size_t(n_ch);
+        NcoChan* hp = h_nco_pin.get() + size_t(slot) * size_t(n_ch);
+        NcoChan* dp = d_nco_ring.get() + size_t(slot) * size_t(n_ch);
         nco_params(hp, 0, n_ch, n, false);
         HBD_CUDA_CHECK(cudaMemcpyAsync(dp, hp, sizeof(NcoChan) * size_t(n_ch), cudaMemcpyHostToDevice, stream));
-        HBD_CUDA_CHECK(cudaEventRecord(ev_nco[slot], stream));
+        HBD_CUDA_CHECK(cudaEventRecord(ev_nco[slot].get(), stream));
         in = DeviceInput{src, pitch, n, HBD_IQ_CF32, dp};
         return HBD_OK;
     }
@@ -1726,7 +1676,7 @@ int hbd_set_kernel_timing(hbd_decoder* h, int on)
     if (on) {   // events are created here, not on the issue path of the calls being measured
         cudaSetDevice(h->device);
         for (auto* pool : {&h->ev_k1, &h->ev_rest})
-            while (pool->size() < 1024) { cudaEvent_t e; if (cudaEventCreate(&e) != cudaSuccess) return HBD_ERR_CUDA; pool->push_back(e); }
+            while (pool->size() < 1024) { Event e; if (event_create(e, cudaEventDefault) != cudaSuccess) return HBD_ERR_CUDA; pool->push_back(std::move(e)); }
     }
     return HBD_OK;
 }
@@ -1747,9 +1697,9 @@ int hbd_get_kernel_timing(hbd_decoder* h, int which, double* total_ms, unsigned*
         const size_t calls = std::min(h->ev_used_k1, h->ev_used_rest) / 2;
         for (size_t i = 0; i < calls; ++i) {
             cudaEvent_t a = nullptr, b = nullptr;
-            if (which == 2 && i + 1 < calls) { a = h->ev_k1[2 * i + 1]; b = h->ev_k1[2 * i + 2]; }        // K1 end -> next K1 start
-            else if (which == 3) { a = h->ev_k1[2 * i + 1]; b = h->ev_rest[2 * i]; }                      // K1 end -> own tail start
-            else if (which == 4 && i + 2 < calls) { a = h->ev_rest[2 * i + 1]; b = h->ev_k1[2 * i + 4]; } // tail end -> K1 start two calls on
+            if (which == 2 && i + 1 < calls) { a = h->ev_k1[2 * i + 1].get(); b = h->ev_k1[2 * i + 2].get(); }        // K1 end -> next K1 start
+            else if (which == 3) { a = h->ev_k1[2 * i + 1].get(); b = h->ev_rest[2 * i].get(); }                      // K1 end -> own tail start
+            else if (which == 4 && i + 2 < calls) { a = h->ev_rest[2 * i + 1].get(); b = h->ev_k1[2 * i + 4].get(); } // tail end -> K1 start two calls on
             if (!a) continue;
             float ms = 0;
             if (cudaEventElapsedTime(&ms, a, b) != cudaSuccess) return HBD_ERR_CUDA;
@@ -1759,11 +1709,11 @@ int hbd_get_kernel_timing(hbd_decoder* h, int which, double* total_ms, unsigned*
         if (count) *count = cnt;
         return HBD_OK;
     }
-    const std::vector<cudaEvent_t>& pool = which == 0 ? h->ev_k1 : h->ev_rest;
+    const std::vector<Event>& pool = which == 0 ? h->ev_k1 : h->ev_rest;
     const size_t used = which == 0 ? h->ev_used_k1 : h->ev_used_rest;
     for (size_t i = 0; i + 1 < used; i += 2) {
         float ms = 0;
-        if (cudaEventElapsedTime(&ms, pool[i], pool[i + 1]) != cudaSuccess) return HBD_ERR_CUDA;
+        if (cudaEventElapsedTime(&ms, pool[i].get(), pool[i + 1].get()) != cudaSuccess) return HBD_ERR_CUDA;
         tot += ms; ++cnt;
     }
     if (total_ms) *total_ms = tot;
@@ -1895,9 +1845,10 @@ int hbd_ssdv_check_packets(hbd_decoder* h, unsigned char* windows, size_t n, int
     if (!n) return HBD_OK;
     std::lock_guard<std::mutex> l(h->mtx);
     if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
-    unsigned char* d_w = nullptr; int* d_v = nullptr;
-    auto fail = [&](const char* what) { h->set_error(what); if (d_w) cudaFree(d_w); if (d_v) cudaFree(d_v); return HBD_ERR_CUDA; };
-    if (cudaMalloc((void**)&d_w, n * 256) != cudaSuccess || cudaMalloc((void**)&d_v, n * 2 * sizeof(int)) != cudaSuccess) return fail("cudaMalloc (ssdv check)");
+    DevPtr<unsigned char> w; DevPtr<int> v;
+    auto fail = [&](const char* what) { h->set_error(what); return HBD_ERR_CUDA; };
+    if (dev_alloc(w, n * 256) != cudaSuccess || dev_alloc(v, n * 2) != cudaSuccess) return fail("cudaMalloc (ssdv check)");
+    unsigned char* d_w = w.get(); int* d_v = v.get();
     if (cudaMemcpyAsync(d_w, windows, n * 256, cudaMemcpyHostToDevice, h->stream) != cudaSuccess) return fail("cudaMemcpyAsync (ssdv check)");
     int nl = 0;
     if (launch_ssdv_check(d_w, int(n), d_v, d_v + n, h->stream, &nl) != cudaSuccess) return fail("ssdv_check_kernel launch");
@@ -1906,7 +1857,6 @@ int hbd_ssdv_check_packets(hbd_decoder* h, unsigned char* windows, size_t n, int
         cudaMemcpyAsync(verdict, d_v, n * sizeof(int), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
         cudaMemcpyAsync(errors, d_v + n, n * sizeof(int), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
         cudaStreamSynchronize(h->stream) != cudaSuccess) return fail("ssdv check read-back");
-    cudaFree(d_w); cudaFree(d_v);
     return HBD_OK;
 }
 
@@ -1950,7 +1900,7 @@ static int fetch_state(hbd_decoder* h, int ch, ChanState* st)
 {
     cudaSetDevice(h->device);
     if (h->sync_groups() || cudaStreamSynchronize(h->stream) != cudaSuccess) return HBD_ERR_CUDA;
-    return cudaMemcpy(st, h->d_state + ch, sizeof(ChanState), cudaMemcpyDeviceToHost) == cudaSuccess ? HBD_OK : HBD_ERR_CUDA;
+    return cudaMemcpy(st, h->d_state.get() + ch, sizeof(ChanState), cudaMemcpyDeviceToHost) == cudaSuccess ? HBD_OK : HBD_ERR_CUDA;
 }
 static size_t fetch_floats(hbd_decoder* h, const void* dsrc, size_t n, float* out, size_t cap)
 {
@@ -1969,7 +1919,7 @@ size_t hbd_get_fft(hbd_decoder* h, int ch, float* out, size_t cap)
     std::lock_guard<std::mutex> l(h->mtx);
     ChanState st; if (fetch_state(h, ch, &st)) return 0;
     if (!st.have_spectrum) return 0; // freq_out_ is empty before the first FFT
-    return fetch_floats(h, h->d_spectrum + size_t(ch) * size_t(h->fft_n), 2 * size_t(h->fft_n), out, cap);
+    return fetch_floats(h, h->fft.spectrum.get() + size_t(ch) * size_t(h->fft_n), 2 * size_t(h->fft_n), out, cap);
 }
 size_t hbd_get_power_spectrum(hbd_decoder* h, int ch, float* out, size_t cap)
 {
@@ -1977,7 +1927,7 @@ size_t hbd_get_power_spectrum(hbd_decoder* h, int ch, float* out, size_t cap)
     std::lock_guard<std::mutex> l(h->mtx);
     ChanState st; if (fetch_state(h, ch, &st)) return 0;
     if (!st.have_spectrum) return 0;
-    return fetch_floats(h, h->d_power + size_t(ch) * size_t(h->fft_n), size_t(h->fft_n), out, cap);
+    return fetch_floats(h, h->fft.power.get() + size_t(ch) * size_t(h->fft_n), size_t(h->fft_n), out, cap);
 }
 size_t hbd_get_demodulated(hbd_decoder* h, int ch, float* out, size_t cap)
 {
@@ -1985,8 +1935,8 @@ size_t hbd_get_demodulated(hbd_decoder* h, int ch, float* out, size_t cap)
     std::lock_guard<std::mutex> l(h->mtx);
     h->sync_ctrs();
     const size_t n = h->hc[size_t(ch)].demod_n;   // a call that demodulates nothing leaves the previous block in place
-    if (!h->d_demod) return 0;
-    return fetch_floats(h, h->d_demod + size_t(ch) * h->demod_pitch, n, out, cap);
+    if (!h->demod.get()) return 0;
+    return fetch_floats(h, h->demod.get() + size_t(ch) * h->demod.pitch, n, out, cap);
 }
 int hbd_get_peaks(hbd_decoder* h, int ch, int* pl, int* pr)
 {
@@ -2015,7 +1965,7 @@ int hbd_reset_frequency_correction(hbd_decoder* h, int ch, double corr)
     HBD_CHECK_CH(h, ch); std::lock_guard<std::mutex> l(h->mtx);
     cudaSetDevice(h->device);
     h->sync_groups(); // ordered after everything in flight, like a call between two process() calls
-    if (launch_afc_reset(h->d_state, ch, corr, h->fs_in / h->factor, h->fft_n, h->stream) != cudaSuccess) return HBD_ERR_CUDA;
+    if (launch_afc_reset(h->d_state.get(), ch, corr, h->fs_in / h->factor, h->fft_n, h->stream) != cudaSuccess) return HBD_ERR_CUDA;
     cudaStreamSynchronize(h->stream);
     ++h->launches;
     return HBD_OK;
@@ -2024,13 +1974,10 @@ int hbd_reset_frequency_correction(hbd_decoder* h, int ch, double corr)
 int hbd_decoder::ensure_frames(size_t pitch)
 {
     if (pitch <= frames_pitch && d_frames) return HBD_OK;
-    if (d_frames) cudaFree(d_frames);
-    d_frames = nullptr;
     pitch = (pitch + 255) & ~size_t(255);
-    HBD_CUDA_CHECK(cudaMalloc((void**)&d_frames, size_t(n_ch) * pitch));
-    frames_pitch = pitch;
-    if (!d_frame_sizes) HBD_CUDA_CHECK(dalloc(&d_frame_sizes, size_t(n_ch)));
-    h_frame_sizes.resize(size_t(n_ch));
+    DevPtr<unsigned char> frames;
+    HBD_CUDA_CHECK(dev_alloc(frames, size_t(n_ch) * pitch));
+    d_frames = std::move(frames); frames_pitch = pitch;
     return HBD_OK;
 }
 
@@ -2040,11 +1987,10 @@ int hbd_decoder::ensure_dacc()
     const double fs_dec = fs_in / factor;
     size_t need = 0;
     for (const auto& x : hc) if (x.baud > 0) need = std::max(need, size_t(fs_dec / x.baud * 50));
-    need += demod_pitch + 64;
-    if (!d_dacc_n) { HBD_CUDA_CHECK(dalloc(&d_dacc_n, size_t(n_ch))); HBD_CUDA_CHECK(cudaMemset(d_dacc_n, 0, sizeof(unsigned) * size_t(n_ch))); }
-    if (need > dacc_pitch) {
+    need += demod.pitch + 64;
+    if (need > dacc.pitch) {
         if (sync_groups()) return HBD_ERR_CUDA;
-        HBD_CUDA_CHECK(grow_rows(&d_dacc, &dacc_pitch, (need + 15) & ~size_t(15), size_t(n_ch), dacc_pitch, stream));
+        HBD_CUDA_CHECK(dacc.grow((need + 15) & ~size_t(15), size_t(n_ch), dacc.pitch, stream));
     }
     return HBD_OK;
 }
@@ -2066,33 +2012,33 @@ static size_t fetch_frames(hbd_decoder* h, int ch0, int nc, bool spectrum, float
     cudaSetDevice(h->device);
     if (h->sync_groups() || cudaStreamSynchronize(h->stream) != cudaSuccess) return 0;
     const size_t hdr = spectrum ? size_t(kSpectrumHeaderBytes) : size_t(kDemodHeaderBytes);
-    const size_t max_n = spectrum ? size_t(h->fft_n) : std::max<size_t>(h->dacc_pitch, 1);
+    const size_t max_n = spectrum ? size_t(h->fft_n) : std::max<size_t>(h->dacc.pitch, 1);
     const size_t need = hdr + std::min<size_t>(max_n, size_t(resolution)) * size_t(type_size);
     if (h->ensure_frames(need)) return 0;
     int nl = 0;
     cudaError_t e;
     if (spectrum) {
         SpectrumFrameArgs a{};
-        a.state = h->d_state; a.power = h->d_power; a.fft_n = h->fft_n; a.fs_dec = h->fs_in / h->factor; a.zoom = zoom; a.resolution = resolution; a.type_size = type_size;
-        a.out = h->d_frames; a.out_pitch = h->frames_pitch; a.sizes = h->d_frame_sizes; a.ch0 = ch0;
+        a.state = h->d_state.get(); a.power = h->fft.power.get(); a.fft_n = h->fft_n; a.fs_dec = h->fs_in / h->factor; a.zoom = zoom; a.resolution = resolution; a.type_size = type_size;
+        a.out = h->d_frames.get(); a.out_pitch = h->frames_pitch; a.sizes = h->d_frame_sizes.get(); a.ch0 = ch0;
         e = launch_spectrum_frames(a, nc, h->stream, &nl);
     } else {
-        if (!h->d_dacc || !h->d_dacc_n) return 0;
+        if (!h->dacc.get()) return 0;
         DemodFrameArgs a{};
-        a.acc = h->d_dacc; a.acc_pitch = h->dacc_pitch; a.acc_n = h->d_dacc_n; a.resolution = resolution; a.type_size = type_size;
-        a.out = h->d_frames; a.out_pitch = h->frames_pitch; a.sizes = h->d_frame_sizes; a.ch0 = ch0;
+        a.acc = h->dacc.get(); a.acc_pitch = h->dacc.pitch; a.acc_n = h->d_dacc_n.get(); a.resolution = resolution; a.type_size = type_size;
+        a.out = h->d_frames.get(); a.out_pitch = h->frames_pitch; a.sizes = h->d_frame_sizes.get(); a.ch0 = ch0;
         e = launch_demod_frames(a, nc, h->stream, &nl);
     }
     h->launches += unsigned(nl);
     if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return 0; }
-    if (cudaMemcpyAsync(h->h_frame_sizes.data(), h->d_frame_sizes, sizeof(unsigned) * size_t(nc), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess) return 0;
+    if (cudaMemcpyAsync(h->h_frame_sizes.data(), h->d_frame_sizes.get(), sizeof(unsigned) * size_t(nc), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess) return 0;
     if (cudaStreamSynchronize(h->stream) != cudaSuccess) return 0;
     size_t longest = 0;
     for (int i = 0; i < nc; ++i) longest = std::max<size_t>(longest, h->h_frame_sizes[size_t(i)]);
     if (sizes) for (int i = 0; i < nc; ++i) sizes[i] = h->h_frame_sizes[size_t(i)];
     if (out && pitch && longest) {
         const size_t w = std::min(pitch, longest);
-        if (cudaMemcpy2D(out, pitch, h->d_frames, h->frames_pitch, w, size_t(nc), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
+        if (cudaMemcpy2D(out, pitch, h->d_frames.get(), h->frames_pitch, w, size_t(nc), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
     }
     return longest;
 }
@@ -2132,14 +2078,14 @@ int hbd_afc_retune(hbd_decoder* h, double min_abs_hz, double* applied_out)
     cudaSetDevice(h->device);
     if (h->sync_groups()) return HBD_ERR_CUDA;
     const size_t n = size_t(h->n_ch);
-    double* d_applied = nullptr;
-    if (cudaMalloc((void**)&d_applied, n * sizeof(double)) != cudaSuccess) return HBD_ERR_NOMEM;
+    DevPtr<double> applied_d;
+    if (dev_alloc(applied_d, n) != cudaSuccess) return HBD_ERR_NOMEM;
+    double* d_applied = applied_d.get();
     std::vector<double> applied(n, 0.0);
-    cudaError_t e = launch_afc_retune(h->d_state, h->n_ch, min_abs_hz, h->fs_in / h->factor, d_applied, h->fft_n, h->stream);
+    cudaError_t e = launch_afc_retune(h->d_state.get(), h->n_ch, min_abs_hz, h->fs_in / h->factor, d_applied, h->fft_n, h->stream);
     ++h->launches;
     if (e == cudaSuccess) e = cudaMemcpyAsync(applied.data(), d_applied, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    cudaFree(d_applied);
     if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
     int count = 0;
     for (size_t c = 0; c < n; ++c) {
@@ -2159,7 +2105,7 @@ size_t hbd_get_stats_batch(hbd_decoder* h, double* out, size_t cap_doubles)
     h->sync_groups();
     cudaStreamSynchronize(h->stream);
     std::vector<ChanState> st(n);
-    if (cudaMemcpy(st.data(), h->d_state, n * sizeof(ChanState), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
+    if (cudaMemcpy(st.data(), h->d_state.get(), n * sizeof(ChanState), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
     for (size_t c = 0; c < n; ++c) {
         out[6 * c + 0] = st[c].afc_correction; out[6 * c + 1] = st[c].afc_shift_hz;
         out[6 * c + 2] = st[c].afc_noise_floor; out[6 * c + 3] = st[c].afc_noise_var;
@@ -2196,30 +2142,30 @@ size_t hbd_debug_stage(hbd_decoder* h, int ch, int stage, float* out, size_t cap
     const HostChan& x = h->hc[size_t(ch)];
     switch (stage) {
     case HBD_STAGE_DECIMATED:
-        if (!h->d_rec_dec) return 0;
-        return fetch_floats(h, h->d_rec_dec + size_t(ch) * h->rec_pitch, 2 * size_t(x.last_n2), out, cap);
+        if (!h->rec.get(0)) return 0;
+        return fetch_floats(h, h->rec.get(0) + size_t(ch) * h->rec.pitch, 2 * size_t(x.last_n2), out, cap);
     case HBD_STAGE_FILTERED:
-        if (!h->d_rec_filt) return 0;
-        return fetch_floats(h, h->d_rec_filt + size_t(ch) * h->rec_pitch, 2 * size_t(x.last_nf), out, cap);
+        if (!h->rec.get(1)) return 0;
+        return fetch_floats(h, h->rec.get(1) + size_t(ch) * h->rec.pitch, 2 * size_t(x.last_nf), out, cap);
     case HBD_STAGE_DEMOD:
-        if (!h->d_demod) return 0;
-        return fetch_floats(h, h->d_demod + size_t(ch) * h->demod_pitch, size_t(x.last_nf), out, cap);
+        if (!h->demod.get()) return 0;
+        return fetch_floats(h, h->demod.get() + size_t(ch) * h->demod.pitch, size_t(x.last_nf), out, cap);
     case HBD_STAGE_LPTAPS:
-        return fetch_floats(h, h->d_lptaps + size_t(ch) * kLpMaxTaps, x.lp_ntaps, out, cap);
+        return fetch_floats(h, h->d_lptaps.get() + size_t(ch) * kLpMaxTaps, x.lp_ntaps, out, cap);
     case HBD_STAGE_PENDING: {
         ChanState st; if (fetch_state(h, ch, &st)) return 0;
-        if (!h->d_slicer) return 0;
-        return fetch_floats(h, h->d_slicer + size_t(ch) * h->slicer_pitch, st.slicer_n, out, cap);
+        if (!h->slicer.get()) return 0;
+        return fetch_floats(h, h->slicer.get() + size_t(ch) * h->slicer.pitch, st.slicer_n, out, cap);
     }
     case HBD_STAGE_BITS: {
-        if (!h->d_rec_bits) return 0;
+        if (!h->d_rec_bits.get()) return 0;
         cudaSetDevice(h->device); h->sync_groups(); cudaStreamSynchronize(h->stream);
         unsigned nb = 0;
-        cudaMemcpy(&nb, h->d_rec_bits_n + ch, 4, cudaMemcpyDeviceToHost);
+        cudaMemcpy(&nb, h->d_rec_bits_n.get() + ch, 4, cudaMemcpyDeviceToHost);
         nb = std::min(nb, h->rec_bits_pitch);
         if (out && cap && nb) {
             std::vector<unsigned char> b(nb);
-            cudaMemcpy(b.data(), h->d_rec_bits + size_t(ch) * h->rec_bits_pitch, nb, cudaMemcpyDeviceToHost);
+            cudaMemcpy(b.data(), h->d_rec_bits.get() + size_t(ch) * h->rec_bits_pitch, nb, cudaMemcpyDeviceToHost);
             for (size_t i = 0; i < std::min<size_t>(nb, cap); ++i) out[i] = float(b[i]);
         }
         return nb;

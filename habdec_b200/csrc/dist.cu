@@ -7,6 +7,7 @@
 // used.  Only the long-stable part of the NCCL API is touched.
 #include "../../include/habdec_b200.h"
 #include "api_internal.h"
+#include "cuda_res.h"
 
 #include <cuda_runtime.h>
 #include <dlfcn.h>
@@ -65,40 +66,30 @@ struct DistCtx {
     int rank = 0, world = 1;
     ncclComm comm = nullptr;
     bool own_comm = false;
-    cudaStream_t stream = nullptr;
+    hbd::Stream stream;                        // declared before the buffers and events, so it is destroyed after them
     std::vector<int> counts, offsets;          // channels per rank, first record of every rank in the gathered buffer
     int total = 0;
     // A gather must not stall the thread that also feeds the GPU: senders enqueue and return (their buffers rotate through
     // a pool of kPool slots, a slot is reused once its send has completed), and rank 0 hands its pinned receive buffer to
     // the sink WITHOUT copying (hbd::sink_feed_borrowed); the sink is flushed before that slot comes round again.
     static constexpr int kPool = 4;
-    hbd_result_record* h_send[kPool] = {};     // pinned, counts[rank] records each
-    hbd_result_record* d_send[kPool] = {};
-    cudaEvent_t ev_sent[kPool] = {};
-    hbd_result_record* d_recv = nullptr;       // rank 0: total records
-    hbd_result_record* h_recv[kPool] = {};     // rank 0: pinned, total records each
+    hbd::HostPtr<hbd_result_record> h_send[kPool];   // pinned, counts[rank] records each
+    hbd::DevPtr<hbd_result_record> d_send[kPool];
+    hbd::Event ev_sent[kPool];
+    hbd::DevPtr<hbd_result_record> d_recv;     // rank 0: total records
+    hbd::HostPtr<hbd_result_record> h_recv[kPool];   // rank 0: pinned, total records each
     hbd_result_sink* fed[kPool] = {};          // the sink that borrowed slot k
-    int* d_cnt = nullptr;
+    hbd::DevPtr<int> d_cnt;
     unsigned long long gathers = 0;
-};
-
-void free_ctx(DistCtx* c)
-{
-    if (!c) return;
-    if (c->stream) cudaStreamSynchronize(c->stream);
-    if (c->own_comm && c->comm && nccl_api()->CommDestroy) nccl_api()->CommDestroy(c->comm);
-    for (int k = 0; k < DistCtx::kPool; ++k) {
-        if (c->fed[k]) hbd::sink_flush(c->fed[k]);
-        if (c->h_send[k]) cudaFreeHost(c->h_send[k]);
-        if (c->h_recv[k]) cudaFreeHost(c->h_recv[k]);
-        if (c->d_send[k]) cudaFree(c->d_send[k]);
-        if (c->ev_sent[k]) cudaEventDestroy(c->ev_sent[k]);
+    // the steps that must come before the members release themselves: nothing in flight on the stream, the owned
+    // communicator destroyed, every sink that borrows a pinned receive buffer flushed
+    ~DistCtx()
+    {
+        if (stream) cudaStreamSynchronize(stream.get());
+        if (own_comm && comm && nccl_api()->CommDestroy) nccl_api()->CommDestroy(comm);
+        for (hbd_result_sink* f : fed) if (f) hbd::sink_flush(f);
     }
-    if (c->d_recv) cudaFree(c->d_recv);
-    if (c->d_cnt) cudaFree(c->d_cnt);
-    if (c->stream) cudaStreamDestroy(c->stream);
-    delete c;
-}
+};
 
 int fail(hbd_decoder* h, const std::string& what)
 {
@@ -110,33 +101,33 @@ int setup(hbd_decoder* h, DistCtx* c)
 {
     NcclApi* n = nccl_api();
     const int n_ch = hbd_n_channels(h);
-    if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) return fail(h, "dist: stream");
+    if (hbd::stream_create(c->stream) != cudaSuccess) return fail(h, "dist: stream");
     // every rank learns how many channels the others own (one tiny all-gather at start-up)
-    if (cudaMalloc((void**)&c->d_cnt, sizeof(int) * size_t(c->world + 1)) != cudaSuccess) return fail(h, "dist: cudaMalloc");
-    if (cudaMemcpyAsync(c->d_cnt + c->world, &n_ch, sizeof(int), cudaMemcpyHostToDevice, c->stream) != cudaSuccess) return fail(h, "dist: memcpy");
+    if (hbd::dev_alloc(c->d_cnt, size_t(c->world + 1)) != cudaSuccess) return fail(h, "dist: cudaMalloc");
+    if (cudaMemcpyAsync(c->d_cnt.get() + c->world, &n_ch, sizeof(int), cudaMemcpyHostToDevice, c->stream.get()) != cudaSuccess) return fail(h, "dist: memcpy");
     c->counts.assign(size_t(c->world), n_ch);
     if (c->world > 1) {
-        const ncclResult r = n->AllGather(c->d_cnt + c->world, c->d_cnt, 1, kNcclInt32, c->comm, c->stream);
+        const ncclResult r = n->AllGather(c->d_cnt.get() + c->world, c->d_cnt.get(), 1, kNcclInt32, c->comm, c->stream.get());
         if (r) return fail(h, std::string("ncclAllGather: ") + n->GetErrorString(r));
-        if (cudaMemcpyAsync(c->counts.data(), c->d_cnt, sizeof(int) * size_t(c->world), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) return fail(h, "dist: memcpy");
+        if (cudaMemcpyAsync(c->counts.data(), c->d_cnt.get(), sizeof(int) * size_t(c->world), cudaMemcpyDeviceToHost, c->stream.get()) != cudaSuccess) return fail(h, "dist: memcpy");
     }
-    if (cudaStreamSynchronize(c->stream) != cudaSuccess) return fail(h, "dist: all-gather of the channel counts failed");
+    if (cudaStreamSynchronize(c->stream.get()) != cudaSuccess) return fail(h, "dist: all-gather of the channel counts failed");
     c->offsets.assign(size_t(c->world), 0);
     c->total = 0;
     for (int r = 0; r < c->world; ++r) { c->offsets[size_t(r)] = c->total; c->total += c->counts[size_t(r)]; }
-    const size_t mine = sizeof(hbd_result_record) * size_t(n_ch), all = sizeof(hbd_result_record) * size_t(c->total);
+    const size_t mine = size_t(n_ch), all = size_t(c->total);
     for (int k = 0; k < DistCtx::kPool; ++k) {
-        if (cudaHostAlloc((void**)&c->h_send[k], mine, cudaHostAllocDefault) != cudaSuccess || cudaMalloc((void**)&c->d_send[k], mine) != cudaSuccess ||
-            cudaEventCreateWithFlags(&c->ev_sent[k], cudaEventDisableTiming) != cudaSuccess) return fail(h, "dist: buffers");
-        if (c->rank == 0 && c->world > 1 && cudaHostAlloc((void**)&c->h_recv[k], all, cudaHostAllocDefault) != cudaSuccess) return fail(h, "dist: buffers");
+        if (hbd::host_alloc(c->h_send[k], mine) != cudaSuccess || hbd::dev_alloc(c->d_send[k], mine) != cudaSuccess ||
+            hbd::event_create(c->ev_sent[k]) != cudaSuccess) return fail(h, "dist: buffers");
+        if (c->rank == 0 && c->world > 1 && hbd::host_alloc(c->h_recv[k], all) != cudaSuccess) return fail(h, "dist: buffers");
     }
-    if (c->rank == 0 && c->world > 1 && cudaMalloc((void**)&c->d_recv, all) != cudaSuccess) return fail(h, "dist: buffers");
+    if (c->rank == 0 && c->world > 1 && hbd::dev_alloc(c->d_recv, all) != cudaSuccess) return fail(h, "dist: buffers");
     return HBD_OK;
 }
 
 } // namespace
 
-namespace hbd { void internal_free_dist(void* ctx) { free_ctx(static_cast<DistCtx*>(ctx)); } }
+namespace hbd { void internal_free_dist(void* ctx) { delete static_cast<DistCtx*>(ctx); } }
 
 extern "C" {
 
@@ -153,14 +144,14 @@ int hbd_dist_unique_id(unsigned char out[128])
 
 static int dist_attach(hbd_decoder* h, int rank, int world, ncclComm comm, bool own)
 {
-    void** slot = hbd::internal_dist_slot(h);
-    if (*slot) { free_ctx(static_cast<DistCtx*>(*slot)); *slot = nullptr; }
-    DistCtx* c = new DistCtx;
+    hbd::DistSlot& slot = hbd::internal_dist_slot(h);
+    slot.reset();
+    std::unique_ptr<DistCtx> c(new DistCtx);
     c->rank = rank; c->world = world; c->comm = comm; c->own_comm = own;
-    int rc = setup(h, c);
+    int rc = setup(h, c.get());
     if (!rc) rc = hbd_set_stats_snapshot(h, 1);   // a gather never waits for calls in flight
-    if (rc) { free_ctx(c); return rc; }
-    *slot = c;
+    if (rc) return rc;
+    slot.reset(c.release());
     return HBD_OK;
 }
 
@@ -191,15 +182,15 @@ int hbd_dist_use_comm(hbd_decoder* h, void* nccl_comm, int rank, int world)
 int hbd_dist_finalize(hbd_decoder* h)
 {
     if (!h) return HBD_ERR_ARG;
-    void** slot = hbd::internal_dist_slot(h);
-    if (*slot) { cudaSetDevice(hbd::internal_device(h)); free_ctx(static_cast<DistCtx*>(*slot)); *slot = nullptr; }   // flushes the sinks it fed
+    hbd::DistSlot& slot = hbd::internal_dist_slot(h);
+    if (slot) { cudaSetDevice(hbd::internal_device(h)); slot.reset(); }   // flushes the sinks it fed
     return HBD_OK;
 }
 
 int hbd_dist_total_channels(hbd_decoder* h)
 {
     if (!h) return 0;
-    DistCtx* c = static_cast<DistCtx*>(*hbd::internal_dist_slot(h));
+    DistCtx* c = static_cast<DistCtx*>(hbd::internal_dist_slot(h).get());
     return c ? c->total : hbd_n_channels(h);
 }
 
@@ -209,7 +200,7 @@ int hbd_dist_total_channels(hbd_decoder* h)
 int hbd_gather_results(hbd_decoder* h, hbd_result_sink* sink)
 {
     if (!h) return HBD_ERR_ARG;
-    DistCtx* c = static_cast<DistCtx*>(*hbd::internal_dist_slot(h));
+    DistCtx* c = static_cast<DistCtx*>(hbd::internal_dist_slot(h).get());
     if (!c) { hbd::internal_set_error(h, "hbd_gather_results: call hbd_dist_init first"); return HBD_ERR_STATE; }
     if (c->rank == 0 && !sink) return HBD_ERR_ARG;
     if (cudaSetDevice(hbd::internal_device(h)) != cudaSuccess) return HBD_ERR_CUDA;
@@ -217,37 +208,37 @@ int hbd_gather_results(hbd_decoder* h, hbd_result_sink* sink)
     const int mine = c->counts[size_t(c->rank)];
     const int k = int(c->gathers % DistCtx::kPool);
     // slot k comes round again: its send has long completed; a sink that still borrows it takes its records in now
-    if (c->gathers >= DistCtx::kPool && cudaEventSynchronize(c->ev_sent[k]) != cudaSuccess) return fail(h, "gather: earlier send failed");
+    if (c->gathers >= DistCtx::kPool && cudaEventSynchronize(c->ev_sent[k].get()) != cudaSuccess) return fail(h, "gather: earlier send failed");
     if (c->fed[k]) { hbd::sink_flush(c->fed[k]); c->fed[k] = nullptr; }
-    const size_t got = hbd_pack_results(h, c->offsets[size_t(c->rank)], c->h_send[k], size_t(mine));
+    const size_t got = hbd_pack_results(h, c->offsets[size_t(c->rank)], c->h_send[k].get(), size_t(mine));
     if (got != size_t(mine)) return HBD_ERR_STATE;
     const size_t rec = sizeof(hbd_result_record);
     if (c->world > 1) {
         if (c->rank != 0) {
             // enqueue and return: nothing here waits for rank 0 (which may be busy draining its own channels)
-            if (cudaMemcpyAsync(c->d_send[k], c->h_send[k], rec * size_t(mine), cudaMemcpyHostToDevice, c->stream) != cudaSuccess) return fail(h, "gather: H2D");
-            const ncclResult r = n->Send(c->d_send[k], rec * size_t(mine), kNcclInt8, 0, c->comm, c->stream);
+            if (cudaMemcpyAsync(c->d_send[k].get(), c->h_send[k].get(), rec * size_t(mine), cudaMemcpyHostToDevice, c->stream.get()) != cudaSuccess) return fail(h, "gather: H2D");
+            const ncclResult r = n->Send(c->d_send[k].get(), rec * size_t(mine), kNcclInt8, 0, c->comm, c->stream.get());
             if (r) return fail(h, std::string("ncclSend: ") + n->GetErrorString(r));
-            if (cudaEventRecord(c->ev_sent[k], c->stream) != cudaSuccess) return fail(h, "gather: event");
+            if (cudaEventRecord(c->ev_sent[k].get(), c->stream.get()) != cudaSuccess) return fail(h, "gather: event");
         } else {
             ncclResult r = n->GroupStart();
             for (int p = 1; p < c->world && !r; ++p)
-                r = n->Recv(c->d_recv + c->offsets[size_t(p)], rec * size_t(c->counts[size_t(p)]), kNcclInt8, p, c->comm, c->stream);
+                r = n->Recv(c->d_recv.get() + c->offsets[size_t(p)], rec * size_t(c->counts[size_t(p)]), kNcclInt8, p, c->comm, c->stream.get());
             if (!r) r = n->GroupEnd();
             if (r) return fail(h, std::string("ncclRecv: ") + n->GetErrorString(r));
-            if (cudaMemcpyAsync(c->h_recv[k] + mine, c->d_recv + mine, rec * size_t(c->total - mine), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess)
+            if (cudaMemcpyAsync(c->h_recv[k].get() + mine, c->d_recv.get() + mine, rec * size_t(c->total - mine), cudaMemcpyDeviceToHost, c->stream.get()) != cudaSuccess)
                 return fail(h, "gather: D2H");
-            if (cudaEventRecord(c->ev_sent[k], c->stream) != cudaSuccess) return fail(h, "gather: event");
-            if (cudaStreamSynchronize(c->stream) != cudaSuccess) return fail(h, "gather: transfer failed");
+            if (cudaEventRecord(c->ev_sent[k].get(), c->stream.get()) != cudaSuccess) return fail(h, "gather: event");
+            if (cudaStreamSynchronize(c->stream.get()) != cudaSuccess) return fail(h, "gather: transfer failed");
         }
     }
     ++c->gathers;
     if (c->rank != 0) {   // a sink on another rank mirrors that rank's own channels (same global numbering)
-        if (sink) { const int rc = hbd::sink_feed_borrowed(sink, c->h_send[k], size_t(mine)); if (rc) return rc; c->fed[k] = sink; }
+        if (sink) { const int rc = hbd::sink_feed_borrowed(sink, c->h_send[k].get(), size_t(mine)); if (rc) return rc; c->fed[k] = sink; }
         return mine;
     }
-    int rc = hbd::sink_feed_borrowed(sink, c->h_send[k], size_t(mine));
-    if (c->world > 1 && !rc) rc = hbd::sink_feed_borrowed(sink, c->h_recv[k] + mine, size_t(c->total - mine));
+    int rc = hbd::sink_feed_borrowed(sink, c->h_send[k].get(), size_t(mine));
+    if (c->world > 1 && !rc) rc = hbd::sink_feed_borrowed(sink, c->h_recv[k].get() + mine, size_t(c->total - mine));
     c->fed[k] = sink;
     return rc ? rc : c->total;
 }

@@ -15,6 +15,7 @@
 //          shared memory), |X|^2, and the float64 sums of its 16 R bins kept in registers across the batch.
 // A batch holds at most 2^22 / N segments, so Y (32 MB) stays in L2 between the two passes.  No cuFFT.
 #include "../../include/habdec_b200.h"
+#include "cuda_res.h"
 #include "fft_dev.cuh"
 #include "iq_format.cuh"
 #include "scan.cuh"
@@ -179,17 +180,15 @@ struct hbd_scanner {
     int N = 0;
     int max_batch = 1;                 // segments per launch pair: 2^22 / N, Y = 32 MB
     cudaStream_t stream = nullptr;
-    bool own_stream = false;
-    cudaEvent_t ev_up = nullptr;       // a host push's upload has been read
-    float* d_win = nullptr;
-    float2* d_tw = nullptr;
-    float2* d_inter = nullptr;
-    double* d_acc = nullptr;
-    float2* d_carry[2] = {nullptr, nullptr};
+    Stream own_stream;                 // declared before the buffers and events, so it is destroyed after them
+    Event ev_up;                       // a host push's upload has been read
+    DevPtr<float> d_win;
+    DevPtr<float2> d_tw, d_inter;
+    DevPtr<double> d_acc;
+    DevPtr<float2> d_carry[2];
     int cur = 0;                       // d_carry[cur] holds the m samples from the next segment's start on
     size_t m = 0;
-    void* d_up = nullptr;              // host push staging
-    size_t up_bytes = 0;
+    Rows<unsigned char> up;            // host push staging, one row of `pitch` bytes
     double fs = 0;
     bool fs_set = false;
     unsigned long long n_seg = 0;
@@ -197,14 +196,8 @@ struct hbd_scanner {
 
     int fail(int rc, const std::string& what) { err = what; return rc; }
     int cuda_fail(cudaError_t e, const char* what) { return fail(HBD_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e)); }
-    void free_all()
-    {
-        for (void* p : {(void*)d_win, (void*)d_tw, (void*)d_inter, (void*)d_acc, (void*)d_carry[0], (void*)d_carry[1], d_up})
-            if (p) cudaFree(p);
-        if (ev_up) cudaEventDestroy(ev_up);
-        if (own_stream && stream) cudaStreamDestroy(stream);
-    }
     int process(const void* src, int format, size_t n);
+    ~hbd_scanner() { cudaSetDevice(device); if (stream) cudaStreamSynchronize(stream); }   // then the members release themselves
 };
 
 // the capture's next n samples (device memory, `format`) after the carry: every segment that is complete now, then the new carry
@@ -212,18 +205,18 @@ int hbd_scanner::process(const void* src, int format, size_t n)
 {
     const size_t H = size_t(N / 2), total = m + n;
     const size_t S = total >= size_t(N) ? (total - size_t(N)) / H + 1 : 0;
-    const ScanSrc s{d_carry[cur], m, src, format};
+    const ScanSrc s{d_carry[cur].get(), m, src, format};
     for (size_t b = 0; b < S; b += size_t(max_batch)) {
         const int nb = int(std::min<size_t>(size_t(max_batch), S - b));
-        const cudaError_t e = launch_scan_segments(s, b * H, nb, N, d_win, d_tw, d_inter, d_acc, stream);
+        const cudaError_t e = launch_scan_segments(s, b * H, nb, N, d_win.get(), d_tw.get(), d_inter.get(), d_acc.get(), stream);
         if (e != cudaSuccess) return cuda_fail(e, "scan kernels");
     }
     const size_t next = S * H, keep = total - next;   // < N
     if (!S) {   // no segment completed: the new samples are appended to the carry in place (most pushes at large N)
-        const cudaError_t e = launch_scan_carry(s, m, n, d_carry[cur] + m, stream);
+        const cudaError_t e = launch_scan_carry(s, m, n, d_carry[cur].get() + m, stream);
         if (e != cudaSuccess) return cuda_fail(e, "scan carry");
     } else {
-        const cudaError_t e = launch_scan_carry(s, next, keep, d_carry[cur ^ 1], stream);
+        const cudaError_t e = launch_scan_carry(s, next, keep, d_carry[cur ^ 1].get(), stream);
         if (e != cudaSuccess) return cuda_fail(e, "scan carry");
         cur ^= 1;
     }
@@ -242,22 +235,18 @@ int hbd_scanner_create(int cuda_device, size_t n_fft, hbd_scanner** out)
     int count = 0;
     if (cudaGetDeviceCount(&count) != cudaSuccess || cuda_device < 0 || cuda_device >= count) return HBD_ERR_CUDA;
     if (cudaSetDevice(cuda_device) != cudaSuccess) return HBD_ERR_CUDA;
-    hbd_scanner* s = new (std::nothrow) hbd_scanner;
+    std::unique_ptr<hbd_scanner> s(new (std::nothrow) hbd_scanner);
     if (!s) return HBD_ERR_NOMEM;
     const size_t N = n_fft;
     s->device = cuda_device;
     s->N = int(N);
     s->max_batch = int(std::max<size_t>(1, (size_t(1) << 22) / N));
-    auto bail = [&](int rc) { s->free_all(); delete s; return rc; };
-    if (cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking) != cudaSuccess) return bail(HBD_ERR_CUDA);
-    s->own_stream = true;
-    if (cudaEventCreateWithFlags(&s->ev_up, cudaEventDisableTiming) != cudaSuccess) return bail(HBD_ERR_CUDA);
-    if (cudaMalloc((void**)&s->d_win, N * sizeof(float)) != cudaSuccess ||
-        cudaMalloc((void**)&s->d_tw, (N + 4096 + 256 + N / 4096) * sizeof(float2)) != cudaSuccess ||
-        cudaMalloc((void**)&s->d_inter, size_t(s->max_batch) * N * sizeof(float2)) != cudaSuccess ||
-        cudaMalloc((void**)&s->d_acc, N * sizeof(double)) != cudaSuccess ||
-        cudaMalloc((void**)&s->d_carry[0], N * sizeof(float2)) != cudaSuccess ||
-        cudaMalloc((void**)&s->d_carry[1], N * sizeof(float2)) != cudaSuccess) return bail(HBD_ERR_NOMEM);
+    if (stream_create(s->own_stream) != cudaSuccess) return HBD_ERR_CUDA;
+    s->stream = s->own_stream.get();
+    if (event_create(s->ev_up) != cudaSuccess) return HBD_ERR_CUDA;
+    if (dev_alloc(s->d_win, N) != cudaSuccess || dev_alloc(s->d_tw, N + 4096 + 256 + N / 4096) != cudaSuccess ||
+        dev_alloc(s->d_inter, size_t(s->max_batch) * N) != cudaSuccess || dev_alloc(s->d_acc, N) != cudaSuccess ||
+        dev_alloc(s->d_carry[0], N) != cudaSuccess || dev_alloc(s->d_carry[1], N) != cudaSuccess) return HBD_ERR_NOMEM;
     // 4-term Blackman-Harris (habdec_windows.h:27-53), float64 -> float32, stored [r][n1] = w[R n1 + r]
     const size_t R = N / 4096;
     std::vector<float> w(N);
@@ -276,24 +265,14 @@ int hbd_scanner_create(int cuda_device, size_t n_fft, hbd_scanner** out)
     for (size_t k1 = 0; k1 < 16; ++k1) for (size_t t = 0; t < 256; ++t) tw[N + k1 * 256 + t] = cw(double(t * k1), 4096.0);
     for (size_t j1 = 0; j1 < 16; ++j1) for (size_t m2 = 0; m2 < 16; ++m2) tw[N + 4096 + j1 * 16 + m2] = cw(double(16 * m2 * j1), 4096.0);
     for (size_t j = 0; j < R; ++j) tw[N + 4096 + 256 + j] = cw(double(j), double(R));
-    if (cudaMemcpy(s->d_win, w.data(), N * sizeof(float), cudaMemcpyHostToDevice) != cudaSuccess ||
-        cudaMemcpy(s->d_tw, tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice) != cudaSuccess ||
-        cudaMemset(s->d_acc, 0, N * sizeof(double)) != cudaSuccess) return bail(HBD_ERR_CUDA);
-    *out = s;
+    if (cudaMemcpy(s->d_win.get(), w.data(), N * sizeof(float), cudaMemcpyHostToDevice) != cudaSuccess ||
+        cudaMemcpy(s->d_tw.get(), tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice) != cudaSuccess ||
+        cudaMemset(s->d_acc.get(), 0, N * sizeof(double)) != cudaSuccess) return HBD_ERR_CUDA;
+    *out = s.release();
     return HBD_OK;
 }
 
-void hbd_scanner_destroy(hbd_scanner* s)
-{
-    if (!s) return;
-    {
-        std::lock_guard<std::mutex> l(s->mtx);
-        cudaSetDevice(s->device);
-        cudaStreamSynchronize(s->stream);
-        s->free_all();
-    }
-    delete s;
-}
+void hbd_scanner_destroy(hbd_scanner* s) { delete s; }
 
 const char* hbd_scanner_last_error(hbd_scanner* s) { return s ? s->err.c_str() : "null handle"; }
 
@@ -303,9 +282,8 @@ int hbd_scanner_set_stream(hbd_scanner* s, void* cuda_stream)
     std::lock_guard<std::mutex> l(s->mtx);
     cudaSetDevice(s->device);
     cudaStreamSynchronize(s->stream);
-    if (s->own_stream) cudaStreamDestroy(s->stream);
+    s->own_stream.reset();
     s->stream = (cudaStream_t)cuda_stream;
-    s->own_stream = false;
     return HBD_OK;
 }
 
@@ -326,22 +304,15 @@ static int scan_push(hbd_scanner* s, const void* iq, int format, size_t n, doubl
     // host capture: uploaded in pieces of at most 2^24 samples (the spectrum does not depend on the cut), the caller owns
     // `iq` again on return
     const size_t piece = size_t(1) << 24;
-    const size_t want = std::min(n, piece) * bytes;
-    if (want > s->up_bytes) {
-        cudaStreamSynchronize(s->stream);
-        if (s->d_up) cudaFree(s->d_up);
-        s->d_up = nullptr; s->up_bytes = 0;
-        if (cudaMalloc(&s->d_up, want) != cudaSuccess) return s->fail(HBD_ERR_NOMEM, "scan upload buffer");
-        s->up_bytes = want;
-    }
+    if (s->up.grow(std::min(n, piece) * bytes, 1, 0, s->stream) != cudaSuccess) return s->fail(HBD_ERR_NOMEM, "scan upload buffer");
     for (size_t o = 0; o < n; o += piece) {
         const size_t k = std::min(piece, n - o);
-        cudaError_t e = cudaMemcpyAsync(s->d_up, static_cast<const unsigned char*>(iq) + o * bytes, k * bytes, cudaMemcpyHostToDevice, s->stream);
+        cudaError_t e = cudaMemcpyAsync(s->up.get(), static_cast<const unsigned char*>(iq) + o * bytes, k * bytes, cudaMemcpyHostToDevice, s->stream);
         if (e != cudaSuccess) return s->cuda_fail(e, "scan upload");
-        const int rc = s->process(s->d_up, format, k);
+        const int rc = s->process(s->up.get(), format, k);
         if (rc) return rc;
-        e = cudaEventRecord(s->ev_up, s->stream);
-        if (e == cudaSuccess) e = cudaEventSynchronize(s->ev_up);
+        e = cudaEventRecord(s->ev_up.get(), s->stream);
+        if (e == cudaSuccess) e = cudaEventSynchronize(s->ev_up.get());
         if (e != cudaSuccess) return s->cuda_fail(e, "scan upload sync");
     }
     return HBD_OK;
@@ -355,7 +326,7 @@ int hbd_scan_reset(hbd_scanner* s)
     if (!s) return HBD_ERR_ARG;
     std::lock_guard<std::mutex> l(s->mtx);
     if (cudaSetDevice(s->device) != cudaSuccess) return s->fail(HBD_ERR_CUDA, "cudaSetDevice");
-    const cudaError_t e = cudaMemsetAsync(s->d_acc, 0, size_t(s->N) * sizeof(double), s->stream);
+    const cudaError_t e = cudaMemsetAsync(s->d_acc.get(), 0, size_t(s->N) * sizeof(double), s->stream);
     if (e != cudaSuccess) return s->cuda_fail(e, "scan reset");
     s->m = 0; s->n_seg = 0; s->fs = 0; s->fs_set = false;
     return HBD_OK;
@@ -369,7 +340,7 @@ static int scan_psd(hbd_scanner* s, std::vector<float>& psd)
     if (!s->n_seg) return HBD_OK;
     std::vector<double> acc(N);
     if (cudaSetDevice(s->device) != cudaSuccess) return s->fail(HBD_ERR_CUDA, "cudaSetDevice");
-    cudaError_t e = cudaMemcpyAsync(acc.data(), s->d_acc, N * sizeof(double), cudaMemcpyDeviceToHost, s->stream);
+    cudaError_t e = cudaMemcpyAsync(acc.data(), s->d_acc.get(), N * sizeof(double), cudaMemcpyDeviceToHost, s->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s->stream);
     if (e != cudaSuccess) return s->cuda_fail(e, "scan read-back");
     const double den = double(s->n_seg) * s->win_sq;

@@ -59,7 +59,8 @@ const char* hbd_last_error(hbd_decoder* h);
 /* run all work on this cudaStream_t (default: a private non-blocking stream) */
 int  hbd_set_stream(hbd_decoder* h, void* cuda_stream);
 /* spectrum / AFC FFT size: 4096 (the reference's fft_bins_cnt_, Decoder.h:163; default) or 16384 (the 16k-bin
- * spectrum of BASELINE configs[1]).  Restarts spectrum collection and the AFC averages of every channel. */
+ * spectrum of BASELINE configs[1]).  Restarts spectrum collection and the AFC averages of every channel.
+ * On failure the previous size, spectra and AFC averages stay in force. */
 int  hbd_set_fft_size(hbd_decoder* h, size_t n_bins);
 /* keep per-call stage arrays (decimated IQ, filtered IQ, slicer bits) for hbd_debug_stage(); test use */
 int  hbd_set_record(hbd_decoder* h, int on);
@@ -80,6 +81,7 @@ int    hbd_get_dc_remove(hbd_decoder* h, int ch);
 /* returns the new factor; the current one if out of [1,256]; 0 if not a supported power of two (:268-332) */
 size_t hbd_setup_decimation_factor(hbd_decoder* h, size_t factor);
 /* Decoder::setupDecimationStagesBW (:336-412); returns 0 before the first push latched a sampling rate */
+/* Either setup returns 0 when the new plan cannot be installed (e.g. out of device memory): the previous plan stays in force. */
 size_t hbd_setup_decimation_bw(hbd_decoder* h, double max_sampling_rate);
 
 /* ---- feed (Decoder::pushSamples, Decoder.h:206-219).  iq = interleaved cf32, n in complex samples.
