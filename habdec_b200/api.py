@@ -143,6 +143,7 @@ SIGNATURES = {
     "hbd_collect": (C.c_int, [_H]),
     "hbd_collect_ready": (C.c_int, [_H, C.c_uint]),
     "hbd_synchronize": (C.c_int, [_H]),
+    "hbd_reset_channels": (C.c_int, [_H, C.c_void_p, C.c_size_t]),
     "hbd_kernel_launches": (C.c_ulonglong, [_H]),
     "hbd_set_kernel_timing": (C.c_int, [_H, C.c_int]),
     "hbd_get_kernel_timing": (C.c_int, [_H, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_uint)]),
@@ -216,6 +217,7 @@ SIGNATURES = {
     "hbd_tracker_push": (C.c_int, [C.c_void_p, C.c_int, C.c_char_p, C.c_char_p, C.c_char_p]),
     "hbd_tracker_push_sentence": (C.c_int, [C.c_void_p, C.c_int, C.c_char_p]),
     "hbd_tracker_poll": (C.c_size_t, [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t]),
+    "hbd_tracker_reset": (C.c_int, [C.c_void_p, C.c_int]),
     "hbd_tracker_stats": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(ChannelStats)]),
     "hbd_tracker_stats_payload": (C.c_size_t, [C.c_void_p, C.c_int, C.c_int, C.c_char_p, C.c_size_t]),
     "hbd_tracker_get_sentence": (C.c_size_t, [C.c_void_p, C.c_int, C.c_int, C.c_char_p, C.c_size_t]),
@@ -467,6 +469,10 @@ class Tracker:
     def set_clock(self, now_unix: int): self._lib.hbd_tracker_set_clock(self._t, int(now_unix))
     def push(self, ch: int, callsign: bytes, data: bytes, crc: bytes) -> int: return self._lib.hbd_tracker_push(self._t, ch, callsign, data, crc)
     def push_sentence(self, ch: int, sentence: bytes) -> int: return self._lib.hbd_tracker_push_sentence(self._t, ch, sentence)
+    def reset(self, ch: int):
+        """Forget channel `ch`: its stats, sentences map and unpolled records (hbd_tracker_reset)."""
+        if self._lib.hbd_tracker_reset(self._t, int(ch)) != HBD_OK:
+            raise HbdError("hbd_tracker_reset failed")
 
     def set_callback(self, fn):
         self._cb = TELEMETRY_CB(lambda user, ch, t, s: fn(ch, _telemetry_dict(t.contents), s)) if fn else C.cast(None, TELEMETRY_CB)
@@ -725,10 +731,17 @@ class BatchDecoder:
     def collect(self): self._chk(self._lib.hbd_collect(self._h))
     def collect_ready(self, lag: int): self._chk(self._lib.hbd_collect_ready(self._h, int(lag)))
     def synchronize(self): self._chk(self._lib.hbd_synchronize(self._h))
+
+    def reset_channels(self, chs):
+        """Channels `chs` start over like a new decoder with the same settings (hbd_reset_channels): calls in flight are
+        drained first, unpolled output stays queued, the configuration and NCO frequency are kept."""
+        arr = np.ascontiguousarray(np.atleast_1d(np.asarray(chs, dtype=np.int32)))
+        self._chk(self._lib.hbd_reset_channels(self._h, arr.ctypes.data, arr.size))
     def kernel_launches(self) -> int: return int(self._lib.hbd_kernel_launches(self._h))
     def set_kernel_timing(self, on): self._chk(self._lib.hbd_set_kernel_timing(self._h, int(on)))   # 0 off, 1 K1 only, 2 K1 + rest of step
     def kernel_timing(self, which: int):
-        """(total_ms, launches) of K1 (which=0) or of the rest of the step (which=1) since set_kernel_timing."""
+        """(total_ms, count) since set_kernel_timing: K1 (which=0) or the rest of the step (which=1) with their launches; 5: the
+        drains' host replay and calls drained; 6: host planning of the calls and frame counters stepped (hbd_get_kernel_timing)."""
         ms, cnt = C.c_double(0), C.c_uint(0)
         self._chk(self._lib.hbd_get_kernel_timing(self._h, which, C.byref(ms), C.byref(cnt)))
         return ms.value, cnt.value

@@ -63,11 +63,12 @@ constexpr int kMaxMidStages = 6;   // a cascaded plan has at most 8 stages: K1's
 // host mirror of one channel, part 1: stream counters that are pure functions of the push sizes (and of the
 // low-pass configuration).  While every channel is fed the same way they are identical for all channels, and only
 // hc[0]'s copy is kept current (hbd_decoder::ctr_uniform / sync_ctrs): a steady-state call costs O(1) host work.
+// The FFT frame fill is not among them (HostChan::fft_have, hbd_decoder::fft_lvl): a channel reset in mid-stream
+// starts its frame empty while the others are partway through theirs, and agrees with them in everything else.
 struct ChanCtr {
     unsigned in_r = 0, dec_pending = 0;
     size_t grown1 = 0, grown2 = 0, grown_lp = 0;
     size_t grown_mid[kMaxMidStages] = {0, 0, 0, 0, 0, 0};   // work-buffer sizes of the middle stages of a cascaded plan
-    unsigned fft_have = 0;   // mirror of ChanState::fft_have: tells the host which calls complete an FFT frame (K4 launch)
     size_t lp_input_size = 0, lp_ntaps = 0;
     unsigned pushed = 0;     // samples waiting in the staging row
     unsigned last_nf = 0, last_n2 = 0;
@@ -77,7 +78,7 @@ struct ChanCtr {
     {
         for (int k = 0; k < kMaxMidStages; ++k) if (grown_mid[k] != o.grown_mid[k]) return false;
         return in_r == o.in_r && dec_pending == o.dec_pending && grown1 == o.grown1 && grown2 == o.grown2 && grown_lp == o.grown_lp &&
-               fft_have == o.fft_have && lp_input_size == o.lp_input_size && lp_ntaps == o.lp_ntaps && pushed == o.pushed &&
+               lp_input_size == o.lp_input_size && lp_ntaps == o.lp_ntaps && pushed == o.pushed &&
                last_nf == o.last_nf && last_n2 == o.last_n2 && demod_n == o.demod_n && lp_dirty == o.lp_dirty;
     }
 };
@@ -90,6 +91,9 @@ struct HostChan : ChanCtr {
     bool dc_remove = false;
     double nco_freq = 0, nco_phase = 0; // pre-mixer: frequency in Hz, phase (cycles) of the next pushed sample
     bool cfg_dirty = true;
+    // mirror of ChanState::fft_have: tells the host which calls complete an FFT frame (K4 launch).  Current in per-channel
+    // mode only; in uniform mode the channel's frame level (hbd_decoder::fft_lvl) holds it.
+    unsigned fft_have = 0;
     ChanCtr& ctr() { return *this; }
 };
 
@@ -104,7 +108,6 @@ struct ChanStep {
     bool zero_lphist = false;      // FirFilter.h:141-147
     bool taps_changed = false;     // low-pass redesigned: upload `taps`
     size_t taps_old = 0, taps_new = 0;
-    bool frame_done = false;       // this call completes an FFT frame (K4 runs)
     unsigned nf = 0;
 };
 
@@ -129,6 +132,37 @@ __global__ void init_cfg_kernel(ChanState* st, const double* baud, const float* 
     st[ch].rtty_bits = bits[ch];
     st[ch].dc_remove = dc[ch];
     st[ch].lp_ntaps = ntaps[ch];
+}
+
+// ChanState of a newly created decoder: Average<T>'s constructor add()s one 0, so the counts start at 1 (Average.h:34-37);
+// the configuration fields are those of a channel no setter has reached yet (the next call's upload fills them in)
+__host__ __device__ inline void fresh_state(ChanState& s)
+{
+    memset(&s, 0, sizeof(s));
+    s.baud = 1; // SymbolExtractor.h:96
+    s.nf_cnt = s.nv_cnt = s.pl_cnt = s.pr_cnt = 1;
+}
+
+// hbd_reset_channels: one CTA per listed channel.  Besides the state it restarts what the next call reads below a count
+// it does not find in ChanState: the low-pass work buffer with its stale-input slots (FirFilter.h:139-147 keep them
+// for a longer filter), and the per-channel counts of the demod accumulator, the SSDV ring and the recorded bits.
+// The carry and stage histories are zeroed by the next call's plan (grown* == 0); every other row is rewritten
+// before it is read (FFT frame from fft_have = 0, spectra behind have_spectrum, slicer / mask / UART rows below
+// their counts).
+struct ResetArgs {
+    ChanState* state; const int* list;
+    float2* decq; size_t dq_pitch;   // nullptr before the first call sized it
+    unsigned* dacc_n; unsigned* ssdv_total; unsigned* ssdv_scanned; unsigned* rec_bits_n;   // the last three may be nullptr
+};
+__global__ void reset_chan_kernel(ResetArgs a)
+{
+    const int ch = a.list[blockIdx.x];
+    if (a.decq) for (int i = threadIdx.x; i < kLpHist; i += blockDim.x) a.decq[size_t(ch) * a.dq_pitch + i] = make_float2(0.f, 0.f);
+    if (threadIdx.x) return;
+    fresh_state(a.state[ch]);
+    a.dacc_n[ch] = 0;
+    if (a.ssdv_total) { a.ssdv_total[ch] = 0; a.ssdv_scanned[ch] = 0; }
+    if (a.rec_bits_n) a.rec_bits_n[ch] = 0;
 }
 
 // the per-channel scalars that travel with the gathered results (hbd_result_record), packed after every call
@@ -234,7 +268,29 @@ struct hbd_decoder {
     bool derived_dirty = true;       // max_lp_taps_c / max_spb_c need recomputing
     size_t max_lp_taps_c = 1; double max_spb_c = 1;
     void sync_ctrs() { if (ctr_stale) { for (size_t c = 1; c < hc.size(); ++c) hc[c].ctr() = hc[0].ctr(); ctr_stale = false; } }
-    void leave_uniform() { sync_ctrs(); ctr_uniform = false; }
+    // FFT frame levels: in uniform mode the distinct frame fills of the channels (fft_lvl) and each channel's index into it
+    // (lvl_of).  A uniform call steps every level once; without resets there is exactly one.
+    std::vector<unsigned> fft_lvl{0u}, lvl_of;
+    void leave_uniform()
+    {
+        sync_ctrs();
+        if (ctr_uniform) for (size_t c = 0; c < hc.size(); ++c) hc[c].fft_have = fft_lvl[lvl_of[c]];
+        ctr_uniform = false;
+    }
+    // back to uniform mode once every channel's ChanCtr agrees again; the frame fills become levels.  O(n log n), called
+    // only where the channels have just been stepped or changed one by one.
+    void regroup()
+    {
+        ctr_uniform = true;
+        for (size_t c = 1; c < hc.size() && ctr_uniform; ++c) ctr_uniform = hc[c].same(hc[0]);
+        if (!ctr_uniform) return;
+        fft_lvl.clear();
+        for (const HostChan& x : hc) fft_lvl.push_back(x.fft_have);
+        std::sort(fft_lvl.begin(), fft_lvl.end());
+        fft_lvl.erase(std::unique(fft_lvl.begin(), fft_lvl.end()), fft_lvl.end());
+        for (size_t c = 0; c < hc.size(); ++c) lvl_of[c] = unsigned(std::lower_bound(fft_lvl.begin(), fft_lvl.end(), hc[c].fft_have) - fft_lvl.begin());
+    }
+    double plan_host_ms = 0; unsigned plan_steps = 0;   // host time of plan_call and frame counters it stepped (which = 6)
     // staged (host-pushed, not yet processed) samples: the same count in every channel?
     bool queue_depth_equal(unsigned& base)
     {
@@ -372,6 +428,8 @@ struct hbd_decoder {
     int enqueue_call(const CallPlan& cp);
     int process_async_locked();
     int collect_locked(unsigned lag);
+    HostPtr<int> h_reset; DevPtr<int> d_reset;   // channel list of hbd_reset_channels (allocated by the first one)
+    int reset_channels(const int* chs, size_t k);
     int log_pressure();
 };
 
@@ -427,11 +485,8 @@ int hbd_decoder::alloc_fixed()
     const size_t n = size_t(n_ch);
     HBD_CUDA_CHECK(dev_alloc(d_state, n));
     {
-        // Average<T>'s constructor add()s one 0: count starts at 1 (Average.h:34-37)
         ChanState init;
-        memset(&init, 0, sizeof(init));
-        init.baud = 1; // SymbolExtractor.h:96
-        init.nf_cnt = init.nv_cnt = init.pl_cnt = init.pr_cnt = 1;
+        fresh_state(init);
         std::vector<ChanState> all(n, init);
         HBD_CUDA_CHECK(cudaMemcpy(d_state.get(), all.data(), n * sizeof(ChanState), cudaMemcpyHostToDevice));
     }
@@ -607,7 +662,7 @@ int hbd_decoder::ensure_call_capacity(size_t n_in_max)
 // No CUDA calls in here.  Returns HBD_OK or HBD_ERR_ARG (nothing has been changed in that case)
 static int step_channel(hbd_decoder* h, HostChan& x, unsigned pushed, ChanStep& o, std::vector<float>& taps)
 {
-    const int factor = h->factor, M1 = h->M1, T1 = h->T1, M2 = h->M2, T2 = h->T2, fft_n = h->fft_n;
+    const int factor = h->factor, M1 = h->M1, T1 = h->T1, M2 = h->M2, T2 = h->T2;
     const double fs_dec = h->fs_in / factor;
     ChanPlan& p = o.plan;
     p.r = x.in_r; p.n = pushed;
@@ -642,10 +697,6 @@ static int step_channel(hbd_decoder* h, HostChan& x, unsigned pushed, ChanStep& 
     x.in_r = total - p.consumed;
     x.pushed = 0;
     x.last_n2 = p.n2; x.last_nf = 0;
-    if (p.n2 && x.fft_have < unsigned(fft_n)) {   // FFT frame assembly, Decoder.h:467-473 (mirror of K2's arithmetic)
-        x.fft_have += std::min(unsigned(fft_n) - x.fft_have, p.n2);
-        if (x.fft_have >= unsigned(fft_n)) { o.frame_done = true; x.fft_have = 0; }   // transformed and cleared in this call
-    }
     if (M1 > 1) {   // history re-zeroing when the reference's work buffers grow (Decimator.h:74-79)
         const size_t need = size_t(p.consumed) + size_t(T1) + size_t(M1);
         if (x.grown1 < need) { x.grown1 = need; o.zero_carry = true; }
@@ -673,6 +724,17 @@ static int step_channel(hbd_decoder* h, HostChan& x, unsigned pushed, ChanStep& 
     const size_t need = size_t(nf) + x.lp_ntaps;
     if (x.grown_lp < need) { x.grown_lp = need; o.zero_lphist = true; }   // FirFilter.h:141-147
     return HBD_OK;
+}
+
+// FFT frame assembly, Decoder.h:467-473 (mirror of K2's arithmetic): a frame fill `have` after n2 more decimated samples;
+// true when the call completes the frame (K4 transforms it and clears the fill in that call)
+static bool step_frame(unsigned& have, unsigned n2, unsigned fft_n)
+{
+    if (!n2 || have >= fft_n) return false;
+    have += std::min(fft_n - have, n2);
+    if (have < fft_n) return false;
+    have = 0;
+    return true;
 }
 
 // Keep the character / SSDV logs from filling up: look at what the completed calls have appended (their committed
@@ -732,7 +794,7 @@ int hbd_decoder::plan_call(CallPlan& cp)
     groups_idle = false;
     // uniform mode (whole-batch pushes only, one low-pass setting): channel 0 stands for all of them, O(1) per call
     const bool uni = ctr_uniform && lp_cfg_uniform;
-    if (!uni) { sync_ctrs(); h_plan.resize(n); }
+    if (!uni) { leave_uniform(); h_plan.resize(n); }
     const size_t stepped = uni ? 1 : n;
     auto pushed = [&](size_t c) { return in.p ? unsigned(in.n) : hc[c].pushed; };
     size_t max_total = 0;
@@ -745,12 +807,27 @@ int hbd_decoder::plan_call(CallPlan& cp)
         ChanStep st;
         int rc = step_channel(this, hc[c], pushed(c), st, new_taps);
         if (rc) return rc;   // channels below c have been stepped: their samples are gone (documented in the header)
-        if (uni) { ctr_stale = true; cp.uplan = st.plan; } else h_plan[c] = st.plan;
-        cp.any_work |= !(st.plan.flags & 1u); cp.need_k4 |= st.frame_done;
+        if (uni) { ctr_stale = true; cp.uplan = st.plan; } else { h_plan[c] = st.plan; cp.need_k4 |= step_frame(hc[c].fft_have, st.plan.n2, unsigned(fft_n)); }
+        cp.any_work |= !(st.plan.flags & 1u);
         cp.max_n1 = std::max(cp.max_n1, st.plan.n1); max_nf = std::max(max_nf, st.nf);
         rc = apply_step(st, c, uni ? n : 1, new_taps);
         if (rc) return rc;
     }
+    if (uni) {   // each frame level once; levels that complete their frames in the same call are all back at 0: merge them
+        unsigned done = 0;
+        for (unsigned& v : fft_lvl) done += step_frame(v, cp.uplan.n2, unsigned(fft_n)) ? 1u : 0u;
+        cp.need_k4 = done > 0;
+        plan_steps += unsigned(fft_lvl.size());
+        if (done > 1) {
+            std::vector<unsigned> to(fft_lvl.size()), merged;
+            for (size_t i = 0; i < fft_lvl.size(); ++i) {
+                to[i] = unsigned(std::find(merged.begin(), merged.end(), fft_lvl[i]) - merged.begin());
+                if (to[i] == merged.size()) merged.push_back(fft_lvl[i]);
+            }
+            for (unsigned& l : lvl_of) l = to[l];
+            fft_lvl.swap(merged);
+        }
+    } else plan_steps += unsigned(n);
     if (demod_acc_on) { const int rc = ensure_dacc(); if (rc) return rc; }
 
     if (cfg_dirty_any) {
@@ -774,8 +851,7 @@ int hbd_decoder::plan_call(CallPlan& cp)
     }
     if (!uni) {
         // back to uniform mode as soon as the channels agree again (e.g. after a round of per-channel pushes of one size)
-        ctr_uniform = true;
-        for (size_t c = 1; c < n && ctr_uniform; ++c) ctr_uniform = hc[c].same(hc[0]);
+        regroup();
         for (size_t c = 1; c < n && cp.plan_uniform; ++c) cp.plan_uniform = memcmp(&h_plan[c], &h_plan[0], sizeof(ChanPlan)) == 0;
         cp.uplan = h_plan[0];
         if (!cp.plan_uniform && (h_plan_uploaded.size() != n || memcmp(h_plan.data(), h_plan_uploaded.data(), n * sizeof(ChanPlan)) != 0)) {
@@ -904,7 +980,9 @@ int hbd_decoder::process_async_locked()
     HBD_CUDA_CHECK(cudaSetDevice(device));
     { const int rc = log_pressure(); if (rc) return rc; }
     CallPlan cp;
+    const auto t_plan0 = std::chrono::steady_clock::now();
     { const int rc = plan_call(cp); if (rc) return rc; }
+    plan_host_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_plan0).count();
     if (in.p && in.format != HBD_IQ_CF32 && !decim1_supports_native_iq(M1, T1)) {   // the plan changed after a native integer push
         size_t wp = 0;
         const int rc = widen(in.p, in.pitch, in.format, n_ch, in.n, &wp);
@@ -1175,6 +1253,53 @@ int hbd_decoder::enable_snap()
     return HBD_OK;
 }
 
+// hbd_reset_channels: the listed channels become channel 0 of a new handle with the same settings.  The drain comes first,
+// so that what the calls in flight decoded goes through the old text and SSDV state; then the host state restarts and one
+// kernel restarts the device state on the handle's stream (the next call's K1 waits for it through ev_in).
+int hbd_decoder::reset_channels(const int* chs, size_t k)
+{
+    std::vector<unsigned char> listed(size_t(n_ch), 0);
+    for (size_t i = 0; i < k; ++i) {
+        if (chs[i] < 0 || chs[i] >= n_ch || listed[size_t(chs[i])]) { set_error("reset_channels: channel out of range or listed twice"); return HBD_ERR_ARG; }
+        listed[size_t(chs[i])] = 1;
+    }
+    if (!k) return HBD_OK;
+    sync_ctrs();
+    bool staged = in.p != nullptr;
+    for (size_t c = 0; c < hc.size() && !staged; ++c) staged = hc[c].pushed != 0;
+    if (staged) { set_error("reset_channels: pushed samples have not been processed yet"); return HBD_ERR_STATE; }
+    HBD_CUDA_CHECK(cudaSetDevice(device));
+    { const int rc = collect_locked(0); if (rc) return rc; }   // also: the previous reset's list upload is complete
+    if (!h_reset) {   // both buffers are allocated together
+        HostPtr<int> hp; DevPtr<int> dp;
+        HBD_CUDA_CHECK(host_alloc(hp, size_t(n_ch)));
+        HBD_CUDA_CHECK(dev_alloc(dp, size_t(n_ch)));
+        h_reset = std::move(hp); d_reset = std::move(dp);
+    }
+    leave_uniform();
+    for (size_t i = 0; i < k; ++i) {
+        const size_t c = size_t(chs[i]);
+        HostChan& x = hc[c];
+        x.ctr() = ChanCtr();   // grown* == 0: the next call zeroes the carry and stage histories of this row (apply_step)
+        x.fft_have = 0; x.nco_phase = 0;
+        x.cfg_dirty = true;    // the configuration goes onto the fresh ChanState with the next call's upload, as on a new handle
+        text[c].restart();
+        if (c < ssdv.size()) ssdv[c].restart();
+        h_reset.get()[i] = chs[i];
+    }
+    cfg_dirty_any = derived_dirty = true;
+    regroup();   // resetting every channel keeps the handle uniform, on one frame level
+    HBD_CUDA_CHECK(cudaMemcpyAsync(d_reset.get(), h_reset.get(), k * sizeof(int), cudaMemcpyHostToDevice, stream));
+    ResetArgs a{};
+    a.state = d_state.get(); a.list = d_reset.get();
+    a.decq = decq.get(); a.dq_pitch = decq.pitch;
+    a.dacc_n = d_dacc_n.get(); a.ssdv_total = d_ssdv_total.get(); a.ssdv_scanned = d_ssdv_scanned.get(); a.rec_bits_n = d_rec_bits_n.get();
+    reset_chan_kernel<<<unsigned(k), 128, 0, stream>>>(a);
+    ++launches;
+    HBD_CUDA_CHECK(cudaGetLastError());
+    return HBD_OK;
+}
+
 namespace hbd {
 int internal_device(hbd_decoder* h) { return h->device; }
 void internal_set_error(hbd_decoder* h, const std::string& what) { std::lock_guard<std::mutex> l(h->mtx); h->set_error(what); }
@@ -1265,6 +1390,7 @@ int hbd_create(int n_channels, int cuda_device, hbd_decoder** out)
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, cuda_device) == cudaSuccess) h->n_sms = prop.multiProcessorCount;
     h->hc.resize(size_t(n_channels));
+    h->lvl_of.assign(size_t(n_channels), 0u);
     h->text.resize(size_t(n_channels));
     for (auto& tc : h->text) { tc.text_stream.reserve(120); tc.last_sentence.reserve(96); }   // no allocation on the drain path in steady state
     { hbd_result_record z; memset(&z, 0, sizeof(z)); h->pend.assign(size_t(n_channels), z); }
@@ -1334,8 +1460,9 @@ int hbd_set_fft_size(hbd_decoder* h, size_t n_bins)
     if (cudaMemcpy(h->d_state.get(), st.data(), st.size() * sizeof(ChanState), cudaMemcpyHostToDevice) != cudaSuccess) return HBD_ERR_CUDA;
     h->fft = std::move(f);
     h->fft_n = int(n_bins);
-    h->sync_ctrs();
     for (auto& x : h->hc) x.fft_have = 0;
+    h->fft_lvl.assign(1, 0u);
+    h->lvl_of.assign(h->hc.size(), 0u);
     return HBD_OK;
 }
 
@@ -1377,7 +1504,7 @@ static int set_lp(hbd_decoder* h, int ch, float bw, float trans, bool set_bw)
     }
     cudaSetDevice(h->device);
     h->sync_groups();
-    h->sync_ctrs();
+    h->leave_uniform();
     std::vector<float> taps;
     for (int c = (ch < 0 ? 0 : ch); c < (ch < 0 ? h->n_ch : ch + 1); ++c) {
         HostChan& x = h->hc[size_t(c)];
@@ -1391,12 +1518,10 @@ static int set_lp(hbd_decoder* h, int ch, float bw, float trans, bool set_bw)
             if (cudaMemcpy(h->d_lptaps.get() + size_t(c) * kLpMaxTaps, taps.data(), 4 * T, cudaMemcpyHostToDevice) != cudaSuccess) return HBD_ERR_CUDA;
         }
     }
-    bool cfg_same = true, ctr_same = true;
-    for (size_t c = 1; c < h->hc.size(); ++c) {
-        cfg_same = cfg_same && h->hc[c].lp_bw == h->hc[0].lp_bw && h->hc[c].lp_trans == h->hc[0].lp_trans;
-        ctr_same = ctr_same && h->hc[c].same(h->hc[0]);
-    }
-    h->lp_cfg_uniform = cfg_same; h->ctr_uniform = ctr_same;
+    bool cfg_same = true;
+    for (size_t c = 1; c < h->hc.size(); ++c) cfg_same = cfg_same && h->hc[c].lp_bw == h->hc[0].lp_bw && h->hc[c].lp_trans == h->hc[0].lp_trans;
+    h->lp_cfg_uniform = cfg_same;
+    h->regroup();
     return HBD_OK;
 }
 int hbd_set_lowpass_bw(hbd_decoder* h, int ch, float bw) { return set_lp(h, ch, bw, 0, true); }
@@ -1656,6 +1781,11 @@ int hbd_process(hbd_decoder* h)
         return h->collect_locked(0);
     });
 }
+int hbd_reset_channels(hbd_decoder* h, const int* channels, size_t n)
+{
+    if (!h || (n && !channels)) return HBD_ERR_ARG;
+    return locked_then_fire(h, [h, channels, n] { return h->reset_channels(channels, n); });
+}
 int hbd_synchronize(hbd_decoder* h)
 {
     HBD_CHECK_H(h);
@@ -1673,6 +1803,7 @@ int hbd_set_kernel_timing(hbd_decoder* h, int on)
     h->timing = on < 0 ? 0 : on;
     h->ev_used_k1 = h->ev_used_rest = 0;
     h->drain_host_ms = 0; h->drain_calls = 0;
+    h->plan_host_ms = 0; h->plan_steps = 0;
     if (on) {   // events are created here, not on the issue path of the calls being measured
         cudaSetDevice(h->device);
         for (auto* pool : {&h->ev_k1, &h->ev_rest})
@@ -1691,6 +1822,11 @@ int hbd_get_kernel_timing(hbd_decoder* h, int which, double* total_ms, unsigned*
     if (which == 5) {   // host time spent replaying drained calls through the sentence layer (wall clock of the caller's thread)
         if (total_ms) *total_ms = h->drain_host_ms;
         if (count) *count = h->drain_calls;
+        return HBD_OK;
+    }
+    if (which == 6) {   // host time of the calls' planning (plan_call), and the frame counters it stepped
+        if (total_ms) *total_ms = h->plan_host_ms;
+        if (count) *count = h->plan_steps;
         return HBD_OK;
     }
     if (which >= 2) {   // pipeline diagnostics (one channel group): signed gaps between events of different pairs

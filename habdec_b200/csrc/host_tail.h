@@ -42,6 +42,9 @@ struct TextChannel {
     bool scan_clean = true;         // text_stream is known to hold no extractable sentence (see feed)
     bool latent = false;            // ... except one that only waits for a '*' to appear in the stream (see feed)
     void feed(const unsigned char* raw, size_t n, int ch, const SentenceSink& sink, bool keep_raw, hbd_result_record& pend);
+    // the text state of a new Decoder (hbd_reset_channels); what waits to be polled (the pending record, the spills,
+    // raw_pending) is output, not state, and stays
+    void restart() { text_stream.clear(); last_sentence.clear(); scan_clean = true; latent = false; }
     // pull the end of the string feed() appends to into the cache (the drain loop knows its next channels)
     void prefetch_tails() const { __builtin_prefetch(text_stream.data() + text_stream.size()); }
 
@@ -106,6 +109,8 @@ struct SsdvChannel {
 
     // one SSDV_wraper_t::push(); true (and `ev` filled) when a packet was filed
     bool push(const unsigned char* chars, size_t n, SsdvEvent& ev);
+    // a new SSDV_wraper_t (hbd_reset_channels); packets not polled yet (events_pending) stay
+    void restart() { buff.clear(); packet_begin = -1; stream_end = 0; verdicts.clear(); packets.clear(); last_key = ImageKey("", 0); }
     size_t image(const std::string& callsign, int image_id, unsigned char* out, size_t cap) const;
 };
 

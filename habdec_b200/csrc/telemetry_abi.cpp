@@ -139,6 +139,12 @@ int hbd_tracker_push_sentence(hbd_tracker* t, int ch, const char* sentence)
     return tracker_feed(t, ch, s.substr(0, comma), s.substr(comma + 1, star - comma - 1), s.substr(star + 1));
 }
 
+int hbd_tracker_reset(hbd_tracker* t, int ch)
+{
+    if (!t) return HBD_ERR_ARG;
+    std::lock_guard<std::mutex> l(t->mtx); t->chans.erase(ch); return HBD_OK;
+}
+
 size_t hbd_tracker_poll(hbd_tracker* t, int ch, hbd_telemetry* out, size_t cap)
 {
     if (!t) return 0;

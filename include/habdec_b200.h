@@ -139,12 +139,26 @@ int hbd_process_async(hbd_decoder* h);  /* kernels only, returns immediately */
 int hbd_collect(hbd_decoder* h);        /* drain results of all async calls so far (sentence layer + callbacks) */
 /* like hbd_collect but leaves the newest `lag` calls in flight: the GPU keeps running while the host drains */
 int hbd_collect_ready(hbd_decoder* h, unsigned lag);
+/* Return channels to the state of channel 0 of a newly created handle with the same settings, e.g. to hand a channel of
+ * a wideband receiver to a new payload (a new Decoder<float> in the reference).  Kept: the decimation plan, sampling
+ * rate, FFT size, the handle-wide switches, and each channel's baud, framing, low-pass, dc_remove and NCO frequency.
+ * Restarted: every filter history, the low-pass design, the spectrum and AFC, the slicer and UART, the demod
+ * accumulation, SSDV and bit recording, the NCO phase (to 0), the text stream and last sentence, the SSDV image map.
+ * Output not yet polled or gathered (characters, sentences, raw characters, SSDV packets) stays queued.
+ * Every call in flight is drained first (callbacks fire before this returns, with the old text state); the reset itself
+ * is one kernel on the handle's stream, ordered before the next call.  Out-of-range or duplicate channels: HBD_ERR_ARG;
+ * samples pushed but not yet processed (in any channel): HBD_ERR_STATE; nothing is changed in either case.  n == 0: no-op.
+ * The first call after a reset plans every channel on its own; from the second one on, batch and wideband pushes whose
+ * size is a multiple of the factor are planned in O(1) of the channel count again (see hbd_get_kernel_timing, which 6). */
+int hbd_reset_channels(hbd_decoder* h, const int* channels, size_t n);
 int hbd_synchronize(hbd_decoder* h);
 /* number of CUDA kernels this handle has launched so far */
 unsigned long long hbd_kernel_launches(hbd_decoder* h);
 /* measurement hook: on = 1 records CUDA events around every K1 (stage-1 decimator) launch, on = 2 also around the rest of
  * the step (two more event records per call on the low-priority stream); `which` 0 = K1, 1 = rest; 2..4 = signed pipeline gaps (K1 end -> next K1 start, K1 end -> own tail start,
- * tail end -> K1 start two calls later); 5 = host time of the drains' sentence-layer replay (count = calls drained).
+ * tail end -> K1 start two calls later); 5 = host time of the drains' sentence-layer replay (count = calls drained);
+ * 6 = host time of the calls' planning (count = frame counters stepped: one per FFT frame level in a call planned for all
+ * channels at once, one per channel otherwise).
  * Calling set (on or off) clears the accumulated samples. */
 int hbd_set_kernel_timing(hbd_decoder* h, int on);
 int hbd_get_kernel_timing(hbd_decoder* h, int which, double* total_ms, unsigned* count);
@@ -327,6 +341,9 @@ int    hbd_tracker_set_callback(hbd_tracker* t, hbd_telemetry_cb cb, void* user)
 int    hbd_tracker_push(hbd_tracker* t, int ch, const char* callsign, const char* data, const char* crc);
 int    hbd_tracker_push_sentence(hbd_tracker* t, int ch, const char* sentence);    /* "callsign,data*crc" as polled */
 size_t hbd_tracker_poll(hbd_tracker* t, int ch, hbd_telemetry* out, size_t cap);   /* records since the previous poll */
+/* channel `ch` as if no sentence had reached it: stats, sentences_map_ and unpolled records are dropped.  Pairs with
+ * hbd_reset_channels when a channel is handed to a new payload (hbd_reset_channels leaves an attached tracker alone). */
+int    hbd_tracker_reset(hbd_tracker* t, int ch);
 int    hbd_tracker_stats(hbd_tracker* t, int ch, hbd_channel_stats* out);
 /* "cmd::info:stats=ok:..,dist_line:..,...,alt:..[,age:..]" (habdec_ws_protocol.cpp:486-498) */
 size_t hbd_tracker_stats_payload(hbd_tracker* t, int ch, int with_age, char* out, size_t cap);

@@ -119,6 +119,9 @@ public:
     int processAsync() { return status_ = hbd_process_async(h_); }
     int collect() { return status_ = hbd_collect(h_); }
     int collectReady(unsigned lag) { return status_ = hbd_collect_ready(h_, lag); }
+    // channels start over like a new Decoder<float> with the same settings (hbd_reset_channels); unpolled output stays queued
+    int resetChannels(const std::vector<int>& chs) { return status_ = hbd_reset_channels(h_, chs.data(), chs.size()); }
+    int resetChannel(int ch) { return resetChannels({ch}); }
     int lastStatus() const { return status_; }
     std::string lastError() const { return hbd_last_error(h_); }
 
