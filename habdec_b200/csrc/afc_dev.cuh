@@ -67,4 +67,16 @@ __device__ __forceinline__ void afc_store(ChanState& dst, const ChanState& src)
     dst.gui_left = src.gui_left; dst.gui_right = src.gui_right;
 }
 
+// AFC::resetFrequencyCorrection (AFC.h:188-194): the peak averages move by `corr` Hz and restart, the correction is 0 again
+__device__ __forceinline__ void afc_reset(ChanState& st, double corr, double fs_dec, int n_fft)
+{
+    // the reference divides fft_samples_.size() by its sampling rate: both are 0 before the first spectrum
+    const double bins_per_hz = st.have_spectrum ? __ddiv_rn(double(n_fft), fs_dec) : __ddiv_rn(0.0, 0.0);
+    const double l = __dsub_rn(avg_get_i(st.pl_sum, st.pl_cnt), __dmul_rn(corr, bins_per_hz));
+    const double r = __dsub_rn(avg_get_i(st.pr_sum, st.pr_cnt), __dmul_rn(corr, bins_per_hz));
+    st.pl_sum = int(fmax(0.0, l)); st.pl_cnt = 1;
+    st.pr_sum = int(fmax(0.0, r)); st.pr_cnt = 1;
+    st.afc_correction = 0;
+}
+
 } // namespace hbd

@@ -165,15 +165,21 @@ __global__ void reset_chan_kernel(ResetArgs a)
     if (a.rec_bits_n) a.rec_bits_n[ch] = 0;
 }
 
+// a channel's AFC scalars in the order of hbd_get_stats_batch and hbd_result_record: correction, shift, noise floor,
+// noise variance, peak left, peak right
+template <class T>
+__host__ __device__ inline void afc_scalars(const ChanState& s, T out[6])
+{
+    out[0] = T(s.afc_correction); out[1] = T(s.afc_shift_hz); out[2] = T(s.afc_noise_floor); out[3] = T(s.afc_noise_var);
+    out[4] = T(s.gui_left); out[5] = T(s.gui_right);
+}
+
 // the per-channel scalars that travel with the gathered results (hbd_result_record), packed after every call
 __global__ void stats_snap_kernel(const ChanState* __restrict__ st, float* __restrict__ out, int n_ch)
 {
     const int ch = blockIdx.x * blockDim.x + threadIdx.x;
     if (ch >= n_ch) return;
-    const ChanState& s = st[ch];
-    float* o = out + size_t(ch) * 6;
-    o[0] = float(s.afc_correction); o[1] = float(s.afc_shift_hz); o[2] = float(s.afc_noise_floor); o[3] = float(s.afc_noise_var);
-    o[4] = float(s.gui_left); o[5] = float(s.gui_right);
+    afc_scalars(st[ch], out + size_t(ch) * 6);
 }
 
 } // namespace
@@ -226,11 +232,24 @@ struct hbd_decoder {
         if (lo && cudaStreamSynchronize(lo.get()) != cudaSuccess) return HBD_ERR_CUDA;
         return HBD_OK;
     }
+    // wait until everything the handle has enqueued is done: the compute streams, then the caller's stream
+    int settle()
+    {
+        HBD_CUDA_CHECK(cudaSetDevice(device));
+        if (sync_groups()) { set_error("stream sync failed"); return HBD_ERR_CUDA; }
+        HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
+        return HBD_OK;
+    }
+    // the device state of channels [c0, c0 + n) once everything enqueued is done
+    int read_states(size_t c0, size_t n, ChanState* out)
+    {
+        if (settle()) return HBD_ERR_CUDA;
+        HBD_CUDA_CHECK(cudaMemcpy(out, d_state.get() + c0, n * sizeof(ChanState), cudaMemcpyDeviceToHost));
+        return HBD_OK;
+    }
     ~hbd_decoder()
     {
-        cudaSetDevice(device);
-        sync_groups();
-        if (stream) cudaStreamSynchronize(stream);
+        settle();
         dist_ctx.reset();
     }
     // plan_call: wait for the compute streams once, before the first host-side change a kernel in flight could see
@@ -559,9 +578,7 @@ int hbd_decoder::make_fft(int N_, FftBufs& f)
 // Taps and carry of the new plan go into locals first: on failure the previous plan stays in force.
 int hbd_decoder::set_plan(const std::vector<TapTable>& st, size_t total_factor)
 {
-    HBD_CUDA_CHECK(cudaSetDevice(device));
-    if (sync_groups()) return HBD_ERR_CUDA;
-    HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
+    if (settle()) return HBD_ERR_CUDA;
     const size_t n = size_t(n_ch);
     sync_ctrs();
     const TapTable none{1, nullptr, 1};   // M == 1: no such stage (a plan without one keeps the tap buffer it has)
@@ -994,16 +1011,26 @@ int hbd_decoder::process_async_locked()
     return HBD_OK;
 }
 
+// entries [tail, tail + n) of a device ring of `cap` entries (a power of two) into dst: one copy, or two where the range
+// wraps, then a synchronise of `s` (none for n == 0)
+template <class T>
+static cudaError_t read_ring(std::vector<T>& dst, const T* ring, unsigned cap, unsigned tail, unsigned n, cudaStream_t s)
+{
+    dst.resize(n);
+    if (!n) return cudaSuccess;
+    const unsigned i0 = tail & (cap - 1u), first = std::min(n, cap - i0);
+    cudaError_t e = cudaMemcpyAsync(dst.data(), ring + i0, size_t(first) * sizeof(T), cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess && n > first) e = cudaMemcpyAsync(dst.data() + first, ring, size_t(n - first) * sizeof(T), cudaMemcpyDeviceToHost, s);
+    return e == cudaSuccess ? cudaStreamSynchronize(s) : e;
+}
+
 // Drain decoded characters of all calls up to (last enqueued - lag) and run the sentence layer on them, call by
 // call like Decoder::process().  lag == 0 waits for everything; lag > 0 leaves the newest calls in flight so the GPU
 // keeps working while the host is busy here.  User callbacks are only RECORDED here (h->deferred).
 int hbd_decoder::collect_locked(unsigned lag)
 {
     HBD_CUDA_CHECK(cudaSetDevice(device));
-    if (call_seq == calls_collected) {
-        if (lag == 0) { if (sync_groups()) return HBD_ERR_CUDA; HBD_CUDA_CHECK(cudaStreamSynchronize(stream)); }
-        return HBD_OK;
-    }
+    if (call_seq == calls_collected) return lag == 0 ? settle() : HBD_OK;
     if (call_seq - calls_collected <= lag) return HBD_OK;
     if (lag == 0 && call_seq - calls_collected > 2) {
         // a full drain behind a queue of calls: take the finished calls first, in halving steps, so the host's sentence
@@ -1015,8 +1042,7 @@ int hbd_decoder::collect_locked(unsigned lag)
     }
     const unsigned upto = call_seq - lag;            // calls [calls_collected, upto) get drained
     if (lag == 0) {
-        if (sync_groups()) { set_error("stream sync failed"); return HBD_ERR_CUDA; }
-        HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
+        if (settle()) return HBD_ERR_CUDA;
     } else {
         HBD_CUDA_CHECK(cudaEventSynchronize(ev_call[(upto - 1) % ev_call.size()].get()));
     }
@@ -1039,18 +1065,9 @@ int hbd_decoder::collect_locked(unsigned lag)
             ovf_seen[1] = heads[kCtlSsdvOvf];
             result = HBD_ERR_STATE;
         }
-        const unsigned avail_p = std::min(heads[kCtlSsdvHead] - ssdv_log_tail, kSsdvLogCap);
-        h_ssdv_log.resize(avail_p);
-        if (avail_p) {
-            const unsigned i0 = ssdv_log_tail & (kSsdvLogCap - 1u);
-            const unsigned first = std::min(avail_p, kSsdvLogCap - i0);
-            HBD_CUDA_CHECK(cudaMemcpyAsync(h_ssdv_log.data(), d_ssdv_log.get() + i0, size_t(first) * sizeof(SsdvLogEntry), cudaMemcpyDeviceToHost, copy_stream.get()));
-            if (avail_p > first)
-                HBD_CUDA_CHECK(cudaMemcpyAsync(h_ssdv_log.data() + first, d_ssdv_log.get(), size_t(avail_p - first) * sizeof(SsdvLogEntry), cudaMemcpyDeviceToHost, copy_stream.get()));
-            HBD_CUDA_CHECK(cudaStreamSynchronize(copy_stream.get()));
-        }
-        for (unsigned k = 0; k < avail_p; ++k) {
-            const SsdvLogEntry& e = h_ssdv_log[k];
+        HBD_CUDA_CHECK(read_ring(h_ssdv_log, d_ssdv_log.get(), kSsdvLogCap, ssdv_log_tail, std::min(heads[kCtlSsdvHead] - ssdv_log_tail, kSsdvLogCap),
+                                 copy_stream.get()));
+        for (const SsdvLogEntry& e : h_ssdv_log) {
             if (e.ch >= unsigned(n_ch)) continue;
             SsdvVerdict v; v.pos = e.pos; v.errors = e.errors; memcpy(v.data.data(), e.data, 256);
             ssdv[e.ch].verdicts.push_back(v);
@@ -1072,16 +1089,7 @@ int hbd_decoder::collect_locked(unsigned lag)
                                        cudaMemcpyDeviceToHost, copy_stream.get()));
         h_snap_valid = true;
     }
-    const unsigned avail = head - log_tail;
-    h_log.resize(avail);
-    if (avail) {
-        const unsigned i0 = log_tail & (log_cap - 1u);
-        const unsigned first = std::min(avail, log_cap - i0);
-        HBD_CUDA_CHECK(cudaMemcpyAsync(h_log.data(), d_log.get() + i0, size_t(first) * sizeof(uint2), cudaMemcpyDeviceToHost, copy_stream.get()));
-        if (avail > first)
-            HBD_CUDA_CHECK(cudaMemcpyAsync(h_log.data() + first, d_log.get(), size_t(avail - first) * sizeof(uint2), cudaMemcpyDeviceToHost, copy_stream.get()));
-        HBD_CUDA_CHECK(cudaStreamSynchronize(copy_stream.get()));
-    }
+    HBD_CUDA_CHECK(read_ring(h_log, d_log.get(), log_cap, log_tail, head - log_tail, copy_stream.get()));
     // the writers may reuse everything below the new tail
     log_tail = head;
     h_tail_pin.get()[0] = log_tail; h_tail_pin.get()[1] = ssdv_log_tail;
@@ -1321,16 +1329,10 @@ size_t hbd_pack_results(hbd_decoder* h, int ch_offset, hbd_result_record* out, s
     const float* st = h->h_snap.get();
     if (!(h->snap_on && h->h_snap_valid)) {   // read the live state (waits for the calls in flight)
         if (h->enable_snap() != HBD_OK) return 0;
-        cudaSetDevice(h->device);
-        h->sync_groups();
-        cudaStreamSynchronize(h->stream);
         std::vector<ChanState> cs(n);
-        if (cudaMemcpy(cs.data(), h->d_state.get(), n * sizeof(ChanState), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
+        if (h->read_states(0, n, cs.data())) return 0;
         live.resize(6 * n);
-        for (size_t c = 0; c < n; ++c) {
-            live[6 * c + 0] = float(cs[c].afc_correction); live[6 * c + 1] = float(cs[c].afc_shift_hz); live[6 * c + 2] = float(cs[c].afc_noise_floor);
-            live[6 * c + 3] = float(cs[c].afc_noise_var); live[6 * c + 4] = float(cs[c].gui_left); live[6 * c + 5] = float(cs[c].gui_right);
-        }
+        for (size_t c = 0; c < n; ++c) afc_scalars(cs[c], live.data() + 6 * c);
         st = live.data();
     }
     // the pending slots ARE the records: copy, stamp, reset (and move spilled bytes up).  Cut by channel range like the
@@ -1428,9 +1430,7 @@ int hbd_set_stream(hbd_decoder* h, void* s)
 {
     HBD_CHECK_H(h);
     std::lock_guard<std::mutex> l(h->mtx);
-    cudaSetDevice(h->device);
-    h->sync_groups();
-    cudaStreamSynchronize(h->stream);
+    if (h->settle()) return HBD_ERR_CUDA;
     h->own_stream.reset();
     h->stream = (cudaStream_t)s;
     return HBD_OK;
@@ -1442,15 +1442,14 @@ int hbd_set_fft_size(hbd_decoder* h, size_t n_bins)
     HBD_CHECK_H(h);
     if (n_bins != size_t(kFftN) && n_bins != size_t(kFftNMax)) return HBD_ERR_ARG;
     std::lock_guard<std::mutex> l(h->mtx);
-    cudaSetDevice(h->device);
-    if (h->sync_groups() || cudaStreamSynchronize(h->stream) != cudaSuccess) return HBD_ERR_CUDA;
+    if (h->settle()) return HBD_ERR_CUDA;
     if (int(n_bins) == h->fft_n) return HBD_OK;
     hbd_decoder::FftBufs f;   // swapped in after the state reset below: on failure the old size and spectra stay
     const int rc = h->make_fft(int(n_bins), f);
     if (rc) return rc;
     // spectrum / AFC state back to a freshly constructed decoder's (Average<T> starts with one 0 sample)
     std::vector<ChanState> st(size_t(h->n_ch));
-    if (cudaMemcpy(st.data(), h->d_state.get(), st.size() * sizeof(ChanState), cudaMemcpyDeviceToHost) != cudaSuccess) return HBD_ERR_CUDA;
+    if (h->read_states(0, st.size(), st.data())) return HBD_ERR_CUDA;
     for (auto& s : st) {
         s.fft_have = s.fft_ready = s.have_spectrum = 0;
         s.afc_correction = s.afc_noise_floor = s.afc_noise_var = s.afc_shift_hz = 0;
@@ -1790,9 +1789,7 @@ int hbd_synchronize(hbd_decoder* h)
 {
     HBD_CHECK_H(h);
     std::lock_guard<std::mutex> l(h->mtx);
-    cudaSetDevice(h->device);
-    if (h->sync_groups()) return HBD_ERR_CUDA;
-    return cudaStreamSynchronize(h->stream) == cudaSuccess ? HBD_OK : HBD_ERR_CUDA;
+    return h->settle();
 }
 unsigned long long hbd_kernel_launches(hbd_decoder* h) { return h ? h->launches : 0; }
 
@@ -1816,8 +1813,7 @@ int hbd_get_kernel_timing(hbd_decoder* h, int which, double* total_ms, unsigned*
 {
     HBD_CHECK_H(h);
     std::lock_guard<std::mutex> l(h->mtx);
-    cudaSetDevice(h->device);
-    if (h->sync_groups() || cudaStreamSynchronize(h->stream) != cudaSuccess) return HBD_ERR_CUDA;
+    if (h->settle()) return HBD_ERR_CUDA;
     double tot = 0; unsigned cnt = 0;
     if (which == 5) {   // host time spent replaying drained calls through the sentence layer (wall clock of the caller's thread)
         if (total_ms) *total_ms = h->drain_host_ms;
@@ -2032,20 +2028,10 @@ double hbd_get_symbol_rate(hbd_decoder* h, int ch) { return hbd_get_baud(h, ch);
 int hbd_n_channels(hbd_decoder* h) { return h ? h->n_ch : 0; }
 size_t hbd_get_bins_count(hbd_decoder* h) { if (!h) return size_t(kFftN); std::lock_guard<std::mutex> l(h->mtx); return size_t(h->fft_n); }
 
-static int fetch_state(hbd_decoder* h, int ch, ChanState* st)
+// min(n, cap) floats from the device into out (the caller has settled the handle); returns n, or 0 when the copy fails
+static size_t fetch_floats(const void* dsrc, size_t n, float* out, size_t cap)
 {
-    cudaSetDevice(h->device);
-    if (h->sync_groups() || cudaStreamSynchronize(h->stream) != cudaSuccess) return HBD_ERR_CUDA;
-    return cudaMemcpy(st, h->d_state.get() + ch, sizeof(ChanState), cudaMemcpyDeviceToHost) == cudaSuccess ? HBD_OK : HBD_ERR_CUDA;
-}
-static size_t fetch_floats(hbd_decoder* h, const void* dsrc, size_t n, float* out, size_t cap)
-{
-    if (out && cap && n) {
-        cudaSetDevice(h->device);
-        h->sync_groups();
-        cudaStreamSynchronize(h->stream);
-        if (cudaMemcpy(out, dsrc, std::min(n, cap) * sizeof(float), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
-    }
+    if (out && cap && n && cudaMemcpy(out, dsrc, std::min(n, cap) * sizeof(float), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
     return n;
 }
 
@@ -2053,17 +2039,17 @@ size_t hbd_get_fft(hbd_decoder* h, int ch, float* out, size_t cap)
 {
     if (!h || ch < 0 || ch >= h->n_ch) return 0;
     std::lock_guard<std::mutex> l(h->mtx);
-    ChanState st; if (fetch_state(h, ch, &st)) return 0;
-    if (!st.have_spectrum) return 0; // freq_out_ is empty before the first FFT
-    return fetch_floats(h, h->fft.spectrum.get() + size_t(ch) * size_t(h->fft_n), 2 * size_t(h->fft_n), out, cap);
+    ChanState st;
+    if (h->read_states(size_t(ch), 1, &st) || !st.have_spectrum) return 0; // freq_out_ is empty before the first FFT
+    return fetch_floats(h->fft.spectrum.get() + size_t(ch) * size_t(h->fft_n), 2 * size_t(h->fft_n), out, cap);
 }
 size_t hbd_get_power_spectrum(hbd_decoder* h, int ch, float* out, size_t cap)
 {
     if (!h || ch < 0 || ch >= h->n_ch) return 0;
     std::lock_guard<std::mutex> l(h->mtx);
-    ChanState st; if (fetch_state(h, ch, &st)) return 0;
-    if (!st.have_spectrum) return 0;
-    return fetch_floats(h, h->fft.power.get() + size_t(ch) * size_t(h->fft_n), size_t(h->fft_n), out, cap);
+    ChanState st;
+    if (h->read_states(size_t(ch), 1, &st) || !st.have_spectrum) return 0;
+    return fetch_floats(h->fft.power.get() + size_t(ch) * size_t(h->fft_n), size_t(h->fft_n), out, cap);
 }
 size_t hbd_get_demodulated(hbd_decoder* h, int ch, float* out, size_t cap)
 {
@@ -2071,40 +2057,39 @@ size_t hbd_get_demodulated(hbd_decoder* h, int ch, float* out, size_t cap)
     std::lock_guard<std::mutex> l(h->mtx);
     h->sync_ctrs();
     const size_t n = h->hc[size_t(ch)].demod_n;   // a call that demodulates nothing leaves the previous block in place
-    if (!h->demod.get()) return 0;
-    return fetch_floats(h, h->demod.get() + size_t(ch) * h->demod.pitch, n, out, cap);
+    if (!h->demod.get() || h->settle()) return 0;
+    return fetch_floats(h->demod.get() + size_t(ch) * h->demod.pitch, n, out, cap);
 }
 int hbd_get_peaks(hbd_decoder* h, int ch, int* pl, int* pr)
 {
     HBD_CHECK_CH(h, ch); std::lock_guard<std::mutex> l(h->mtx);
-    ChanState st; const int rc = fetch_state(h, ch, &st); if (rc) return rc;
+    ChanState st; const int rc = h->read_states(size_t(ch), 1, &st); if (rc) return rc;
     if (pl) *pl = st.gui_left; if (pr) *pr = st.gui_right; return HBD_OK;
 }
 int hbd_get_noise_floor(hbd_decoder* h, int ch, double* nf, double* nv)
 {
     HBD_CHECK_CH(h, ch); std::lock_guard<std::mutex> l(h->mtx);
-    ChanState st; const int rc = fetch_state(h, ch, &st); if (rc) return rc;
+    ChanState st; const int rc = h->read_states(size_t(ch), 1, &st); if (rc) return rc;
     if (nf) *nf = st.afc_noise_floor; if (nv) *nv = st.afc_noise_var; return HBD_OK;
 }
 double hbd_get_shift(hbd_decoder* h, int ch)
 {
     if (!h || ch < 0 || ch >= h->n_ch) return 0; std::lock_guard<std::mutex> l(h->mtx);
-    ChanState st; if (fetch_state(h, ch, &st)) return 0; return st.afc_shift_hz;
+    ChanState st; if (h->read_states(size_t(ch), 1, &st)) return 0; return st.afc_shift_hz;
 }
 double hbd_get_frequency_correction(hbd_decoder* h, int ch)
 {
     if (!h || ch < 0 || ch >= h->n_ch) return 0; std::lock_guard<std::mutex> l(h->mtx);
-    ChanState st; if (fetch_state(h, ch, &st)) return 0; return st.afc_correction;
+    ChanState st; if (h->read_states(size_t(ch), 1, &st)) return 0; return st.afc_correction;
 }
 int hbd_reset_frequency_correction(hbd_decoder* h, int ch, double corr)
 {
     HBD_CHECK_CH(h, ch); std::lock_guard<std::mutex> l(h->mtx);
     cudaSetDevice(h->device);
-    h->sync_groups(); // ordered after everything in flight, like a call between two process() calls
-    if (launch_afc_reset(h->d_state.get(), ch, corr, h->fs_in / h->factor, h->fft_n, h->stream) != cudaSuccess) return HBD_ERR_CUDA;
-    cudaStreamSynchronize(h->stream);
+    // ordered after everything in flight, like a call between two process() calls
+    if (h->sync_groups() || launch_afc_reset(h->d_state.get(), ch, corr, h->fs_in / h->factor, h->fft_n, h->stream) != cudaSuccess) return HBD_ERR_CUDA;
     ++h->launches;
-    return HBD_OK;
+    return cudaStreamSynchronize(h->stream) == cudaSuccess ? HBD_OK : HBD_ERR_CUDA;
 }
 // ---- websocket wire formats ---------------------------------------------------------------------------------
 int hbd_decoder::ensure_frames(size_t pitch)
@@ -2145,8 +2130,7 @@ static size_t fetch_frames(hbd_decoder* h, int ch0, int nc, bool spectrum, float
 {
     if (type_size != 1 && type_size != 2 && type_size != 4) return 0;
     if (resolution < 0) resolution = 0;
-    cudaSetDevice(h->device);
-    if (h->sync_groups() || cudaStreamSynchronize(h->stream) != cudaSuccess) return 0;
+    if (h->settle()) return 0;
     const size_t hdr = spectrum ? size_t(kSpectrumHeaderBytes) : size_t(kDemodHeaderBytes);
     const size_t max_n = spectrum ? size_t(h->fft_n) : std::max<size_t>(h->dacc.pitch, 1);
     const size_t need = hdr + std::min<size_t>(max_n, size_t(resolution)) * size_t(type_size);
@@ -2214,13 +2198,14 @@ int hbd_afc_retune(hbd_decoder* h, double min_abs_hz, double* applied_out)
     cudaSetDevice(h->device);
     if (h->sync_groups()) return HBD_ERR_CUDA;
     const size_t n = size_t(h->n_ch);
-    DevPtr<double> applied_d;
-    if (dev_alloc(applied_d, n) != cudaSuccess) return HBD_ERR_NOMEM;
-    double* d_applied = applied_d.get();
+    DevPtr<double> d_applied;
     std::vector<double> applied(n, 0.0);
-    cudaError_t e = launch_afc_retune(h->d_state.get(), h->n_ch, min_abs_hz, h->fs_in / h->factor, d_applied, h->fft_n, h->stream);
-    ++h->launches;
-    if (e == cudaSuccess) e = cudaMemcpyAsync(applied.data(), d_applied, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
+    cudaError_t e = dev_alloc(d_applied, n);
+    if (e == cudaSuccess) {
+        e = launch_afc_retune(h->d_state.get(), h->n_ch, min_abs_hz, h->fs_in / h->factor, d_applied.get(), h->fft_n, h->stream);
+        ++h->launches;
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(applied.data(), d_applied.get(), n * sizeof(double), cudaMemcpyDeviceToHost, h->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
     if (e != cudaSuccess) { h->set_error(cudaGetErrorString(e)); return HBD_ERR_CUDA; }
     int count = 0;
@@ -2237,37 +2222,31 @@ size_t hbd_get_stats_batch(hbd_decoder* h, double* out, size_t cap_doubles)
     std::lock_guard<std::mutex> l(h->mtx);
     const size_t n = size_t(h->n_ch);
     if (!out || cap_doubles < 6 * n) return 6 * n;
-    cudaSetDevice(h->device);
-    h->sync_groups();
-    cudaStreamSynchronize(h->stream);
     std::vector<ChanState> st(n);
-    if (cudaMemcpy(st.data(), h->d_state.get(), n * sizeof(ChanState), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
-    for (size_t c = 0; c < n; ++c) {
-        out[6 * c + 0] = st[c].afc_correction; out[6 * c + 1] = st[c].afc_shift_hz;
-        out[6 * c + 2] = st[c].afc_noise_floor; out[6 * c + 3] = st[c].afc_noise_var;
-        out[6 * c + 4] = st[c].gui_left; out[6 * c + 5] = st[c].gui_right;
-    }
+    if (h->read_states(0, n, st.data())) return 0;
+    for (size_t c = 0; c < n; ++c) afc_scalars(st[c], out + 6 * c);
     return 6 * n;
 }
 
+// one query under one lock: the spectrum and the scalars come from the same completed call
 size_t hbd_get_spectrum_info(hbd_decoder* h, int ch, hbd_spectrum_info* info, float* power, size_t cap)
 {
     if (!h || ch < 0 || ch >= h->n_ch || !info) return 0;
-    std::vector<float> p(size_t(h->fft_n));
-    const size_t n = hbd_get_power_spectrum(h, ch, p.data(), p.size());
     memset(info, 0, sizeof(*info));
-    if (!n) return 0; // Decoder.h:818-819
+    std::lock_guard<std::mutex> l(h->mtx);
+    ChanState st;
+    if (h->read_states(size_t(ch), 1, &st) || !st.have_spectrum) return 0; // Decoder.h:818-819
+    std::vector<float> p(size_t(h->fft_n));
+    if (!fetch_floats(h->fft.power.get() + size_t(ch) * p.size(), p.size(), p.data(), p.size())) return 0;
     info->min_ = *std::min_element(p.begin(), p.end());
     info->max_ = *std::max_element(p.begin(), p.end());
-    int pl = 0, pr = 0;
-    hbd_get_peaks(h, ch, &pl, &pr);
-    info->peak_left_ = std::abs(pl); info->peak_left_valid_ = pl > 0;
-    info->peak_right_ = std::abs(pr); info->peak_right_valid_ = pr > 0;
-    hbd_get_noise_floor(h, ch, &info->noise_floor_, &info->noise_variance_);
-    info->sampling_rate_ = hbd_get_decimated_sampling_rate(h);
-    info->shift_ = hbd_get_shift(h, ch);
-    if (power && cap) memcpy(power, p.data(), std::min(cap, n) * sizeof(float));
-    return n;
+    info->peak_left_ = std::abs(st.gui_left); info->peak_left_valid_ = st.gui_left > 0;
+    info->peak_right_ = std::abs(st.gui_right); info->peak_right_valid_ = st.gui_right > 0;
+    info->noise_floor_ = st.afc_noise_floor; info->noise_variance_ = st.afc_noise_var;
+    info->sampling_rate_ = h->fs_in / h->factor;
+    info->shift_ = st.afc_shift_hz;
+    if (power && cap) memcpy(power, p.data(), std::min(cap, p.size()) * sizeof(float));
+    return p.size();
 }
 
 size_t hbd_debug_stage(hbd_decoder* h, int ch, int stage, float* out, size_t cap)
@@ -2278,30 +2257,30 @@ size_t hbd_debug_stage(hbd_decoder* h, int ch, int stage, float* out, size_t cap
     const HostChan& x = h->hc[size_t(ch)];
     switch (stage) {
     case HBD_STAGE_DECIMATED:
-        if (!h->rec.get(0)) return 0;
-        return fetch_floats(h, h->rec.get(0) + size_t(ch) * h->rec.pitch, 2 * size_t(x.last_n2), out, cap);
+        if (!h->rec.get(0) || h->settle()) return 0;
+        return fetch_floats(h->rec.get(0) + size_t(ch) * h->rec.pitch, 2 * size_t(x.last_n2), out, cap);
     case HBD_STAGE_FILTERED:
-        if (!h->rec.get(1)) return 0;
-        return fetch_floats(h, h->rec.get(1) + size_t(ch) * h->rec.pitch, 2 * size_t(x.last_nf), out, cap);
+        if (!h->rec.get(1) || h->settle()) return 0;
+        return fetch_floats(h->rec.get(1) + size_t(ch) * h->rec.pitch, 2 * size_t(x.last_nf), out, cap);
     case HBD_STAGE_DEMOD:
-        if (!h->demod.get()) return 0;
-        return fetch_floats(h, h->demod.get() + size_t(ch) * h->demod.pitch, size_t(x.last_nf), out, cap);
+        if (!h->demod.get() || h->settle()) return 0;
+        return fetch_floats(h->demod.get() + size_t(ch) * h->demod.pitch, size_t(x.last_nf), out, cap);
     case HBD_STAGE_LPTAPS:
-        return fetch_floats(h, h->d_lptaps.get() + size_t(ch) * kLpMaxTaps, x.lp_ntaps, out, cap);
+        if (h->settle()) return 0;
+        return fetch_floats(h->d_lptaps.get() + size_t(ch) * kLpMaxTaps, x.lp_ntaps, out, cap);
     case HBD_STAGE_PENDING: {
-        ChanState st; if (fetch_state(h, ch, &st)) return 0;
-        if (!h->slicer.get()) return 0;
-        return fetch_floats(h, h->slicer.get() + size_t(ch) * h->slicer.pitch, st.slicer_n, out, cap);
+        ChanState st;
+        if (!h->slicer.get() || h->read_states(size_t(ch), 1, &st)) return 0;
+        return fetch_floats(h->slicer.get() + size_t(ch) * h->slicer.pitch, st.slicer_n, out, cap);
     }
     case HBD_STAGE_BITS: {
-        if (!h->d_rec_bits.get()) return 0;
-        cudaSetDevice(h->device); h->sync_groups(); cudaStreamSynchronize(h->stream);
+        if (!h->d_rec_bits.get() || h->settle()) return 0;
         unsigned nb = 0;
-        cudaMemcpy(&nb, h->d_rec_bits_n.get() + ch, 4, cudaMemcpyDeviceToHost);
+        if (cudaMemcpy(&nb, h->d_rec_bits_n.get() + ch, 4, cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
         nb = std::min(nb, h->rec_bits_pitch);
         if (out && cap && nb) {
             std::vector<unsigned char> b(nb);
-            cudaMemcpy(b.data(), h->d_rec_bits.get() + size_t(ch) * h->rec_bits_pitch, nb, cudaMemcpyDeviceToHost);
+            if (cudaMemcpy(b.data(), h->d_rec_bits.get() + size_t(ch) * h->rec_bits_pitch, nb, cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
             for (size_t i = 0; i < std::min<size_t>(nb, cap); ++i) out[i] = float(b[i]);
         }
         return nb;

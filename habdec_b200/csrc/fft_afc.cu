@@ -385,17 +385,10 @@ cudaError_t launch_fft_afc(const FftArgs& a, int n_channels, cudaStream_t stream
     return launch_fft_n<4096>(a, n_channels, stream, launches);   // fft_afc4096_kernel
 }
 
-// AFC::resetFrequencyCorrection (AFC.h:188-194), one thread per call
+// hbd_reset_frequency_correction, one thread per call
 __global__ void afc_reset_kernel(ChanState* state, int ch, double corr, double fs_dec, int n_fft)
 {
-    ChanState& st = state[ch];
-    // the reference divides fft_samples_.size() by its sampling rate: both are 0 before the first spectrum
-    const double bins_per_hz = st.have_spectrum ? __ddiv_rn(double(n_fft), fs_dec) : __ddiv_rn(0.0, 0.0);
-    const double l = __dsub_rn(avg_get_i(st.pl_sum, st.pl_cnt), __dmul_rn(corr, bins_per_hz));
-    const double r = __dsub_rn(avg_get_i(st.pr_sum, st.pr_cnt), __dmul_rn(corr, bins_per_hz));
-    st.pl_sum = int(fmax(0.0, l)); st.pl_cnt = 1;
-    st.pr_sum = int(fmax(0.0, r)); st.pr_cnt = 1;
-    st.afc_correction = 0;
+    afc_reset(state[ch], corr, fs_dec, n_fft);
 }
 
 cudaError_t launch_afc_reset(ChanState* state, int ch, double corr, double fs_dec, int n_fft, cudaStream_t stream)
@@ -415,12 +408,7 @@ __global__ void afc_retune_kernel(ChanState* state, int n_ch, double min_abs_hz,
     const double corr = st.afc_correction;
     if (!(min_abs_hz < fabs(corr))) { applied[ch] = 0.0; return; }
     applied[ch] = corr;
-    const double bins_per_hz = st.have_spectrum ? __ddiv_rn(double(n_fft), fs_dec) : __ddiv_rn(0.0, 0.0);
-    const double l = __dsub_rn(avg_get_i(st.pl_sum, st.pl_cnt), __dmul_rn(corr, bins_per_hz));
-    const double r = __dsub_rn(avg_get_i(st.pr_sum, st.pr_cnt), __dmul_rn(corr, bins_per_hz));
-    st.pl_sum = int(fmax(0.0, l)); st.pl_cnt = 1;
-    st.pr_sum = int(fmax(0.0, r)); st.pr_cnt = 1;
-    st.afc_correction = 0;
+    afc_reset(st, corr, fs_dec, n_fft);
 }
 
 cudaError_t launch_afc_retune(ChanState* state, int n_ch, double min_abs_hz, double fs_dec, double* applied, int n_fft, cudaStream_t stream)
