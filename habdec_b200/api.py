@@ -94,6 +94,16 @@ class ScanParams(C.Structure):
     _fields_ = [("min_snr_db", C.c_double), ("min_shift_hz", C.c_double), ("max_shift_hz", C.c_double), ("max_tone_ratio_db", C.c_double)]
 
 
+class BaudEstimate(C.Structure):
+    _fields_ = [("baud", C.c_double), ("nominal", C.c_double), ("confidence", C.c_double), ("runs", C.c_uint), ("long_runs", C.c_uint)]
+
+
+# hbd_baud_estimate as a numpy record (BatchDecoder.baud_estimates)
+BAUD_ESTIMATE_DTYPE = np.dtype([("baud", np.float64), ("nominal", np.float64), ("confidence", np.float64), ("runs", np.uint32),
+                                ("long_runs", np.uint32)])
+assert BAUD_ESTIMATE_DTYPE.itemsize == C.sizeof(BaudEstimate)
+
+
 class ScanSignal(C.Structure):
     _fields_ = [("center_hz", C.c_double), ("shift_hz", C.c_double), ("snr_db", C.c_double), ("bin_lo", C.c_int), ("bin_hi", C.c_int)]
 
@@ -233,6 +243,10 @@ SIGNATURES = {
     "hbd_scan_default_params": (None, [C.POINTER(ScanParams)]),
     "hbd_scan_find": (C.c_int, [C.c_void_p, C.POINTER(ScanParams), C.c_void_p, C.c_size_t]),
     "hbd_scan_detect": (C.c_int, [C.c_void_p, C.c_size_t, C.c_double, C.POINTER(ScanParams), C.c_void_p, C.c_size_t]),
+    "hbd_set_baud_estimation": (C.c_int, [_H, C.c_int]),
+    "hbd_get_baud_estimates": (C.c_int, [_H, C.c_void_p, C.c_size_t]),
+    "hbd_apply_baud_estimates": (C.c_int, [_H, C.c_double, C.c_uint, C.c_void_p]),
+    "hbd_get_baud_histogram": (C.c_size_t, [_H, C.c_int, C.c_void_p, C.c_size_t]),
     "hbd_debug_stage": (C.c_size_t, [_H, C.c_int, C.c_int, C.c_void_p, C.c_size_t]),
     "hbd_design_lowpass": (C.c_size_t, [C.c_float, C.c_float, C.c_size_t, C.c_size_t, C.c_void_p, C.c_size_t]),
     "hbd_extract_sentence": (C.c_int, [C.c_char_p, C.c_size_t, C.c_char_p, C.c_char_p, C.c_char_p, C.c_size_t, C.POINTER(C.c_size_t)]),
@@ -684,6 +698,33 @@ class BatchDecoder:
         rc = self._lib.hbd_afc_retune(self._h, float(min_abs_hz), out.ctypes.data)
         if rc < 0:
             self._chk(rc)
+        return out
+
+    # ---- baud-rate estimation (hbd_set_baud_estimation ..., the estimator is stated in include/habdec_b200.h)
+    def set_baud_estimation(self, on): self._chk(self._lib.hbd_set_baud_estimation(self._h, int(bool(on))))
+
+    def baud_estimates(self) -> np.ndarray:
+        """Every channel's estimate as of all calls so far: a BAUD_ESTIMATE_DTYPE array [n_channels]."""
+        out = np.zeros(self.n_channels, dtype=BAUD_ESTIMATE_DTYPE)
+        rc = self._lib.hbd_get_baud_estimates(self._h, out.ctypes.data, out.size)
+        if rc < 0:
+            self._chk(rc)
+        return out
+
+    def apply_baud_estimates(self, min_confidence: float = 0.8, min_runs: int = 100) -> np.ndarray:
+        """Set each confident channel's baud to its nominal rate; returns the rates set [n_channels] (0 = unchanged)."""
+        out = np.zeros(self.n_channels, dtype=np.float64)
+        rc = self._lib.hbd_apply_baud_estimates(self._h, float(min_confidence), int(min_runs), out.ctypes.data)
+        if rc < 0:
+            self._chk(rc)
+        return out
+
+    def baud_histogram(self, ch: int) -> np.ndarray:
+        """The channel's run histogram H[0 .. Lmax] (test hook; empty while estimation is off or before the first push)."""
+        n = self._lib.hbd_get_baud_histogram(self._h, int(ch), None, 0)
+        out = np.zeros(n, dtype=np.uint32)
+        if n and self._lib.hbd_get_baud_histogram(self._h, int(ch), out.ctypes.data, n) != n:
+            raise HbdError("hbd_get_baud_histogram failed: %s" % (self._lib.hbd_last_error(self._h) or b"").decode())
         return out
 
     def pushWideband(self, iq: np.ndarray, fs: float):

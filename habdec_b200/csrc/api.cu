@@ -17,6 +17,7 @@
 #include <thread>
 #include <vector>
 
+#include "baud.cuh"
 #include "decim1.cuh"
 #include "iq_format.cuh"
 #include "mid.cuh"
@@ -148,17 +149,20 @@ __host__ __device__ inline void fresh_state(ChanState& s)
 // for a longer filter), and the per-channel counts of the demod accumulator, the SSDV ring and the recorded bits.
 // The carry and stage histories are zeroed by the next call's plan (grown* == 0); every other row is rewritten
 // before it is read (FFT frame from fft_have = 0, spectra behind have_spectrum, slicer / mask / UART rows below
-// their counts).
+// their counts).  With baud estimation on it also restarts the channel's estimator.
 struct ResetArgs {
     ChanState* state; const int* list;
     float2* decq; size_t dq_pitch;   // nullptr before the first call sized it
     unsigned* dacc_n; unsigned* ssdv_total; unsigned* ssdv_scanned; unsigned* rec_bits_n;   // the last three may be nullptr
+    unsigned* bhist; size_t bhist_pitch; BaudTrack* btrack;   // nullptr while baud estimation has no rows
 };
 __global__ void reset_chan_kernel(ResetArgs a)
 {
     const int ch = a.list[blockIdx.x];
     if (a.decq) for (int i = threadIdx.x; i < kLpHist; i += blockDim.x) a.decq[size_t(ch) * a.dq_pitch + i] = make_float2(0.f, 0.f);
+    if (a.bhist) for (size_t i = threadIdx.x; i < a.bhist_pitch; i += blockDim.x) a.bhist[size_t(ch) * a.bhist_pitch + i] = 0u;
     if (threadIdx.x) return;
+    if (a.btrack) a.btrack[ch] = BaudTrack{};
     fresh_state(a.state[ch]);
     a.dacc_n[ch] = 0;
     if (a.ssdv_total) { a.ssdv_total[ch] = 0; a.ssdv_scanned[ch] = 0; }
@@ -439,6 +443,16 @@ struct hbd_decoder {
     DistSlot dist_ctx;               // dist.cu
     int enable_snap();
 
+    // baud-rate estimation (baud.cu); off until hbd_set_baud_estimation, and then without rows until fs_dec is known
+    bool baud_on = false;
+    double baud_fs = 0;                  // fs_dec the rows were sized and zeroed for; 0: the estimator restarts at its next use
+    int baud_lmax = 0;
+    DevPtr<unsigned> d_bhist;            // run histograms [n][baud_lmax + 1]
+    DevPtr<BaudTrack> d_btrack;          // edge state [n]
+    DevPtr<hbd_baud_estimate> d_best;    // the score kernel's output [n]
+    int baud_start();
+    int baud_estimates(std::vector<hbd_baud_estimate>& out);
+
     void set_error(const std::string& e) { err = e; }
     int ensure_call_capacity(size_t n_in_max);
     int alloc_fixed();
@@ -628,6 +642,7 @@ int hbd_decoder::set_plan(const std::vector<TapTable>& st, size_t total_factor)
     for (auto& x : hc) { x.grown1 = x.grown2 = 0; for (size_t& g : x.grown_mid) g = 0; }
     cap_n_in = 0;
     h_plan_uploaded.clear();
+    baud_fs = 0;   // fs_dec (the histograms' unit) may have changed, and the stream starts over
     return HBD_OK;
 }
 
@@ -818,6 +833,7 @@ int hbd_decoder::plan_call(CallPlan& cp)
     for (size_t c = 0; c < stepped; ++c) max_total = std::max<size_t>(max_total, size_t(hc[c].in_r) + pushed(c));
     if (max_total > cap_n_in || !s1x.get()) { if (quiesce()) return HBD_ERR_CUDA; }   // buffers are about to be reallocated
     { const int rc = ensure_call_capacity(max_total); if (rc) return rc; }
+    if (baud_on) { const int rc = baud_start(); if (rc) return rc; }
     unsigned max_nf = 0;
     std::vector<float> new_taps;
     for (size_t c = 0; c < stepped; ++c) {
@@ -953,6 +969,15 @@ int hbd_decoder::enqueue_call(const CallPlan& cp)
         // only the tail kernel reads the stage-1 buffer: K1 of the call after next may overwrite it as soon as the
         // tail is done, without waiting for the FFT / SSDV / demod kernels behind it on this stream
         if (!tail_ev_late) { HBD_CUDA_CHECK(cudaEventRecord(ev_tail[s1_cur].get(), lo.get())); tail_recorded = true; }
+        if (baud_on) {   // the run histograms, from the discriminator output the tail kernel has just written
+            BaudHistArgs ba{};
+            ba.plan = d_plan.get(); ba.uplan = cp.uplan; ba.uniform = cp.plan_uniform ? 1 : 0; ba.state = d_state.get();
+            ba.demod = demod.get(); ba.demod_pitch = demod.pitch;
+            ba.hist = d_bhist.get(); ba.hist_pitch = size_t(baud_lmax) + 1; ba.track = d_btrack.get();
+            const BaudGeometry g = baud_geometry(fs_dec);
+            ba.lmax = g.lmax; ba.m = g.m;
+            HBD_CUDA_CHECK(launch_baud_hist(ba, n_ch, lo.get(), &nl));
+        }
         FftArgs fa{};
         fa.state = d_state.get(); fa.fftbuf = fft.buf.get(); fa.spectrum = fft.spectrum.get(); fa.power = fft.power.get(); fa.twiddle = fft.twiddle.get(); fa.fs_dec = fs_dec;
         fa.ch0 = 0; fa.fft_n = fft_n;
@@ -1302,9 +1327,51 @@ int hbd_decoder::reset_channels(const int* chs, size_t k)
     a.state = d_state.get(); a.list = d_reset.get();
     a.decq = decq.get(); a.dq_pitch = decq.pitch;
     a.dacc_n = d_dacc_n.get(); a.ssdv_total = d_ssdv_total.get(); a.ssdv_scanned = d_ssdv_scanned.get(); a.rec_bits_n = d_rec_bits_n.get();
+    a.bhist = d_bhist.get(); a.bhist_pitch = size_t(baud_lmax) + 1; a.btrack = d_btrack.get();
     reset_chan_kernel<<<unsigned(k), 128, 0, stream>>>(a);
     ++launches;
     HBD_CUDA_CHECK(cudaGetLastError());
+    return HBD_OK;
+}
+
+// (Re)start every channel's baud estimator for the current fs_dec: rows sized for its histogram, zeroed.  A no-op while
+// the rows are current; otherwise it waits for the compute streams.  A failed allocation changes nothing.
+int hbd_decoder::baud_start()
+{
+    const double fs = fs_in / factor;
+    if (baud_fs == fs) return HBD_OK;
+    const size_t n = size_t(n_ch);
+    const BaudGeometry g = baud_geometry(fs);
+    const size_t pitch = size_t(g.lmax) + 1;
+    if (sync_groups()) { set_error("stream sync failed"); return HBD_ERR_CUDA; }   // a histogram kernel may still use the rows
+    DevPtr<unsigned> hist; DevPtr<BaudTrack> track; DevPtr<hbd_baud_estimate> est;
+    if (!d_bhist || g.lmax != baud_lmax) {   // the three buffers are allocated together
+        if (dev_alloc(hist, n * pitch) != cudaSuccess || dev_alloc(track, n) != cudaSuccess || dev_alloc(est, n) != cudaSuccess) {
+            set_error("baud estimation: out of device memory");
+            return HBD_ERR_NOMEM;
+        }
+    }
+    HBD_CUDA_CHECK(cudaMemsetAsync(hist ? hist.get() : d_bhist.get(), 0, n * pitch * sizeof(unsigned), stream));
+    HBD_CUDA_CHECK(cudaMemsetAsync(track ? track.get() : d_btrack.get(), 0, n * sizeof(BaudTrack), stream));
+    HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
+    if (hist) { d_bhist = std::move(hist); d_btrack = std::move(track); d_best = std::move(est); baud_lmax = g.lmax; }
+    baud_fs = fs;
+    return HBD_OK;
+}
+
+// every channel's estimate as of all calls enqueued so far (estimation on): zeros before the first push, else one score
+// kernel once everything enqueued is done, and one copy
+int hbd_decoder::baud_estimates(std::vector<hbd_baud_estimate>& out)
+{
+    out.assign(size_t(n_ch), hbd_baud_estimate{});
+    if (!fs_in) return HBD_OK;
+    HBD_CUDA_CHECK(cudaSetDevice(device));
+    { const int rc = baud_start(); if (rc) return rc; }
+    if (settle()) return HBD_ERR_CUDA;
+    HBD_CUDA_CHECK(launch_baud_score(d_bhist.get(), size_t(baud_lmax) + 1, baud_lmax, d_btrack.get(), fs_in / factor, d_best.get(), n_ch, stream));
+    ++launches;
+    HBD_CUDA_CHECK(cudaMemcpyAsync(out.data(), d_best.get(), out.size() * sizeof(hbd_baud_estimate), cudaMemcpyDeviceToHost, stream));
+    HBD_CUDA_CHECK(cudaStreamSynchronize(stream));
     return HBD_OK;
 }
 
@@ -2215,6 +2282,63 @@ int hbd_afc_retune(hbd_decoder* h, double min_abs_hz, double* applied_out)
     }
     return count;
 }
+int hbd_set_baud_estimation(hbd_decoder* h, int on)
+{
+    HBD_CHECK_H(h);
+    std::lock_guard<std::mutex> l(h->mtx);
+    if ((on != 0) == h->baud_on) return HBD_OK;
+    if (cudaSetDevice(h->device) != cudaSuccess) return HBD_ERR_CUDA;
+    if (on) {
+        h->baud_on = true; h->baud_fs = 0;
+        const int rc = h->fs_in ? h->baud_start() : HBD_OK;   // otherwise at the first call
+        if (rc) h->baud_on = false;
+        return rc;
+    }
+    if (h->sync_groups()) { h->set_error("stream sync failed"); return HBD_ERR_CUDA; }
+    h->baud_on = false; h->baud_fs = 0; h->baud_lmax = 0;
+    h->d_bhist.reset(); h->d_btrack.reset(); h->d_best.reset();
+    return HBD_OK;
+}
+int hbd_get_baud_estimates(hbd_decoder* h, hbd_baud_estimate* out, size_t cap)
+{
+    HBD_CHECK_H(h);
+    std::lock_guard<std::mutex> l(h->mtx);
+    if (!h->baud_on) { h->set_error("baud estimation is off"); return HBD_ERR_STATE; }
+    std::vector<hbd_baud_estimate> est;
+    if (out && cap) {
+        const int rc = h->baud_estimates(est);
+        if (rc) return rc;
+        memcpy(out, est.data(), std::min(cap, est.size()) * sizeof(hbd_baud_estimate));
+    }
+    return h->n_ch;
+}
+int hbd_apply_baud_estimates(hbd_decoder* h, double min_confidence, unsigned min_runs, double* applied)
+{
+    HBD_CHECK_H(h);
+    std::lock_guard<std::mutex> l(h->mtx);
+    if (!h->baud_on) { h->set_error("baud estimation is off"); return HBD_ERR_STATE; }
+    std::vector<hbd_baud_estimate> est;
+    { const int rc = h->baud_estimates(est); if (rc) return rc; }
+    int count = 0;
+    for (size_t c = 0; c < est.size(); ++c) {
+        const hbd_baud_estimate& e = est[c];
+        const bool set = e.nominal > 0 && e.runs >= min_runs && e.confidence >= min_confidence && e.nominal != h->hc[c].baud;
+        if (set) { h->hc[c].baud = e.nominal; h->hc[c].cfg_dirty = true; ++count; }   // what hbd_set_baud(h, c, nominal) does
+        if (applied) applied[c] = set ? e.nominal : 0.0;
+    }
+    if (count) h->cfg_dirty_any = h->derived_dirty = true;
+    return count;
+}
+size_t hbd_get_baud_histogram(hbd_decoder* h, int ch, unsigned* out, size_t cap)
+{
+    if (!h || ch < 0 || ch >= h->n_ch) return 0;
+    std::lock_guard<std::mutex> l(h->mtx);
+    if (!h->baud_on || !h->fs_in || cudaSetDevice(h->device) != cudaSuccess || h->baud_start() || h->settle()) return 0;
+    const size_t len = size_t(h->baud_lmax) + 1;
+    if (out && cap && cudaMemcpy(out, h->d_bhist.get() + size_t(ch) * len, std::min(cap, len) * sizeof(unsigned), cudaMemcpyDeviceToHost) != cudaSuccess) return 0;
+    return len;
+}
+
 // all channels in one device->host copy: out[ch*6 + {0..5}] = correction, shift, noise floor, noise variance, peak l, peak r
 size_t hbd_get_stats_batch(hbd_decoder* h, double* out, size_t cap_doubles)
 {

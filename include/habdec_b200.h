@@ -396,6 +396,51 @@ void   hbd_scan_default_params(hbd_scan_params* p);
 int    hbd_scan_find(hbd_scanner* s, const hbd_scan_params* p, hbd_scan_signal* out, size_t cap);
 int    hbd_scan_detect(const float* psd, size_t n, double fs, const hbd_scan_params* p, hbd_scan_signal* out, size_t cap);   /* host only */
 
+/* ---- baud-rate estimation (new; in the reference a person types the rate into the web UI, cmd::set:baud) ----------
+ * Measures each channel's keying rate on the GPU from its discriminator output d[i] (the floats hbd_debug_stage(
+ * HBD_STAGE_DEMOD) returns, in stream order across calls; i counts samples since the estimator (re)started), so that a
+ * channel tuned to a scanned signal can be set to its rate.  It only observes: no channel's decoding changes until the
+ * caller applies a result.  Like the slicer it needs the tone pair to straddle DC (after the NCO).
+ *
+ * fs = fs_dec (hbd_get_decimated_sampling_rate); candidates B = {50, 75, 100, 150, 200, 300, 600} with fs / b >= 8;
+ * debounce m = max(1, floor(fs / 2400)); histogram length Lmax = ceil(6.5 fs / 50).
+ *  1. s[i] = d[i] > 0 (a zero counts as negative).
+ *  2. The channel holds a current sign, taken from its first sample.  An edge is accepted once m consecutive samples have
+ *     the opposite sign (a shorter opposite streak is discarded); its position is the first sample of that streak, and
+ *     the current sign flips.
+ *  3. For each accepted edge after the first, L = position - previous edge position: H[L] += 1 (uint32) if
+ *     1 <= L <= Lmax, else long_runs += 1.  Streak and edge state carry across calls.
+ *  4. On query, for each candidate b with sp = fs / b (double): a run L is explained by b when k = floor(L / sp + 0.5)
+ *     has 1 <= k <= 6 and fabs(L - k sp) <= 0.2 sp (evaluated without fused multiply-adds).  E(b) = sum of H[L] over
+ *     the explained runs (uint64).
+ *  5. runs = sum H.  nominal = the lowest candidate with 10 E(b) >= 9 max E (integers: a harmonic explains the same runs,
+ *     the lower rate wins); confidence = E(nominal) / runs; baud = fs * sum(H[L] k) / sum(H[L] L) over the runs nominal
+ *     explains (uint64 sums, then double; 0 when it explains none): the payload's actual clock, e.g. 297.0 for a
+ *     "300 baud" payload.  runs == 0: baud, nominal and confidence are 0.
+ *
+ * Off by default; while off it launches and allocates nothing.  On, it adds one kernel per call that does work, and
+ * (Lmax + 1) * 4 bytes per channel (4 KB at fs_dec = 8 kHz, 40 KB at 78 125 Hz).  The estimator restarts (histograms and
+ * edge state zeroed) when switched on, for the listed channels on hbd_reset_channels, and for every channel when the
+ * decimation plan changes; the baud, framing, low-pass, NCO and FFT-size setters leave it alone.  Switching it on before
+ * the first push sizes the rows at the first call.  A failed allocation returns HBD_ERR_NOMEM and changes nothing. */
+typedef struct hbd_baud_estimate {
+    double   baud;        /* fitted rate (step 5); 0: no run yet */
+    double   nominal;     /* picked candidate of {50, 75, 100, 150, 200, 300, 600}; 0: no run yet */
+    double   confidence;  /* E(nominal) / runs */
+    unsigned runs;        /* runs histogrammed since the estimator (re)started */
+    unsigned long_runs;   /* runs longer than the histogram (not in `runs`) */
+} hbd_baud_estimate;
+int    hbd_set_baud_estimation(hbd_decoder* h, int on);                         /* handle-wide, default off */
+/* every channel, as of all calls enqueued so far (waits for them); out[0 .. min(cap, n_channels)); returns n_channels
+ * (< 0: error; HBD_ERR_STATE when off) */
+int    hbd_get_baud_estimates(hbd_decoder* h, hbd_baud_estimate* out, size_t cap);
+/* where runs >= min_runs, confidence >= min_confidence and nominal != the channel's baud: exactly hbd_set_baud(h, ch,
+ * nominal).  applied[n_channels] (may be NULL) receives the new rate or 0; returns the number of channels changed
+ * (< 0: error; HBD_ERR_STATE when off) */
+int    hbd_apply_baud_estimates(hbd_decoder* h, double min_confidence, unsigned min_runs, double* applied);
+/* test hook: the channel's H[0 .. Lmax]; returns Lmax + 1 (0: bad channel, estimation off or no push yet) */
+size_t hbd_get_baud_histogram(hbd_decoder* h, int ch, unsigned* out, size_t cap);
+
 /* ---- test hooks ------------------------------------------------------------------------------------------ */
 enum { HBD_STAGE_DECIMATED = 0, HBD_STAGE_FILTERED = 1, HBD_STAGE_DEMOD = 2, HBD_STAGE_LPTAPS = 5,
        HBD_STAGE_PENDING = 6, HBD_STAGE_BITS = 7 };

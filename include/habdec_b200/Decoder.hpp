@@ -95,6 +95,22 @@ public:
     void nco(double freq_hz, int ch = -1) { hbd_set_nco(h_, ch, freq_hz); }
     double nco(int ch) const { return hbd_get_nco(h_, ch); }
     int afcRetune(double min_abs_hz = 100.0, double* applied = nullptr) { return hbd_afc_retune(h_, min_abs_hz, applied); }
+    // baud-rate estimation (include/habdec_b200.h): every channel's keying rate measured on the GPU, applied on request
+    int setBaudEstimation(bool on) { return status_ = hbd_set_baud_estimation(h_, on ? 1 : 0); }
+    std::vector<hbd_baud_estimate> getBaudEstimates()
+    {
+        std::vector<hbd_baud_estimate> v(static_cast<size_t>(channels()));
+        status_ = hbd_get_baud_estimates(h_, v.data(), v.size());
+        if (status_ < 0) v.clear(); else status_ = HBD_OK;
+        return v;
+    }
+    // returns the number of channels retuned (< 0: error); applied[channels()] may be null
+    int applyBaudEstimates(double min_confidence = 0.8, unsigned min_runs = 100, double* applied = nullptr)
+    {
+        const int rc = hbd_apply_baud_estimates(h_, min_confidence, min_runs, applied);
+        status_ = rc < 0 ? rc : HBD_OK;
+        return rc;
+    }
 
     // configure (ch = -1: every channel)
     void baud(double v, int ch = -1) { hbd_set_baud(h_, ch, v); }
